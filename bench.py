@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, sm_100a)
     python bench.py --impl reference --gpus N ...            # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # + what the last timed step returned, as DIR/*.npy
 
 A "step" = one control step of a1_conditional on resident simulator state:
 PD torque x4 (+ action scale/clip), fused post-physics (body-frame carry, 187-point height scan,
@@ -138,6 +139,26 @@ def build_a1(n_local, rank, world, device, terrain=None, seed=1234, carry=True, 
 
 LAUNCHES_PER_STEP = 4 + 1 + 1 + 1 + 1      # pd x4, fused post-physics, compaction, collect, publish (libshifu_b200.so kernels;
                                            # the action copy into the graph input buffer is torch's)
+DUMP_ROWS = 32768                          # envs written by --dump-outputs: 32768 x 262 floats = 34 MB
+
+
+def dump_outputs(env, out_dir):
+    """What ``A1Conditional.step`` returned in the last step (obs, rew, dones, extras) as float32 .npy
+    files in ``out_dir``: per-env arrays for a fixed, seeded sample of DUMP_ROWS envs (all envs when
+    there are fewer; ``env_ids.npy``, float64, lists them), the extras' episode statistics whole.  The inputs are
+    seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    n = env.num_envs
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    idx = torch.from_numpy(rows).to(env.obs_buf.device)
+    out = {"obs": env.obs_buf, "rew": env.rew_buf, "reset": env.reset_buf, "time_outs": env.extras["time_outs"]}
+    out = {k: v.index_select(0, idx).float() for k, v in out.items()}
+    out.update({"episode_" + k: v.float() for k, v in env.extras["episode"].items()})
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_ids.npy"), rows.astype(np.float64))
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.cpu().numpy())
 
 
 def time_steps(env, raw_actions, steps, warmup, barrier=None, flush=None):
@@ -491,6 +512,8 @@ def run_ours(args):
         sampler.start()
     total_ms = time_steps(env, raw, args.steps, args.warmup, barrier)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs)
     t = torch.tensor([total_ms], device=device, dtype=torch.double)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -534,9 +557,6 @@ def run_ours(args):
                        "d2h_bytes_per_step": d2h, "ms_per_step": e_ms / e_steps,
                        "note": "A1Conditional.step with pinned host state+actions -> device, obs+rew+reset -> pinned host; "
                                "upload of step t+1 overlaps read-back of step t (3 streams); PCIe-bound"}
-        # a longer timed region than the driver's K, for the record
-        long_ms = time_steps(env, raw, 200, 5)
-        line["value_200_steps"] = n / (long_ms / 200 * 1e-3)
         if os.environ.get("SHIFU_BENCH_TRAFFIC", "1") != "0":
             tr, how = measure_traffic_live(n)
             if tr is None:
@@ -616,17 +636,31 @@ def _emit(line):
     out.flush()
 
 
+def _count(low):
+    def parse(s):
+        v = int(s)
+        if v < low:
+            raise argparse.ArgumentTypeError(f"must be >= {low}")
+        return v
+    return parse
+
+
 def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
-    ap.add_argument("--warmup", type=int, default=20)
+    ap.add_argument("--steps", type=_count(1), default=200, help="timed control steps")
+    ap.add_argument("--warmup", type=_count(0), default=20, help="untimed control steps before them")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32; "
+                         "env ids float64; at most 35 MB)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs-per-gpu", type=int, default=ENVS_PER_GPU)
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
     ap.add_argument("--quick", action="store_true", help="timed region only (for runs under ncu)")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the CUDA path's outputs; it does not apply to --impl reference")
     if args.impl == "reference":
         run_reference(args)
     else:
