@@ -28,7 +28,7 @@ from __future__ import annotations
 
 import math
 from dataclasses import dataclass, field
-from typing import Dict, List, Optional
+from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 import torch
@@ -88,6 +88,13 @@ def quat_apply_yaw(quat, vec):
 
 A1_REWARD_TERMS = ["tracking_lin_vel", "tracking_ang_vel", "stabilizing_base", "smoothing_action",
                    "leg_collision", "torques_penalize"]   # a1_conditional.py:152-160
+# (p0, p1) of each term: the literals of a1_conditional.py:162-192 for the reference's six terms
+A1_TERM_PARAMS = {"tracking_lin_vel": (1.0, 0.25), "tracking_ang_vel": (0.5, 0.25), "stabilizing_base": (-2.0, -0.005),
+                  "smoothing_action": (-0.005, 0.0), "leg_collision": (-1., 0.1), "torques_penalize": (-2e-5, 0.0)}
+# legged_gym-style terms a user task may list (enum ShifuRewardTerm 8-15); their constants come with the list
+A1_EXTRA_TERMS = ("lin_vel_z", "ang_vel_xy", "orientation", "dof_vel", "action_rate", "base_height", "dof_pos_limits",
+                  "feet_air_time")
+A1_DOF_UNBOUNDED = 3.0e38                 # default dof_pos_limits: (-3e38, 3e38), never reached
 
 
 @dataclass
@@ -121,9 +128,22 @@ class A1Params:
     curriculum: bool = True
     rng_seed: int = 0x5EED
     env_offset: int = 0                      # global id of local env 0 (sharded runs)
+    # reward-term list in accumulation order: (name, p0, p1); default = the reference's six terms
+    terms: List[Tuple[str, float, float]] = None
+    # constants of the legged_gym-style terms beyond (p0, p1)
+    dof_pos_limits: torch.Tensor = None      # (12, 2) lower / upper soft limits; default unbounded
+    feet_bodies: Tuple[int, ...] = (4, 8, 12, 16)
+    feet_contact_force: float = 1.0          # a foot touches when F_z > this
+    air_time_cmd_min: float = 0.1            # feet_air_time is 0 unless |cmd_xy| > this
+    air_time_dt: float = 0.02                # control dt added to swing_time every step
+    air_time_reset: bool = True              # reset_idx zeroes swing_time / last_contacts of the env
 
     def __post_init__(self):
         f = lambda x: torch.tensor(x, dtype=torch.float)
+        if self.terms is None:
+            self.terms = [(k, *A1_TERM_PARAMS[k]) for k in A1_REWARD_TERMS]
+        if self.dof_pos_limits is None:
+            self.dof_pos_limits = f([[-A1_DOF_UNBOUNDED, A1_DOF_UNBOUNDED]] * 12)
         if self.q0 is None:
             self.q0 = f([0.1, 0.8, -1.5, 0.1, 0.8, -1.5, -0.1, 0.8, -1.5, -0.1, 0.8, -1.5])
         if self.kp is None:
@@ -187,6 +207,8 @@ class A1State:
     measured_heights: torch.Tensor = None
     reset_ids: torch.Tensor = None
     height_idx: Optional[torch.Tensor] = None   # (2, N*187) int64 px, py of the last scan
+    swing_time: torch.Tensor = None             # (N, feet) legged_gym feet_air_time
+    last_contacts: torch.Tensor = None          # (N, feet) bool
 
 
 def a1_new_state(p: A1Params, height_samples, terrain_origins, terrain_types, env_origins) -> A1State:
@@ -200,11 +222,12 @@ def a1_new_state(p: A1Params, height_samples, terrain_origins, terrain_types, en
         height_samples=height_samples, terrain_origins=terrain_origins, terrain_types=terrain_types,
         env_origins=env_origins.clone(), terrain_levels=z(n, dtype=torch.long), command=z(n, 3),
         history=z(n, p.n_dof, p.n_hist), ep_len=z(n, dtype=torch.long),
-        ep_sums={k: z(n) for k in A1_REWARD_TERMS}, dof_targets=z(n, p.n_dof),
+        ep_sums={t[0]: z(n) for t in p.terms}, dof_targets=z(n, p.n_dof),
         rand_force=z(n, p.n_bodies, 3), torques=z(n, p.n_dof),
         base_lin_vel=z(n, 3), base_ang_vel=z(n, 3), projected_gravity=g.clone(), gravity_vec=g,
         reset=torch.ones(n, dtype=torch.long), time_out=z(n, dtype=torch.bool),
-        obs=z(n, 259), rew=z(n),
+        obs=z(n, 259), rew=z(n), swing_time=z(n, len(p.feet_bodies)),
+        last_contacts=z(n, len(p.feet_bodies), dtype=torch.bool),
     )
 
 
@@ -255,25 +278,102 @@ def a1_compute_termination(p: A1Params, st: A1State):
 
 
 def a1_reward_terms(p: A1Params, st: A1State) -> Dict[str, torch.Tensor]:
-    """The six terms — a1_conditional.py:162-192 (row a7)."""
-    cf = st.contact_state.view(p.n, -1, 3)
+    """The listed terms in list order, keyed by name (env.py:160-166).  The reference's six terms
+    follow a1_conditional.py:162-192 with their literals replaced by (p0, p1); the legged_gym-style
+    terms are written in legged_gym's torch form.  feet_air_time updates st.swing_time /
+    st.last_contacts (row a7)."""
     out = {}
+    for name, p0, p1 in p.terms:
+        out[name] = _A1_TERMS[name](p, st, p0, p1)
+    return out
+
+
+def _tracking_lin_vel(p, st, p0, p1):
     lin_vel_error = torch.sum(torch.square(st.command[:, :2] - st.base_lin_vel[:, :2]), dim=1)
-    out["tracking_lin_vel"] = 1.0 * torch.exp(-lin_vel_error / 0.25)
+    return p0 * torch.exp(-lin_vel_error / p1)
+
+
+def _tracking_ang_vel(p, st, p0, p1):
     ang_vel_error = torch.square(st.command[:, 2] - st.base_ang_vel[:, 2])
-    out["tracking_ang_vel"] = 0.5 * torch.exp(-ang_vel_error / 0.25)
-    z_vel = -2.0 * torch.square(st.base_lin_vel[:, 2])
-    ang_vel = -0.005 * torch.sum(torch.square(st.base_ang_vel[:, :2]), dim=1)
-    out["stabilizing_base"] = z_vel + ang_vel
+    return p0 * torch.exp(-ang_vel_error / p1)
+
+
+def _stabilizing_base(p, st, p0, p1):
+    z_vel = p0 * torch.square(st.base_lin_vel[:, 2])
+    ang_vel = p1 * torch.sum(torch.square(st.base_ang_vel[:, :2]), dim=1)
+    return z_vel + ang_vel
+
+
+def _smoothing_action(p, st, p0, p1):
     a0, a1, a2 = st.history[..., 0], st.history[..., 1], st.history[..., 2]
     first = torch.sum(torch.square(a1 - a0), dim=1)
     second = torch.sum(torch.square(a2 - 2 * a1 + a0), dim=1)
-    out["smoothing_action"] = -0.005 * (first + second)
+    return p0 * (first + second)
+
+
+def _leg_collision(p, st, p0, p1):
+    cf = st.contact_state.view(p.n, -1, 3)
     leg_idx = torch.tensor(p.leg_indices, dtype=torch.long)
-    leg_touch = (torch.norm(cf[:, leg_idx, :], dim=-1) > 0.1)
-    out["leg_collision"] = -1. * torch.sum(leg_touch.to(torch.float), dim=1)
-    out["torques_penalize"] = -2e-5 * torch.sum(torch.square(st.torques), dim=1)
-    return out
+    leg_touch = (torch.norm(cf[:, leg_idx, :], dim=-1) > p1)
+    return p0 * torch.sum(leg_touch.to(torch.float), dim=1)
+
+
+def _torques_penalize(p, st, p0, p1):
+    return p0 * torch.sum(torch.square(st.torques), dim=1)
+
+
+def _lin_vel_z(p, st, p0, p1):
+    return p0 * torch.square(st.base_lin_vel[:, 2])
+
+
+def _ang_vel_xy(p, st, p0, p1):
+    return p0 * torch.sum(torch.square(st.base_ang_vel[:, :2]), dim=1)
+
+
+def _orientation(p, st, p0, p1):
+    return p0 * torch.sum(torch.square(st.projected_gravity[:, :2]), dim=1)
+
+
+def _dof_vel(p, st, p0, p1):
+    return p0 * torch.sum(torch.square(st.dof_state.view(p.n, p.n_dof, 2)[..., 1]), dim=1)
+
+
+def _action_rate(p, st, p0, p1):
+    # actions_recorder.get_last(0): the history is pushed after the reward, so slot 0 is a_{t-1}
+    return p0 * torch.sum(torch.square(st.history[..., 0] - st.actions), dim=1)
+
+
+def _base_height(p, st, p0, p1):
+    return p0 * torch.square(st.root_state[:, 2] - p1)
+
+
+def _dof_pos_limits(p, st, p0, p1):
+    dof_pos = st.dof_state.view(p.n, p.n_dof, 2)[..., 0]
+    out_of_limits = -(dof_pos - p.dof_pos_limits[:, 0]).clip(max=0.)
+    out_of_limits += (dof_pos - p.dof_pos_limits[:, 1]).clip(min=0.)
+    return p0 * torch.sum(out_of_limits, dim=1)
+
+
+def _feet_air_time(p, st, p0, p1):
+    """legged_gym _reward_feet_air_time on st.swing_time / st.last_contacts."""
+    cf = st.contact_state.view(p.n, -1, 3)
+    contact = cf[:, list(p.feet_bodies), 2] > p.feet_contact_force
+    contact_filt = torch.logical_or(contact, st.last_contacts)
+    st.last_contacts[:] = contact
+    first_contact = (st.swing_time > 0.) * contact_filt
+    st.swing_time += p.air_time_dt
+    rew = torch.sum((st.swing_time - p1) * first_contact, dim=1)
+    rew *= torch.norm(st.command[:, :2], dim=1) > p.air_time_cmd_min
+    st.swing_time *= ~contact_filt
+    return p0 * rew
+
+
+_A1_TERMS = {"tracking_lin_vel": _tracking_lin_vel, "tracking_ang_vel": _tracking_ang_vel,
+             "stabilizing_base": _stabilizing_base, "smoothing_action": _smoothing_action,
+             "leg_collision": _leg_collision, "torques_penalize": _torques_penalize, "lin_vel_z": _lin_vel_z,
+             "ang_vel_xy": _ang_vel_xy, "orientation": _orientation, "dof_vel": _dof_vel,
+             "action_rate": _action_rate, "base_height": _base_height, "dof_pos_limits": _dof_pos_limits,
+             "feet_air_time": _feet_air_time}
 
 
 def a1_compute_reward(p: A1Params, st: A1State):
@@ -329,6 +429,9 @@ def a1_reset_idx(p: A1Params, st: A1State, env_ids):
     st.ep_len[env_ids] = 0
     st.reset[env_ids] = 1
     st.history.index_fill_(0, env_ids, 0.)                  # shifu/utils/train.py:16-17
+    if p.air_time_reset:                                    # legged_gym reset_idx: feet_air_time[env_ids] = 0
+        st.swing_time[env_ids] = 0.
+        st.last_contacts[env_ids] = False
     st.extras["episode"] = {}
     # un-normalised sums of this reset (what a sharded run all-reduces, SURVEY.md §8e)
     st.extras["_stats"] = {"sums": [float(st.ep_sums[k][env_ids].double().sum()) for k in st.ep_sums],

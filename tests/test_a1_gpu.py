@@ -276,22 +276,19 @@ def test_asymmetric_point_grid_matches_oracle():
         util.compare_a1(util.cuda_a1_outputs(hp), util.oracle_a1_outputs(st), f"asym-grid/s{t}")
 
 
-def test_kernel_instantiations_agree(monkeypatch):
-    """The pipelined kernel with / without measured_heights and the barrier-phased kernel are the
-    same function: bit-identical outputs on the same inputs (the bench runs without
-    measured_heights, the parity tests with)."""
+def _instantiations_agree(monkeypatch, term_kw, snap_kw):
     from shifu_b200.sim.synthetic import a1_snapshot
     n = 32 * 40 + 9
     hs, origins, types, env_origins = _terrain(n)
 
     def run(**kw):
-        hp = util.make_cuda_a1(n, hs, origins, types, env_origins, **kw)
+        hp = util.make_cuda_a1(n, hs, origins, types, env_origins, **kw, **term_kw)
         hp.reset_idx(None)
-        util.cuda_a1_step(hp, a1_snapshot(9, 0, n, p_base=0.05), torch.zeros(n, 12))
+        util.cuda_a1_step(hp, a1_snapshot(9, 0, n, **snap_kw), torch.zeros(n, 12))
         hp.ep_len.copy_(torch.from_numpy(np.random.RandomState(1).randint(0, 500, size=n)))
         outs = []
         for t in range(1, 4):
-            snap = a1_snapshot(9, t, n, p_base=0.05)
+            snap = a1_snapshot(9, t, n, **snap_kw)
             util.cuda_a1_step(hp, snap, snap.actions)
             outs.append(util.cuda_a1_outputs(hp))
         return outs
@@ -302,10 +299,26 @@ def test_kernel_instantiations_agree(monkeypatch):
     phased = run()
     for t, (a, b, c) in enumerate(zip(base, lean, phased), 1):
         assert "measured_heights" in a and "measured_heights" not in b
+        assert "swing_time" in a and "last_contacts" in a
         for k, v in a.items():
             if k in b:
                 assert np.array_equal(v, b[k]), f"no-measured-heights instantiation differs: {k} step {t}"
             assert np.array_equal(v, c[k]), f"phased kernel differs: {k} step {t}"
+
+
+def test_kernel_instantiations_agree(monkeypatch):
+    """The pipelined kernel with / without measured_heights and the barrier-phased kernel are the
+    same function: bit-identical outputs on the same inputs (the bench runs without
+    measured_heights, the parity tests with)."""
+    _instantiations_agree(monkeypatch, {}, dict(p_base=0.05))
+
+
+@pytest.mark.parametrize("terms", ["L1", "L2"])
+def test_kernel_instantiations_agree_term_lists(monkeypatch, terms):
+    """The same for the legged_gym-style term lists (tests/util.py::term_list): the HAS_EXTRA
+    instantiation of the pipelined kernel; L2 carries the feet-air-time state, compared too.  Legs touch
+    more often (p_leg) so the feet land."""
+    _instantiations_agree(monkeypatch, util.term_list(terms), dict(p_base=0.05, p_leg=0.3))
 
 
 def test_full_size_properties_1m():
