@@ -21,7 +21,7 @@ INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
 LIB_PATH = os.path.join(PKG_DIR, "libshifu_b200.so")
 
 SOURCES = ["capi.cu"]
-DEPS = ["capi.cu", "a1_kernels.cuh", "a1_fused.cuh", "a1_fused_tma.cuh", "tma_pipe.cuh", "f32x2.cuh","abb_kernels.cuh", "arm_ik.cuh", "camera_gather.cuh", "common_kernels.cuh", "exact_math.cuh", "philox.cuh", "terrain_gen.cuh", "scan_pairs.cuh", "dev_scan_only.cuh"]
+DEPS = ["capi.cu", "a1_kernels.cuh", "a1_fused.cuh", "a1_fused_tma.cuh", "tma_pipe.cuh", "f32x2.cuh","abb_kernels.cuh", "arm_ik.cuh", "camera_gather.cuh", "common_kernels.cuh", "exact_math.cuh", "philox.cuh", "terrain_gen.cuh", "scan_pairs.cuh"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -51,7 +51,7 @@ def source_hash() -> str:
     """Content hash of every source the library depends on (+ the flags).  Content, not mtimes:
     a repo snapshot copied to another machine, or a ``git checkout`` of an unchanged file, must not
     trigger a rebuild — with one process per GPU that would mean N concurrent nvcc runs."""
-    h = hashlib.sha256(" ".join(NVCC_FLAGS + os.environ.get("SHIFU_NVCC_EXTRA", "").split()).encode())
+    h = hashlib.sha256(" ".join(NVCC_FLAGS).encode())
     for path in _dep_paths():
         with open(path, "rb") as f:
             h.update(os.path.basename(path).encode() + b"\0" + f.read())     # not the absolute path: the tree moves
@@ -87,9 +87,8 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
 
 def _build_locked(verbose: bool) -> str:
-    extra = os.environ.get("SHIFU_NVCC_EXTRA", "").split()      # dev knob, e.g. -DV3_CTAS_CFG=3
     tmp = f"{LIB_PATH}.tmp{os.getpid()}"
-    cmd = [_nvcc(), *NVCC_FLAGS, *extra, "-I", INCLUDE, "-o", tmp] + [os.path.join(CSRC, s) for s in SOURCES]
+    cmd = [_nvcc(), *NVCC_FLAGS, "-I", INCLUDE, "-o", tmp] + [os.path.join(CSRC, s) for s in SOURCES]
     digest = source_hash()
     res = subprocess.run(cmd, capture_output=True, text=True)
     if res.returncode != 0:

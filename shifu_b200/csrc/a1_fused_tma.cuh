@@ -35,57 +35,17 @@
 
 namespace shifu {
 
-// B groups of 2 warps each: group g owns the tiles j = g, g + V3_B_GROUPS, ... (dev knob; 1 is fastest)
-#ifndef V3_BG_WARPS_CFG
-#define V3_BG_WARPS_CFG 3
-#endif
-#ifndef V3_B_GROUPS_CFG
-#define V3_B_GROUPS_CFG 1
-#endif
-#ifndef V3_SCAN_WARPS
-#define V3_SCAN_WARPS 12
-#endif
-#ifndef V3_CTAS_CFG
-#if V3_SCAN_WARPS == 6
-#define V3_CTAS_CFG 3
-#else
-#define V3_CTAS_CFG 2
-#endif
-#endif
-#ifndef V3_POLL_B
-#define V3_POLL_B 64
-#endif
-#ifndef V3_POLL_DMA
-#define V3_POLL_DMA 64
-#endif
-#ifndef V3_POLL_SCAN
-#define V3_POLL_SCAN 32
-#endif
-#ifdef V3_PARK_NS
-#define V3_WAIT(ns, bar, par) pipe::mbar_wait_parked(bar, par, V3_PARK_NS)
-#else
-#define V3_WAIT(ns, bar, par) pipe::mbar_wait<ns>(bar, par)
-#endif
-#ifndef V3_STAGES_CFG
-#if V3_SCAN_WARPS == 12
-#define V3_STAGES_CFG 3
-#else
-#define V3_STAGES_CFG 2
-#endif
-#endif
-constexpr int V3_STAGES = V3_STAGES_CFG;          // input stages per CTA (the scalar ring holds 4)
-constexpr int V3_B_GROUPS = V3_B_GROUPS_CFG;
-static_assert(V3_B_GROUPS == 1, "one B group per CTA (the stage ring assumes it)");   // B groups of 2 warps; group g owns tiles j = g, g + V3_B_GROUPS, ...
-constexpr int V3_CTAS_PER_SM = V3_CTAS_CFG;
-constexpr int V3_BG_WARPS = V3_BG_WARPS_CFG;            // warps 0, 1: terms + B2; further warps: terms only
-static_assert(V3_BG_WARPS >= 2 && V3_BG_WARPS <= A1K_TERM_WARPS, "B group: 2..A1K_TERM_WARPS warps");
-constexpr int V3_BG_THREADS = 32 * V3_BG_WARPS, V3_B2_THREADS = 64;
-constexpr int V3_B_THREADS = V3_B_GROUPS * V3_BG_THREADS, V3_C_THREADS = 32 * V3_SCAN_WARPS;
+constexpr int V3_STAGES = 3;                      // input stages per CTA (the scalar ring holds 4)
+constexpr int V3_CTAS_PER_SM = 2;
+constexpr int V3_BG_WARPS = 3;                    // warps 0, 1: terms + B2; warp 2: terms only
+constexpr int V3_SCAN_WARPS = 12;
+static_assert(V3_BG_WARPS <= A1K_TERM_WARPS, "A1K holds a term list per B warp");
+constexpr int V3_B_THREADS = 32 * V3_BG_WARPS, V3_B2_THREADS = 64;
+constexpr int V3_C_THREADS = 32 * V3_SCAN_WARPS;
 constexpr int V3_DMA_THREADS = 32;
 constexpr int V3_THREADS = V3_B_THREADS + V3_C_THREADS + V3_DMA_THREADS;
 constexpr int V3_SCAN_BASE = V3_B_THREADS;
 constexpr int V3_DMA_BASE = V3_B_THREADS + V3_C_THREADS;
-static_assert(V3_SCAN_WARPS == 6 || V3_SCAN_WARPS == 12, "scan group: 6 or 12 warps");
 constexpr uint32_t V3_OBS_CHUNK_BYTES = 8 * A1_OBS * 4;      // 8288 = 16 * 518
 
 struct alignas(128) V3In {            // one tile of simulator/env rows, each member 16-B aligned
@@ -103,7 +63,6 @@ struct alignas(128) V3In {            // one tile of simulator/env rows, each me
   // the B group and bulk-stored by the DMA lane together with the pushed history
   float cout[3][A1_TILE][3];          //  1152 B
 };
-static_assert(V3_STAGES >= 2 && V3_STAGES <= 4, "ring depth");
 static_assert(sizeof(V3In) == 22528 && offsetof(V3In, ep_len) == 18944 && offsetof(V3In, cout) % 16 == 0, "tile layout");
 
 struct alignas(128) V3Smem {
@@ -112,7 +71,7 @@ struct alignas(128) V3Smem {
   // two packed fp32x2 operands: sA = (2zq_e, 2zq_e1, zq_e, zq_e1), sB = (wq_e, wq_e1, x_e, x_e1),
   // sC = (y_e, y_e1, zb_e, zb_e1); (zq, wq) = normalised yaw quaternion of the PRE-reset pose,
   // zb = z_postreset - 0.5
-  // (4-deep ring: the B groups may run ahead of the scan group without an extra hand-shake)
+  // (4-deep ring: the B group may run ahead of the scan group without an extra hand-shake)
   float4 sA[4][A1_TILE / 2];
   float4 sB[4][A1_TILE / 2];
   float4 sC[4][A1_TILE / 2];
@@ -120,70 +79,8 @@ struct alignas(128) V3Smem {
   // accumulates this tile's
   float rterm[2][SHIFU_MAX_REWARD_TERMS][A1_TILE];
   uint64_t full_in[V3_STAGES], e_done[V3_STAGES], b_done[V3_STAGES], h_done[V3_STAGES];
-#ifdef V3_PROFILE
-  long long t_issue[V3_STAGES];
-#endif
 };
 
-// Optional phase timers (-DV3_PROFILE, tools/prof_phases.py): one lead thread per role adds the
-// clock64() cycles it spends in each phase to v3_prof[]; never compiled into the shipped library.
-#ifdef V3_PROFILE
-__device__ unsigned long long v3_prof[32];
-#define V3_T0(lead) const bool _pl = (lead); long long _pt = clock64()
-#define V3_TICK(slot) do { const long long _n = clock64(); if (_pl) atomicAdd(&v3_prof[slot], (unsigned long long)(_n - _pt)); _pt = clock64(); } while (0)
-#define V3_COUNT(slot) do { if (_pl) atomicAdd(&v3_prof[slot], 1ull); } while (0)
-#define V3_STAMP(x) x = clock64()
-#define V3_SINCE(slot, x) do { if (_pl) atomicAdd(&v3_prof[slot], (unsigned long long)(clock64() - (x))); } while (0)
-#else
-#define V3_STAMP(x)
-#define V3_SINCE(slot, x)
-#define V3_T0(lead)
-#define V3_TICK(slot)
-#define V3_COUNT(slot)
-#endif
-
-// dev knobs for the cache behaviour of the table gathers and the obs stores
-#ifndef V3_LD_MODE
-#define V3_LD_MODE 0
-#endif
-#ifndef V3_ST_MODE
-#define V3_ST_MODE 0
-#endif
-__device__ __forceinline__ int v3_gather(const short* p) {
-#ifdef V3_WI_NOGATHER
-  return (int)((unsigned long long)p & 1023);     // what-if: no table access
-#endif
-#if V3_LD_MODE == 0
-  return __ldg(p);
-#elif V3_LD_MODE == 1
-  short v; asm volatile("ld.global.s16 %0, [%1];" : "=h"(v) : "l"(p)); return v;
-#elif V3_LD_MODE == 2
-  short v; asm volatile("ld.global.nc.L1::evict_last.s16 %0, [%1];" : "=h"(v) : "l"(p)); return v;
-#else
-  short v; asm volatile("ld.global.L1::evict_last.s16 %0, [%1];" : "=h"(v) : "l"(p)); return v;
-#endif
-}
-__device__ __forceinline__ void v3_store(float* p, float v) {
-#ifdef V3_WI_NOSTORE
-  if (v == 123.456f) *p = v;      // what-if: keep the value alive, (almost) never store
-  return;
-#endif
-#if V3_ST_MODE == 0
-  __stcs(p, v);
-#elif V3_ST_MODE == 1
-  *p = v;
-#elif V3_ST_MODE == 2
-  __stcg(p, v);
-#else
-  asm volatile("st.global.L1::no_allocate.f32 [%0], %1;" :: "l"(p), "f"(v) : "memory");
-#endif
-}
-
-// what-if: spin for N cycles (dev builds only) to find out which role is on the critical path
-__device__ __forceinline__ void v3_delay(int cycles) {
-  const long long t0 = clock64();
-  while (clock64() - t0 < cycles) { }
-}
 constexpr uint32_t V3_ROW_BYTES = offsetof(V3In, ep_len);
 constexpr uint32_t V3_HIST_BYTES = A1_TILE * A1_DOF * A1_HIST * 4;
 
@@ -193,12 +90,7 @@ __device__ __forceinline__ void v3_issue_hist_load(V3In& in, const ShifuA1StepIO
   pipe::bulk_load(in.hist, io.history + e0 * (A1_DOF * A1_HIST), sizeof(in.hist), bar);
 }
 
-#if V3_SCAN_WARPS == 12 || defined(V3_INLINE)
-#define V3_NOINLINE __forceinline__
-#else
-#define V3_NOINLINE __noinline__
-#endif
-__device__ V3_NOINLINE void v3_issue_loads(V3In& in, const A1K& k, const ShifuA1StepIO& io, long long e0,
+__device__ __forceinline__ void v3_issue_loads(V3In& in, const A1K& k, const ShifuA1StepIO& io, long long e0,
                                                uint64_t* bar, bool with_hist) {
   const uint32_t scalars = sizeof(in.ep_len) + sizeof(in.cla) + k.n_terms * sizeof(in.esum[0]);
   pipe::mbar_arrive_expect_tx(bar, V3_ROW_BYTES + scalars);
@@ -217,8 +109,8 @@ __device__ V3_NOINLINE void v3_issue_loads(V3In& in, const A1K& k, const ShifuA1
 
 // Reward term for env e reading the tile rows of `in` (same arithmetic as a1_eval_term).
 template <bool HAS_EXTRA>
-__device__ V3_NOINLINE float v3_eval_term(int code, int q, float p0, float p1, const A1K& k, const V3In& in, int e,
-                                          const ShifuA1StepIO& io, long long ge) {
+__device__ __forceinline__ float v3_eval_term(int code, int q, float p0, float p1, const A1K& k, const V3In& in, int e,
+                                              const ShifuA1StepIO& io, long long ge) {
   const float* cmd = in.cla[0][e];
   const float* lin = in.cla[1][e];
   const float* ang = in.cla[2][e];
@@ -284,14 +176,7 @@ __global__ void __launch_bounds__(V3_THREADS, V3_CTAS_PER_SM)
 a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io, int num_tiles) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   V3Smem& s = *reinterpret_cast<V3Smem*>(smem_raw);
-#ifdef V3_SCAN_FIRST
-  // warp order scan | B | DMA: the hardware arbiter favours high warp ids, which puts the
-  // latency-critical B group ahead of the throughput-bound scan warps
-  const int t = (threadIdx.x < V3_C_THREADS) ? (int)threadIdx.x + V3_B_THREADS
-              : ((threadIdx.x < V3_C_THREADS + V3_B_THREADS) ? (int)threadIdx.x - V3_C_THREADS : (int)threadIdx.x);
-#else
   const int t = threadIdx.x;
-#endif
   const long long step = (io.step_dev != nullptr) ? *io.step_dev : io.step;
   const int first = blockIdx.x, stride = gridDim.x;
   const int my_tiles = (first < num_tiles) ? (num_tiles - first + stride - 1) / stride : 0;
@@ -313,22 +198,15 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
   if (t >= V3_DMA_BASE && t < V3_DMA_BASE + V3_DMA_THREADS) {
     // ---------------- DMA warp ----------------
     if (t != V3_DMA_BASE) return;
-    for (int j = 0; j < V3_STAGES && j < my_tiles; ++j) {
-      V3_STAMP(s.t_issue[j]);
+    for (int j = 0; j < V3_STAGES && j < my_tiles; ++j)
       v3_issue_loads(s.in[j], k, io, (long long)(first + j * stride) * A1_TILE, &s.full_in[j], true);
-    }
-    V3_T0(true);
     for (int j = 0; j < my_tiles; ++j) {
       const int b = j % V3_STAGES;
       const uint32_t par = (j / V3_STAGES) & 1;
       const long long e0 = (long long)(first + j * stride) * A1_TILE;
       // input rows are dead once the head / history phase is over: store the pushed history and
       // refill the stage right away, long before the tile's height scan finishes
-      V3_WAIT(V3_POLL_DMA, &s.h_done[b], par);
-      V3_TICK(10);
-#ifdef V3_WI_DDELAY
-      v3_delay(V3_WI_DDELAY);
-#endif
+      pipe::mbar_wait<64>(&s.h_done[b], par);
       pipe::bulk_store(io.history + e0 * (A1_DOF * A1_HIST), s.in[b].hist, V3_HIST_BYTES);
       if (io.carry_body_frame) {                              // robot.py:222-229 for the next control step (D7)
         pipe::bulk_store(io.base_lin_vel + e0 * 3, s.in[b].cout[0], sizeof(s.in[b].cout[0]));
@@ -336,40 +214,32 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
         pipe::bulk_store(io.projected_gravity + e0 * 3, s.in[b].cout[2], sizeof(s.in[b].cout[2]));
       }
       pipe::bulk_commit();
-      V3_STAMP(s.t_issue[b]);
       // every other row of the stage is dead already: refill it while the store still reads hist
       const long long en = (long long)(first + (j + V3_STAGES) * stride) * A1_TILE;
       if (j + V3_STAGES < my_tiles) v3_issue_loads(s.in[b], k, io, en, &s.full_in[b], false);
       pipe::bulk_wait_read_all();
       if (j + V3_STAGES < my_tiles) v3_issue_hist_load(s.in[b], io, en, &s.full_in[b]);
-      V3_TICK(11);
-      V3_COUNT(12);
     }
     pipe::bulk_wait_all();                                    // global writes done before exit
     return;
   }
 
   if (t < V3_B_THREADS) {
-    // ---------------- B groups: lane = env ----------------
-    const int g = t / V3_BG_THREADS, tg = t % V3_BG_THREADS;   // group g handles tiles j = g, g+2, ...
-    const int warp = tg >> 5, lane = tg & 31;
-    V3_T0(g == 0 && lane == 0 && warp < 2);
+    // ---------------- B group: lane = env ----------------
+    const int warp = t >> 5, lane = t & 31;
 
-    for (int j = g; j < my_tiles; j += V3_B_GROUPS) {
+    for (int j = 0; j < my_tiles; ++j) {
       const int b = j % V3_STAGES;
       const uint32_t par = (j / V3_STAGES) & 1;
       const long long e0 = (long long)(first + j * stride) * A1_TILE;
       const long long ge = e0 + lane;
       V3In& in = s.in[b];
       const int rb = j & 3;                                   // scalar ring stage (see V3Smem)
-      V3_TICK(warp == 0 ? 0 : 4);
-      V3_WAIT(V3_POLL_B, &s.full_in[b], par);                 // tile rows + per-env scalars have landed
-      if (warp == 1) V3_SINCE(19, s.t_issue[b]);
-      V3_TICK(warp == 0 ? 1 : 5);
+      pipe::mbar_wait<64>(&s.full_in[b], par);                // tile rows + per-env scalars have landed
 
       // ---- B1: yaw normalisation for the scan first (warp 0; the scan group starts its index
-      //          arithmetic as soon as e_done completes), then the reward terms, split over the two
-      //          warps by the host-side cost balance k.term_warp
+      //          arithmetic as soon as e_done completes), then the reward terms, split over the
+      //          B warps by the host-side cost balance k.term_list
       if (warp == 0) {
         // heights are measured at the PRE-reset pose (isaac_gym.py:320-322 runs before post_step)
         const ScanEnv ev = make_scan_env(in.root[lane]);
@@ -385,16 +255,10 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
 #pragma unroll 1
       for (int i = 0; i < k.term_count[warp]; ++i) {
         const int q = k.term_list[warp][i];
-#ifdef V3_WI_NOB1
-        s.rterm[j & 1][q][lane] = 0.0f;
-#else
         s.rterm[j & 1][q][lane] = v3_eval_term<HAS_EXTRA>(k.terms[q], q, k.rp[q][0], k.rp[q][1], k, in, lane, io, ge);
-#endif
       }
-      V3_TICK(warp == 0 ? 2 : 6);
-      pipe::named_barrier(1 + g, V3_BG_THREADS);
-      V3_TICK(warp == 0 ? 3 : 7);
-      if (warp >= 2) continue;                                 // a terms-only warp: on to the next tile's terms
+      pipe::named_barrier(1, V3_B_THREADS);
+      if (warp >= 2) continue;                                // a terms-only warp: on to the next tile's terms
 
       // ---- B2: both warps decide termination (a1_conditional.py:146-150); warp 0 does the ordered
       //          accumulation, flags and episode bookkeeping, warp 1 the state rewrite of resetting envs
@@ -459,13 +323,8 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
         }
         a1_log_sums<1>(k, reset, st_sum, level_delta, lane);
       }
-#ifdef V3_WI_BDELAY
-      v3_delay(V3_WI_BDELAY);
-#endif
       // post-reset rows / command / zb are final: hand the tile to the scan group
       pipe::mbar_arrive(&s.b_done[b]);
-      V3_TICK(warp == 0 ? 13 : 14);
-      V3_COUNT(warp == 0 ? 15 : 31);
     }
     return;
   }
@@ -482,27 +341,7 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
     const f2_t BORDER = pk(k.border, k.border);
     const f2_t RCP = pk(k.hdiv.r, k.hdiv.r), NEGD = pk(-k.hdiv.d, -k.hdiv.d), VS = pk(k.vscale, k.vscale);
     const f2_t NZ = pk(k.neg_zero, k.neg_zero);
-#ifdef V3_ADD_AS_FMA
-    // RN(a + b) == fma(a, 1, b) and RN(a - b) == fma(b, -1, a) exactly
-    const f2_t ONE = pk(k.one, k.one), NEG1 = pk(-k.one, -k.one);
-#define ADD2(a, b) fma2(a, ONE, b)
-#define SUB2(a, b) fma2(b, NEG1, a)
-#define MUL2(a, b) fma2(a, b, NZ)
-#elif defined(V3_ADD_SCALAR)
-    // packed adds split into two scalar adds (the light FMA pipe) — dev experiment
-    auto sadd2 = [](f2_t a, f2_t b) { float a0, a1, b0, b1; upk(a, a0, a1); upk(b, b0, b1); return pk(add_rn(a0, b0), add_rn(a1, b1)); };
-    auto ssub2 = [](f2_t a, f2_t b) { float a0, a1, b0, b1; upk(a, a0, a1); upk(b, b0, b1); return pk(sub_rn(a0, b0), sub_rn(a1, b1)); };
-#define ADD2(a, b) sadd2(a, b)
-#define SUB2(a, b) ssub2(a, b)
-#define MUL2(a, b) mul2(a, b)
-#else
-#define ADD2(a, b) add2(a, b)
-#define SUB2(a, b) sub2(a, b)
-#define MUL2(a, b) mul2(a, b)
-#endif
-#ifndef V3_F2I_CVT
     const f2_t DENORM = pk(__int_as_float(1), __int_as_float(1));     // 2^-149
-#endif
     // Work items of a tile.  The measured-point grid is symmetric about the base (point 186 - pt is
     // -point pt) and round-to-nearest is sign-symmetric, so the yaw rotation of the mirror point is
     // EXACTLY the negated rotation of the point: a lane owns a point AND its mirror and rotates once.
@@ -511,14 +350,12 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
     // point-symmetric to the phased kernel.)
     static_assert(V3_SCAN_WARPS % 3 == 0 && 8 % (V3_SCAN_WARPS / 3) == 0, "scan warps: 3 pair groups x rows");
     constexpr int V3_ITEMS = 8 / (V3_SCAN_WARPS / 3);
-    V3_T0(p == 0);
     for (int j = 0; j < my_tiles; ++j) {
       const int b = j % V3_STAGES;
       const uint32_t par = (j / V3_STAGES) & 1;
       const long long e0 = (long long)(first + j * stride) * A1_TILE;
       const int rb = j & 3;
-      V3_WAIT(V3_POLL_SCAN, &s.e_done[b], par);
-      V3_TICK(16);
+      pipe::mbar_wait<32>(&s.e_done[b], par);
       {
         // item -> (scan point of this lane, first env pair of the batch)
         struct Item { float bx, by; int q0, pt, it; bool live; };
@@ -546,9 +383,8 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
             py0 = min(__float2uint_rz(div_rn(b0, k.hdiv.d)), max_py);
             py1 = min(__float2uint_rz(div_rn(b1, k.hdiv.d)), max_py);
           } else {                         // q0 = x*r; e = fma(-d, q0, x); q = fma(e, r, q0)
-            const f2_t qx = MUL2(ax, RCP), qy = MUL2(ay, RCP);
+            const f2_t qx = mul2(ax, RCP), qy = mul2(ay, RCP);
             const f2_t fx = fma2(fma2(NEGD, qx, ax), RCP, qx), fy = fma2(fma2(NEGD, qy, ay), RCP, qy);
-#ifndef V3_F2I_CVT
             // .long() + clip without the conversion unit: RZ(f * 2^-149) is the denormal whose bit
             // pattern IS trunc(f) for 0 <= f < 2^23 (negative f -> sign bit -> relu -> 0, larger f
             // -> a normal number >= 2^23 -> upper clip); one packed multiply per env pair
@@ -557,12 +393,6 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
             upk_i(mulrz2(fy, DENORM), iy0, iy1);
             px0 = (unsigned)__vimin_s32_relu(ix0, (int)max_px); px1 = (unsigned)__vimin_s32_relu(ix1, (int)max_px);
             py0 = (unsigned)__vimin_s32_relu(iy0, (int)max_py); py1 = (unsigned)__vimin_s32_relu(iy1, (int)max_py);
-#else
-            float fx0, fx1, fy0, fy1;
-            upk(fx, fx0, fx1); upk(fy, fy0, fy1);
-            px0 = min(__float2uint_rz(fx0), max_px); px1 = min(__float2uint_rz(fx1), max_px);
-            py0 = min(__float2uint_rz(fy0), max_py); py1 = min(__float2uint_rz(fy1), max_py);
-#endif
           }
           i0 = ((px0 & ~7u) * c1 + px0) + (py0 << 3);
           i1 = ((px1 & ~7u) * c1 + px1) + (py1 << 3);
@@ -582,18 +412,18 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
             // mul.rn.f32x2 + add.rn.f32x2 into one FFMA2 (single rounding) even under --fmad=false,
             // which flips ~0.3 % of the cell indices; fma(a, b, -0) == RN(a*b) exactly and cannot be
             // contracted again (NZ comes from a kernel parameter, so it is not constant-folded).
-            const f2_t tx = MUL2(Z2, NBY), ty = MUL2(Z2, BX);
-            const f2_t rx = SUB2(ADD2(BX, fma2(W, tx, NZ)), fma2(Z, ty, NZ));
-            const f2_t ry = ADD2(ADD2(BY, fma2(W, ty, NZ)), fma2(Z, tx, NZ));
+            const f2_t tx = mul2(Z2, NBY), ty = mul2(Z2, BX);
+            const f2_t rx = sub2(add2(BX, fma2(W, tx, NZ)), fma2(Z, ty, NZ));
+            const f2_t ry = add2(add2(BY, fma2(W, ty, NZ)), fma2(Z, tx, NZ));
             // + base xy, + border (isaac_gym.py:416-420)
-            cell_pair(ADD2(ADD2(rx, X), BORDER), ADD2(ADD2(ry, Y), BORDER), idx[4 * u], idx[4 * u + 1]);
+            cell_pair(add2(add2(rx, X), BORDER), add2(add2(ry, Y), BORDER), idx[4 * u], idx[4 * u + 1]);
             // the mirror point: rotation = (-rx, -ry) exactly, and RN(-r + X) == RN(X - r)
-            cell_pair(ADD2(SUB2(X, rx), BORDER), ADD2(SUB2(Y, ry), BORDER), idx[4 * u + 2], idx[4 * u + 3]);
+            cell_pair(add2(sub2(X, rx), BORDER), add2(sub2(Y, ry), BORDER), idx[4 * u + 2], idx[4 * u + 3]);
           }
         };
         auto load_batch = [&](const unsigned (&idx)[8], int (&h)[8]) {
 #pragma unroll
-          for (int u = 0; u < 8; ++u) h[u] = v3_gather(table + idx[u]);      // isaac_gym.py:427-431 (folded)
+          for (int u = 0; u < 8; ++u) h[u] = __ldg(table + idx[u]);          // isaac_gym.py:427-431 (folded)
         };
         auto store_batch = [&](const Item& w, const int (&h)[8]) {
           float* ob = io.obs_buf + (e0 + 2 * w.q0) * A1_OBS + A1_HEAD + w.pt;
@@ -602,9 +432,9 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           auto emit = [&](float2 zb, int h0, int h1, float* o, float* m) {
             const f2_t hg2 = fma2(pk((float)h0, (float)h1), VS, NZ);            // * vertical_scale, :433
             float v0, v1;
-            upk(SUB2(pk(zb.x, zb.y), hg2), v0, v1);                             // a1_conditional.py:132
-            v3_store(o, clampf(v0, -hclip, hclip));
-            v3_store(o + A1_OBS, clampf(v1, -hclip, hclip));
+            upk(sub2(pk(zb.x, zb.y), hg2), v0, v1);                             // a1_conditional.py:132
+            __stcs(o, clampf(v0, -hclip, hclip));
+            __stcs(o + A1_OBS, clampf(v1, -hclip, hclip));
             if (HAS_MROW) {
               float g0, g1;
               upk(hg2, g0, g1);
@@ -630,14 +460,10 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
         unsigned idx[8];
         int h[8];    // sign-extended int16 cells
         Item cur = item(0);
-#ifndef V3_WI_NOSCAN
         index_batch(cur, idx);
         load_batch(idx, h);
-#endif
         // ---- obs head (a1_conditional.py:131-144) + history push (train.py:12-14): post-reset rows
-        V3_TICK(20);
-        V3_WAIT(V3_POLL_SCAN, &s.b_done[b], par);
-        V3_TICK(8);
+        pipe::mbar_wait<32>(&s.b_done[b], par);
         {
           // One (env, dof) item and one (env, column) item per thread.  Everything the head reads from the
           // stage is loaded FIRST and the history is pushed, then the stage is handed back (fence + arrive),
@@ -656,25 +482,15 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           in.hist[e][d * A1_HIST + 2] = a1;              // HistoryRecorder.add (train.py:12-14)
           in.hist[e][d * A1_HIST + 1] = a0;
           in.hist[e][d * A1_HIST + 0] = in.act[e][d];
-          V3_TICK(21);
           pipe::fence_proxy_async();                            // pushed history -> visible to the TMA store
           pipe::mbar_arrive(&s.h_done[b]);
-          V3_TICK(9);
-#ifndef V3_WI_NOHEAD
-#define V3_HEAD_ST(ptr, v) __stcs(ptr, v)
-          V3_HEAD_ST(hrow + d, clampf(v, -c, c));
-          V3_HEAD_ST(hrow + 12 + d, clampf(sub_rn(qd.x, k.q0[d]), -c, c));
-          V3_HEAD_ST(hrow + 24 + d, clampf(qd.y, -c, c));
-          V3_HEAD_ST(hrow + 36 + d, clampf(a0, -c, c));         // HistoryRecorder.flatten: slot-major
-          V3_HEAD_ST(hrow + 48 + d, clampf(a1, -c, c));
-          V3_HEAD_ST(hrow + 60 + d, clampf(a2, -c, c));
-#endif
-          V3_TICK(22);
+          __stcs(hrow + d, clampf(v, -c, c));
+          __stcs(hrow + 12 + d, clampf(sub_rn(qd.x, k.q0[d]), -c, c));
+          __stcs(hrow + 24 + d, clampf(qd.y, -c, c));
+          __stcs(hrow + 36 + d, clampf(a0, -c, c));             // HistoryRecorder.flatten: slot-major
+          __stcs(hrow + 48 + d, clampf(a1, -c, c));
+          __stcs(hrow + 60 + d, clampf(a2, -c, c));
         }
-#ifdef V3_WI_SDELAY
-        v3_delay(V3_WI_SDELAY);
-#endif
-#ifndef V3_WI_NOSCAN
 #pragma unroll 1
         for (int it = 1; it < V3_ITEMS; ++it) {
           const Item nxt = item(it);
@@ -684,10 +500,7 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           cur = nxt;
         }
         store_batch(cur, h);
-#endif
       }
-      V3_TICK(17);
-      V3_COUNT(18);
     }
   }
 }

@@ -84,22 +84,6 @@ static const void* const* a1_tma_variants() {
 extern "C" const char* shifu_last_error(void) { return g_err; }
 extern "C" int shifu_abi_version(void) { return SHIFU_ABI_VERSION; }
 
-#ifdef V3_DEV
-#include "dev_scan_only.cuh"
-#endif
-#ifdef V3_PROFILE
-// dev-only (tools/prof_phases.py): read and optionally clear the fused kernel's phase timers
-extern "C" int shifu_debug_profile(unsigned long long* out, int reset) {
-  cudaDeviceSynchronize();
-  cudaError_t e = cudaMemcpyFromSymbol(out, shifu::v3_prof, sizeof(unsigned long long) * 32);
-  if (e == cudaSuccess && reset) {
-    unsigned long long z[32] = {};
-    e = cudaMemcpyToSymbol(shifu::v3_prof, z, sizeof(z));
-  }
-  return (int)e;
-}
-#endif
-
 // Largest float s with sqrtf(s) <= thr (sqrtf is correctly rounded and monotonic), so that
 // "sqrt_rn(s) > thr" can be tested as "s > sqrt_threshold(thr)" with identical results.
 static float sqrt_threshold(float thr) {
@@ -110,12 +94,6 @@ static float sqrt_threshold(float thr) {
   return s;
 }
 
-#ifndef V3_LOAD0
-#define V3_LOAD0 215
-#endif
-#ifndef V3_LOAD1
-#define V3_LOAD1 160
-#endif
 static int fill_a1k(const ShifuA1Desc& d, A1K& k) {
   if (d.abi_version != SHIFU_ABI_VERSION) return fail(SHIFU_E_RANGE, "ShifuA1Desc.abi_version %d != %d", d.abi_version, SHIFU_ABI_VERSION);
   if (d.num_envs <= 0) return fail(SHIFU_E_RANGE, "num_envs must be > 0 (got %d)", d.num_envs);
@@ -163,7 +141,7 @@ static int fill_a1k(const ShifuA1Desc& d, A1K& k) {
   k.xy_span = (float)((double)d.reset_xy_range - (double)(-d.reset_xy_range)); k.xy_low = -d.reset_xy_range;
   k.force_span = (float)((double)d.push_force_max - (double)(-d.push_force_max)); k.force_low = -d.push_force_max;
   for (int i = 0; i < 3; ++i) { k.cmd_span[i] = (float)((double)d.cmd_high[i] - (double)d.cmd_low[i]); k.cmd_low[i] = d.cmd_low[i]; }
-  k.neg_zero = -0.0f; k.one = 1.0f;
+  k.neg_zero = -0.0f;
   k.curriculum = d.curriculum; k.max_level = d.max_terrain_level; k.n_types = d.num_terrain_types;
   k.up_dist = d.level_up_distance; k.down_factor = d.level_down_factor;
   k.n_terms = d.num_reward_terms;
@@ -190,12 +168,11 @@ static int fill_a1k(const ShifuA1Desc& d, A1K& k) {
   static const int term_cost[SHIFU_REW_COUNT] = {30, 25, 12, 135, 70, 40, 20, 20, 8, 10, 10, 40, 60, 8, 70, 90};
   // longest-processing-time split of the term list over the B warps of the pipelined kernel.  Warp 0
   // starts loaded with the yaw normalisation it does first (~115 on the scale of term_cost, from the
-  // phase timers); with terms-only warps present, warps 0 and 1 also carry their B2 halves (~100
-  // and ~160 with the carried body-frame rows), which a terms-only warp overlaps with the next tile's
-  // terms.  The preloads were tuned on the B200 (profiles/README.md: a dozen other splits of the
-  // reference's six terms are 0.5-8 % slower).
-  int load[A1K_TERM_WARPS] = {0}, order[SHIFU_MAX_REWARD_TERMS];
-  load[0] = V3_BG_WARPS > 2 ? V3_LOAD0 : 60; load[1] = V3_BG_WARPS > 2 ? V3_LOAD1 : 0;
+  // phase timers); warps 0 and 1 also carry their B2 halves (~100 and ~160 with the carried
+  // body-frame rows), which the terms-only warp 2 overlaps with the next tile's terms.  The preloads
+  // were tuned on the B200 (profiles/README.md: a dozen other splits of the reference's six terms
+  // are 0.5-8 % slower).
+  int load[A1K_TERM_WARPS] = {215, 160, 0, 0}, order[SHIFU_MAX_REWARD_TERMS];
   for (int i = 0; i < k.n_terms; ++i) order[i] = i;
   auto cost_of = [&](int q) { const int c = k.terms[q]; return (c >= 0 && c < SHIFU_REW_COUNT) ? term_cost[c] : 40; };
   for (int i = 0; i < k.n_terms; ++i)
@@ -316,7 +293,6 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
       carve = (int)((need * 100 + smem_sm - 1) / smem_sm);
       if (carve > 100) carve = 100;
     }
-    if (getenv("SHIFU_CARVEOUT") != nullptr) carve = atoi(getenv("SHIFU_CARVEOUT"));
     for (int v = 0; v < 8 && e == cudaSuccess; ++v) {
       e = cudaFuncSetAttribute(tma_variants[v], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(V3Smem));
       if (e == cudaSuccess)
@@ -448,22 +424,6 @@ extern "C" int shifu_a1_eval_terms(ShifuCtx* c, const ShifuA1StepIO* io, float* 
   CUDA_TRY(cudaGetLastError());
   return SHIFU_OK;
 }
-
-#ifdef V3_DEV
-extern "C" int shifu_debug_scan_only(ShifuCtx* c, const float* root, float* obs, int mode, int ctas_per_sm, int threads,
-                                     void* stream) {
-  const int tiles = c->a1.num_envs / A1_TILE;
-  const int grid = c->sm_count * ctas_per_sm;
-  const int np = (mode >> 8) & 15;      // pairs per batch: 2, 4 or 8
-  mode &= 255;
-#define DEV_LAUNCH(T, P) dev_scan_only_kernel<T, P><<<grid, T, 0, S(stream)>>>(c->a1k, root, obs, tiles, mode)
-  if (threads == 192) { if (np == 8) DEV_LAUNCH(192, 8); else if (np == 2) DEV_LAUNCH(192, 2); else DEV_LAUNCH(192, 4); }
-  else if (threads == 384) { if (np == 8) DEV_LAUNCH(384, 8); else if (np == 2) DEV_LAUNCH(384, 2); else DEV_LAUNCH(384, 4); }
-  else { if (np == 8) DEV_LAUNCH(768, 8); else DEV_LAUNCH(768, 4); }
-  CUDA_TRY(cudaGetLastError());
-  return SHIFU_OK;
-}
-#endif
 
 extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void* stream) {
   REQUIRE_PTR(c); REQUIRE_PTR(io);

@@ -56,23 +56,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
-// Same, but the waiting warp is parked by the hardware for up to `hint_ns` per attempt (no polling
-// instructions while parked); it wakes as soon as the phase completes.
-__device__ __forceinline__ void mbar_wait_parked(uint64_t* bar, uint32_t parity, uint32_t hint_ns) {
-  const uint32_t addr = smem_u32(bar);
-  uint32_t done = 0;
-  for (uint32_t spin = 0; !done; ++spin) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity), "r"(hint_ns)
-        : "memory");
-    if (!done && spin > (1u << 22)) __trap();
-  }
-}
-
 // global -> shared bulk copy, completion signalled on an mbarrier (bytes % 16 == 0, 16-B aligned)
 __device__ __forceinline__ void bulk_load(void* smem_dst, const void* gmem_src, uint32_t bytes, uint64_t* bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
