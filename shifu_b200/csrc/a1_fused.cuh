@@ -28,7 +28,7 @@ struct A1Smem {
   float act[A1_TILE][A1_DOF];
   float head[A1_TILE][A1_HEAD];
   float rterm[SHIFU_MAX_REWARD_TERMS][A1_TILE];   // reward term values, [term][env]
-  float cla[A1_TILE][9];                            // command(3, post-reset), lin vel(3), ang vel(3)
+  float cla[3][A1_TILE][3];                         // command (post-reset), base lin vel, base ang vel
   float4 ev[A1_TILE];                               // (2*zq, zq, wq, unused) of the PRE-reset pose
   float4 pos[A1_TILE];                              // (x + 0, y + 0, zb = z_postreset - 0.5, unused)
 };
@@ -60,8 +60,29 @@ __device__ __forceinline__ void store_span(float* __restrict__ dst, const float*
   }
 }
 
-// One reward term for env e (lane = env).  a1_conditional.py:162-192; every op rounds like the
-// aten elementwise op it stands for.
+// Staging of phase A: the tile's root / dof / contact / history / torque / action rows -> shared memory.
+__device__ __forceinline__ void a1_stage_rows(A1Smem& s, const A1K& k, const ShifuA1StepIO& io, int e0, int ne, int t) {
+  if (k.root_stride == 1 && k.root_offset == 0) {
+    load_span(&s.root[0][0], io.root_state + (long long)e0 * 13, ne * 13, t, A1_THREADS);
+  } else {
+    for (int i = t; i < ne * 13; i += A1_THREADS) {
+      const int e = i / 13, c = i % 13;
+      s.root[e][c] = io.root_state[((long long)(e0 + e) * k.root_stride + k.root_offset) * 13 + c];
+    }
+  }
+  load_span(&s.dof[0][0], io.dof_state + (long long)e0 * (A1_DOF * 2), ne * A1_DOF * 2, t, A1_THREADS);
+  load_span(&s.contact[0][0], io.contact_state + (long long)e0 * (A1_BODIES * 3), ne * A1_BODIES * 3, t, A1_THREADS);
+  load_span(&s.hist[0][0], io.history + (long long)e0 * (A1_DOF * A1_HIST), ne * A1_DOF * A1_HIST, t, A1_THREADS);
+  load_span(&s.tau[0][0], io.torques + (long long)e0 * A1_DOF, ne * A1_DOF, t, A1_THREADS);
+  load_span(&s.act[0][0], io.actions + (long long)e0 * A1_DOF, ne * A1_DOF, t, A1_THREADS);
+}
+
+// |f| > thr for a force row f, tested as "sum of squares > thr_sq" with thr_sq = sqrt_threshold(thr)
+// from the host: sqrt_rn is correctly rounded and monotonic, so this equals norm3_fma(f) > thr exactly.
+__device__ __forceinline__ bool force_exceeds(const float* f, float thr_sq) {
+  return fma_rn(f[2], f[2], fma_rn(f[1], f[1], mul_rn(f[0], f[0]))) > thr_sq;
+}
+
 // Terms 8-15 (legged_gym-style, see enum ShifuRewardTerm).  Everything a term may read for one env:
 struct TermCtx {
   const float *cmd, *lin, *ang, *pg;      // command, body-frame velocities, projected gravity (this step's)
@@ -129,36 +150,44 @@ __device__ __noinline__ float a1_extra_term(int code, float p0, float p1, const 
   }
 }
 
-__device__ __noinline__ float a1_eval_term(int code, float p0, float p1, const A1K& k, const A1Smem& s, int e,
-                                           const ShifuA1StepIO& io, long long ge) {
-  const float* cla = s.cla[e];
-  if (code >= SHIFU_REW_LIN_VEL_Z) {
-    const TermCtx c{cla, cla + 3, cla + 6, io.projected_gravity + ge * 3, s.dof[e], s.hist[e], s.act[e], s.contact[e],
-                    s.root[e][2], io.swing_time ? io.swing_time + ge * k.n_feet : nullptr,
+// One reward term for env e of a staged tile: V3In (pipelined kernel) or A1Smem (phased and eval-terms
+// kernels), which both hold root / dof / contact / hist / tau / act rows and cla = command, base lin vel,
+// base ang vel.  a1_conditional.py:162-192; every op rounds like the aten elementwise op it stands for.
+// Two forms restate the reference exactly: x / p1 is RN(x * rp_inv) when p1 is a power of two (1/p1 is
+// then exact), and the leg-force norm test is force_exceeds.
+// HAS_EXTRA: the term list may hold a code >= SHIFU_REW_LIN_VEL_Z.
+template <bool HAS_EXTRA, class Tile>
+__device__ __forceinline__ float a1_reward_term(int code, int q, float p0, float p1, const A1K& k, const Tile& in, int e,
+                                                const ShifuA1StepIO& io, long long ge) {
+  const float* cmd = in.cla[0][e];
+  const float* lin = in.cla[1][e];
+  const float* ang = in.cla[2][e];
+  if (HAS_EXTRA && code >= SHIFU_REW_LIN_VEL_Z) {   // legged_gym-style terms: pg / air-time state straight from global memory
+    const TermCtx c{cmd, lin, ang, io.projected_gravity + ge * 3, in.dof[e], in.hist[e], in.act[e], in.contact[e],
+                    in.root[e][2], io.swing_time ? io.swing_time + ge * k.n_feet : nullptr,
                     io.last_contacts ? io.last_contacts + ge * k.n_feet : nullptr};
     return a1_extra_term(code, p0, p1, k, c);
   }
   switch (code) {
     case SHIFU_REW_TRACKING_LIN_VEL: {
-      const float dx = sub_rn(cla[0], cla[3]), dy = sub_rn(cla[1], cla[4]);
-      const float err = add_rn(mul_rn(dx, dx), mul_rn(dy, dy));
-      return mul_rn(p0, expf(div_rn(-err, p1)));
+      const float dx = sub_rn(cmd[0], lin[0]), dy = sub_rn(cmd[1], lin[1]);
+      const float ne = -add_rn(mul_rn(dx, dx), mul_rn(dy, dy));
+      return mul_rn(p0, expf(k.rp_pow2[q] ? mul_rn(ne, k.rp_inv[q]) : div_rn(ne, p1)));
     }
     case SHIFU_REW_TRACKING_ANG_VEL: {
-      const float d = sub_rn(cla[2], cla[8]);
-      return mul_rn(p0, expf(div_rn(-mul_rn(d, d), p1)));
+      const float d = sub_rn(cmd[2], ang[2]);
+      const float ne = -mul_rn(d, d);
+      return mul_rn(p0, expf(k.rp_pow2[q] ? mul_rn(ne, k.rp_inv[q]) : div_rn(ne, p1)));
     }
-    case SHIFU_REW_STABILIZING_BASE: {
-      const float zv = mul_rn(p0, mul_rn(cla[5], cla[5]));
-      const float av = mul_rn(p1, add_rn(mul_rn(cla[6], cla[6]), mul_rn(cla[7], cla[7])));
-      return add_rn(zv, av);
-    }
+    case SHIFU_REW_STABILIZING_BASE:
+      return add_rn(mul_rn(p0, mul_rn(lin[2], lin[2])),
+                    mul_rn(p1, add_rn(mul_rn(ang[0], ang[0]), mul_rn(ang[1], ang[1]))));
     case SHIFU_REW_SMOOTHING_ACTION: {
       float f1 = 0.0f, f2 = 0.0f;
 #pragma unroll
       for (int d = 0; d < A1_DOF; ++d) {
-        const float a0 = s.hist[e][d * A1_HIST + 0], a1 = s.hist[e][d * A1_HIST + 1],
-                    a2 = s.hist[e][d * A1_HIST + 2];
+        const float a0 = in.hist[e][d * A1_HIST + 0], a1 = in.hist[e][d * A1_HIST + 1],
+                    a2 = in.hist[e][d * A1_HIST + 2];
         const float d1 = sub_rn(a1, a0);
         const float d2 = add_rn(sub_rn(a2, mul_rn(2.0f, a1)), a0);
         f1 = add_rn(f1, mul_rn(d1, d1));
@@ -168,21 +197,25 @@ __device__ __noinline__ float a1_eval_term(int code, float p0, float p1, const A
     }
     case SHIFU_REW_LEG_COLLISION: {
       int cnt = 0;
-      for (int b = 0; b < k.n_leg; ++b) {
-        const float* f = &s.contact[e][k.leg[b] * 3];
-        cnt += (norm3_fma(f[0], f[1], f[2]) > p1) ? 1 : 0;
-      }
+      for (int b = 0; b < k.n_leg; ++b)   // rolled on purpose: unrolled, the pipelined kernel's B warps spill (0.4376 vs 0.4289 ms)
+        cnt += force_exceeds(&in.contact[e][k.leg[b] * 3], k.rp_thr_sq[q]) ? 1 : 0;
       return mul_rn(p0, (float)cnt);
     }
     case SHIFU_REW_TORQUES: {
       float acc = 0.0f;
 #pragma unroll
-      for (int d = 0; d < A1_DOF; ++d) acc = add_rn(acc, mul_rn(s.tau[e][d], s.tau[e][d]));
+      for (int d = 0; d < A1_DOF; ++d) acc = add_rn(acc, mul_rn(in.tau[e][d], in.tau[e][d]));
       return mul_rn(p0, acc);
     }
     default:
       return 0.0f;
   }
+}
+
+// Term q of the descriptor's list, out of line: the phased and eval-terms kernels call it from a rolled loop.
+__device__ __noinline__ float a1_eval_term(int q, const A1K& k, const A1Smem& s, int e, const ShifuA1StepIO& io,
+                                           long long ge) {
+  return a1_reward_term<true>(k.terms[q], q, k.rp[q][0], k.rp[q][1], k, s, e, io, ge);
 }
 
 template <bool TILED, bool EXACT_DIV>
@@ -216,24 +249,10 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
 #pragma unroll
       for (int j = 0; j < SHIFU_MAX_REWARD_TERMS; ++j) esum[j] = (j < k.n_terms) ? io.ep_sums[j][ge] : 0.0f;
     }
-    if (k.root_stride == 1 && k.root_offset == 0) {
-      load_span(&s.root[0][0], io.root_state + (long long)e0 * 13, ne * 13, t, A1_THREADS);
-    } else {
-      for (int i = t; i < ne * 13; i += A1_THREADS) {
-        const int e = i / 13, c = i % 13;
-        s.root[e][c] = io.root_state[((long long)(e0 + e) * k.root_stride + k.root_offset) * 13 + c];
-      }
-    }
-    load_span(&s.dof[0][0], io.dof_state + (long long)e0 * (A1_DOF * 2), ne * A1_DOF * 2, t, A1_THREADS);
-    load_span(&s.contact[0][0], io.contact_state + (long long)e0 * (A1_BODIES * 3), ne * A1_BODIES * 3, t,
-              A1_THREADS);
-    load_span(&s.hist[0][0], io.history + (long long)e0 * (A1_DOF * A1_HIST), ne * A1_DOF * A1_HIST, t,
-              A1_THREADS);
-    load_span(&s.tau[0][0], io.torques + (long long)e0 * A1_DOF, ne * A1_DOF, t, A1_THREADS);
-    load_span(&s.act[0][0], io.actions + (long long)e0 * A1_DOF, ne * A1_DOF, t, A1_THREADS);
+    a1_stage_rows(s, k, io, e0, ne, t);
     if (warp == 0 && lane_env) {
 #pragma unroll
-      for (int j = 0; j < 9; ++j) s.cla[lane][j] = c9[j];
+      for (int j = 0; j < 9; ++j) s.cla[j / 3][lane][j % 3] = c9[j];
     }
     __syncthreads();
 
@@ -241,12 +260,9 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
     bool contact_term = false;
     if (lane_env) {
 #pragma unroll 1
-      for (int j = warp; j < k.n_terms; j += A1_THREADS / 32)
-        s.rterm[j][lane] = a1_eval_term(k.terms[j], k.rp[j][0], k.rp[j][1], k, s, lane, io, ge);
-      if (warp == 0) {                                                  // a1_conditional.py:146-148
-        const float* fb = &s.contact[lane][k.base_body * 3];
-        contact_term = norm3_fma(fb[0], fb[1], fb[2]) > k.contact_thr;
-      }
+      for (int j = warp; j < k.n_terms; j += A1_THREADS / 32) s.rterm[j][lane] = a1_eval_term(j, k, s, lane, io, ge);
+      if (warp == 0)                                                    // a1_conditional.py:146-148
+        contact_term = force_exceeds(&s.contact[lane][k.base_body * 3], k.contact_thr_sq);
       if (warp == 5) {
         // heights are measured at the PRE-reset pose (isaac_gym.py:320-322 runs before post_step)
         const ScanEnv ev = make_scan_env(s.root[lane]);
@@ -282,12 +298,12 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
         io.time_out_buf[ge] = time_out ? 1 : 0;
         io.contact_term_buf[ge] = contact_term ? 1 : 0;
         if (reset) {                                                       // env.py:101-102
-          float cmd[3] = {s.cla[lane][0], s.cla[lane][1], s.cla[lane][2]};
+          float cmd[3] = {s.cla[0][lane][0], s.cla[0][lane][1], s.cla[0][lane][2]};
           a1_reset_env<true>(k, io, step, ge, s.root[lane], s.dof[lane], s.hist[lane], cmd, esum, len, st_sum,
                              level_delta, io.env_origins[ge * 3LL + 0], io.env_origins[ge * 3LL + 1],
                              io.env_origins[ge * 3LL + 2], k.curriculum ? io.terrain_levels[ge] : 0,
                              k.curriculum ? io.terrain_types[ge] : 0);
-          s.cla[lane][0] = cmd[0]; s.cla[lane][1] = cmd[1]; s.cla[lane][2] = cmd[2];
+          s.cla[0][lane][0] = cmd[0]; s.cla[0][lane][1] = cmd[1]; s.cla[0][lane][2] = cmd[2];
         }
         io.ep_len[ge] = len;
 #pragma unroll
@@ -320,7 +336,7 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
       // (env, j < 12): command, body-frame velocities, gravity_vec
       for (int i = t; i < ne * 12; i += A1_THREADS) {
         const int e = i / 12, j = i - e * 12;
-        const float v = (j < 9) ? s.cla[e][j] : ((j == 11) ? -1.0f : 0.0f);
+        const float v = (j < 9) ? s.cla[j / 3][e][j % 3] : ((j == 11) ? -1.0f : 0.0f);
         s.head[e][j] = clampf(v, -c, c);
       }
       // carried body-frame velocities for the next control step (robot.py:222-229, D7)
@@ -400,27 +416,19 @@ a1_eval_terms_kernel(const __grid_constant__ A1K k, const __grid_constant__ Shif
     const int ne = min(A1_TILE, k.n - e0);
     const int ge = e0 + lane;
     __syncthreads();
-    for (int i = t; i < ne * 13; i += A1_THREADS) {
-      const int e = i / 13, c = i % 13;
-      s.root[e][c] = io.root_state[((long long)(e0 + e) * k.root_stride + k.root_offset) * 13 + c];
-    }
-    load_span(&s.dof[0][0], io.dof_state + (long long)e0 * (A1_DOF * 2), ne * A1_DOF * 2, t, A1_THREADS);
-    load_span(&s.contact[0][0], io.contact_state + (long long)e0 * (A1_BODIES * 3), ne * A1_BODIES * 3, t, A1_THREADS);
-    load_span(&s.hist[0][0], io.history + (long long)e0 * (A1_DOF * A1_HIST), ne * A1_DOF * A1_HIST, t, A1_THREADS);
-    load_span(&s.tau[0][0], io.torques + (long long)e0 * A1_DOF, ne * A1_DOF, t, A1_THREADS);
-    load_span(&s.act[0][0], io.actions + (long long)e0 * A1_DOF, ne * A1_DOF, t, A1_THREADS);
+    a1_stage_rows(s, k, io, e0, ne, t);
     if (warp == 0 && lane < ne) {
 #pragma unroll
       for (int j = 0; j < 3; ++j) {
-        s.cla[lane][j] = io.command[ge * 3LL + j];
-        s.cla[lane][3 + j] = io.base_lin_vel[ge * 3LL + j];
-        s.cla[lane][6 + j] = io.base_ang_vel[ge * 3LL + j];
+        s.cla[0][lane][j] = io.command[ge * 3LL + j];
+        s.cla[1][lane][j] = io.base_lin_vel[ge * 3LL + j];
+        s.cla[2][lane][j] = io.base_ang_vel[ge * 3LL + j];
       }
     }
     __syncthreads();
     if (lane < ne)
-      for (int j = warp; j < k.n_terms; j += A1_THREADS / 32)
-        out[(long long)j * k.n + ge] = a1_eval_term(k.terms[j], k.rp[j][0], k.rp[j][1], k, s, lane, io, ge);
+#pragma unroll 1
+      for (int j = warp; j < k.n_terms; j += A1_THREADS / 32) out[(long long)j * k.n + ge] = a1_eval_term(j, k, s, lane, io, ge);
   }
 }
 

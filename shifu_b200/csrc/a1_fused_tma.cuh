@@ -30,7 +30,7 @@
 // travel through a 4-deep ring, which lets the B group run ahead of the scan group.
 #pragma once
 #include "a1_fused.cuh"
-#include "f32x2.cuh"
+#include "scan_pairs.cuh"
 #include "tma_pipe.cuh"
 
 namespace shifu {
@@ -105,66 +105,6 @@ __device__ __forceinline__ void v3_issue_loads(V3In& in, const A1K& k, const Shi
   pipe::bulk_load(in.cla[1], io.base_lin_vel + e0 * 3, sizeof(in.cla[1]), bar);
   pipe::bulk_load(in.cla[2], io.base_ang_vel + e0 * 3, sizeof(in.cla[2]), bar);
   for (int q = 0; q < k.n_terms; ++q) pipe::bulk_load(in.esum[q], io.ep_sums[q] + e0, sizeof(in.esum[q]), bar);
-}
-
-// Reward term for env e reading the tile rows of `in` (same arithmetic as a1_eval_term).
-template <bool HAS_EXTRA>
-__device__ __forceinline__ float v3_eval_term(int code, int q, float p0, float p1, const A1K& k, const V3In& in, int e,
-                                              const ShifuA1StepIO& io, long long ge) {
-  const float* cmd = in.cla[0][e];
-  const float* lin = in.cla[1][e];
-  const float* ang = in.cla[2][e];
-  if (HAS_EXTRA && code >= SHIFU_REW_LIN_VEL_Z) {   // legged_gym-style terms: pg / air-time state straight from global memory
-    const TermCtx c{cmd, lin, ang, io.projected_gravity + ge * 3, in.dof[e], in.hist[e], in.act[e], in.contact[e],
-                    in.root[e][2], io.swing_time ? io.swing_time + ge * k.n_feet : nullptr,
-                    io.last_contacts ? io.last_contacts + ge * k.n_feet : nullptr};
-    return a1_extra_term(code, p0, p1, k, c);
-  }
-  switch (code) {
-    case SHIFU_REW_TRACKING_LIN_VEL: {
-      const float dx = sub_rn(cmd[0], lin[0]), dy = sub_rn(cmd[1], lin[1]);
-      const float ne = -add_rn(mul_rn(dx, dx), mul_rn(dy, dy));
-      return mul_rn(p0, expf(k.rp_pow2[q] ? mul_rn(ne, k.rp_inv[q]) : div_rn(ne, p1)));
-    }
-    case SHIFU_REW_TRACKING_ANG_VEL: {
-      const float d = sub_rn(cmd[2], ang[2]);
-      const float ne = -mul_rn(d, d);
-      return mul_rn(p0, expf(k.rp_pow2[q] ? mul_rn(ne, k.rp_inv[q]) : div_rn(ne, p1)));
-    }
-    case SHIFU_REW_STABILIZING_BASE:
-      return add_rn(mul_rn(p0, mul_rn(lin[2], lin[2])),
-                    mul_rn(p1, add_rn(mul_rn(ang[0], ang[0]), mul_rn(ang[1], ang[1]))));
-    case SHIFU_REW_SMOOTHING_ACTION: {
-      float f1 = 0.0f, f2 = 0.0f;
-#pragma unroll
-      for (int d = 0; d < A1_DOF; ++d) {
-        const float a0 = in.hist[e][d * A1_HIST + 0], a1 = in.hist[e][d * A1_HIST + 1],
-                    a2 = in.hist[e][d * A1_HIST + 2];
-        const float d1 = sub_rn(a1, a0);
-        const float d2 = add_rn(sub_rn(a2, mul_rn(2.0f, a1)), a0);
-        f1 = add_rn(f1, mul_rn(d1, d1));
-        f2 = add_rn(f2, mul_rn(d2, d2));
-      }
-      return mul_rn(p0, add_rn(f1, f2));
-    }
-    case SHIFU_REW_LEG_COLLISION: {
-      int cnt = 0;
-      for (int b = 0; b < k.n_leg; ++b) {   // rolled on purpose: unrolled, the B warps spill (0.4376 vs 0.4289 ms)
-        const float* f = &in.contact[e][k.leg[b] * 3];
-        // |F| > p1 tested on the sum of squares (threshold pre-squared exactly on the host)
-        cnt += (fma_rn(f[2], f[2], fma_rn(f[1], f[1], mul_rn(f[0], f[0]))) > k.rp_thr_sq[q]) ? 1 : 0;
-      }
-      return mul_rn(p0, (float)cnt);
-    }
-    case SHIFU_REW_TORQUES: {
-      float acc = 0.0f;
-#pragma unroll
-      for (int d = 0; d < A1_DOF; ++d) acc = add_rn(acc, mul_rn(in.tau[e][d], in.tau[e][d]));
-      return mul_rn(p0, acc);
-    }
-    default:
-      return 0.0f;
-  }
 }
 
 // Processes tiles [0, num_tiles) of 32 envs each (the ragged tail, if any, is a separate launch of
@@ -242,20 +182,13 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
       //          B warps by the host-side cost balance k.term_list
       if (warp == 0) {
         // heights are measured at the PRE-reset pose (isaac_gym.py:320-322 runs before post_step)
-        const ScanEnv ev = make_scan_env(in.root[lane]);
-        const int q = lane >> 1, sl = lane & 1;
-        float* a = reinterpret_cast<float*>(&s.sA[rb][q]);
-        float* bb = reinterpret_cast<float*>(&s.sB[rb][q]);
-        float* cc = reinterpret_cast<float*>(&s.sC[rb][q]);
-        a[sl] = ev.z2; a[2 + sl] = ev.z;
-        bb[sl] = ev.w; bb[2 + sl] = ev.x;
-        cc[sl] = ev.y;
+        publish_scan_env(make_scan_env(in.root[lane]), lane, s.sA[rb], s.sB[rb], s.sC[rb]);
         pipe::mbar_arrive(&s.e_done[b]);
       }
 #pragma unroll 1
       for (int i = 0; i < k.term_count[warp]; ++i) {
         const int q = k.term_list[warp][i];
-        s.rterm[j & 1][q][lane] = v3_eval_term<HAS_EXTRA>(k.terms[q], q, k.rp[q][0], k.rp[q][1], k, in, lane, io, ge);
+        s.rterm[j & 1][q][lane] = a1_reward_term<HAS_EXTRA>(k.terms[q], q, k.rp[q][0], k.rp[q][1], k, in, lane, io, ge);
       }
       pipe::named_barrier(1, V3_B_THREADS);
       if (warp >= 2) continue;                                // a terms-only warp: on to the next tile's terms
@@ -263,8 +196,7 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
       // ---- B2: both warps decide termination (a1_conditional.py:146-150); warp 0 does the ordered
       //          accumulation, flags and episode bookkeeping, warp 1 the state rewrite of resetting envs
       long long len = in.ep_len[lane] + 1;                                 // env.py:95
-      const float* fb = &in.contact[lane][k.base_body * 3];
-      const bool contact_term = fma_rn(fb[2], fb[2], fma_rn(fb[1], fb[1], mul_rn(fb[0], fb[0]))) > k.contact_thr_sq;
+      const bool contact_term = force_exceeds(&in.contact[lane][k.base_body * 3], k.contact_thr_sq);
       const bool time_out = len > k.max_len;
       const bool reset = contact_term | time_out;
       double st_sum[SHIFU_MAX_REWARD_TERMS];
@@ -334,17 +266,10 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
     const int p = t - V3_SCAN_BASE;                          // index in the scan group
     const int sw = p >> 5, lane = p & 31;
     const float hclip = fminf(k.h_clip, k.clip_obs);         // clip(clip(v,+-a),+-b) == clip(v,+-min(a,b))
-    const unsigned max_px = (unsigned)(k.trows - 1), max_py = (unsigned)(k.tcols - 1);
-    // banded index: (px>>3)*8*W + py*8 + (px&7)  ==  (px & ~7)*(W-1) + px + 8*py    (3 integer ops)
-    const unsigned c1 = (unsigned)(k.band_w - 1);
     const short* __restrict__ table = k.table;
-    const f2_t BORDER = pk(k.border, k.border);
-    const f2_t RCP = pk(k.hdiv.r, k.hdiv.r), NEGD = pk(-k.hdiv.d, -k.hdiv.d), VS = pk(k.vscale, k.vscale);
-    const f2_t NZ = pk(k.neg_zero, k.neg_zero);
-    const f2_t DENORM = pk(__int_as_float(1), __int_as_float(1));     // 2^-149
-    // Work items of a tile.  The measured-point grid is symmetric about the base (point 186 - pt is
-    // -point pt) and round-to-nearest is sign-symmetric, so the yaw rotation of the mirror point is
-    // EXACTLY the negated rotation of the point: a lane owns a point AND its mirror and rotates once.
+    const PairScanK sk = pair_scan_k(k);
+    const f2_t VS = pk(k.vscale, k.vscale);
+    // Work items of a tile (a lane owns a point and its mirror, see scan_pairs.cuh).
     // Item = (group of 32 point pairs [3 groups cover the 94 pairs], batch of 4 envs): warp w owns pair
     // group w % 3 for the env pairs 2*(V3_ITEMS*(w/3) + it), +1.  (The host routes grids that are not
     // point-symmetric to the phased kernel.)
@@ -370,56 +295,12 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           return r;
         };
         // Index arithmetic of one item in packed fp32x2 (two envs per instruction).
-        // cell index of the packed pair of positions (ax, ay) [already + base xy + border]: the constant
-        // division, .long() + clip and the banded table offset (isaac_gym.py:416-425)
-        auto cell_pair = [&](f2_t ax, f2_t ay, unsigned& i0, unsigned& i1) {
-          unsigned px0, px1, py0, py1;
-          if (EXACT_DIV) {
-            float a0, a1, b0, b1;
-            upk(ax, a0, a1); upk(ay, b0, b1);
-            // .long() + clip (isaac_gym.py:421-425): float->uint truncates and saturates at 0
-            px0 = min(__float2uint_rz(div_rn(a0, k.hdiv.d)), max_px);
-            px1 = min(__float2uint_rz(div_rn(a1, k.hdiv.d)), max_px);
-            py0 = min(__float2uint_rz(div_rn(b0, k.hdiv.d)), max_py);
-            py1 = min(__float2uint_rz(div_rn(b1, k.hdiv.d)), max_py);
-          } else {                         // q0 = x*r; e = fma(-d, q0, x); q = fma(e, r, q0)
-            const f2_t qx = mul2(ax, RCP), qy = mul2(ay, RCP);
-            const f2_t fx = fma2(fma2(NEGD, qx, ax), RCP, qx), fy = fma2(fma2(NEGD, qy, ay), RCP, qy);
-            // .long() + clip without the conversion unit: RZ(f * 2^-149) is the denormal whose bit
-            // pattern IS trunc(f) for 0 <= f < 2^23 (negative f -> sign bit -> relu -> 0, larger f
-            // -> a normal number >= 2^23 -> upper clip); one packed multiply per env pair
-            int ix0, ix1, iy0, iy1;
-            upk_i(mulrz2(fx, DENORM), ix0, ix1);
-            upk_i(mulrz2(fy, DENORM), iy0, iy1);
-            px0 = (unsigned)__vimin_s32_relu(ix0, (int)max_px); px1 = (unsigned)__vimin_s32_relu(ix1, (int)max_px);
-            py0 = (unsigned)__vimin_s32_relu(iy0, (int)max_py); py1 = (unsigned)__vimin_s32_relu(iy1, (int)max_py);
-          }
-          i0 = ((px0 & ~7u) * c1 + px0) + (py0 << 3);
-          i1 = ((px1 & ~7u) * c1 + px1) + (py1 << 3);
-        };
-        // Index arithmetic of one item in packed fp32x2 (two envs per instruction).
         auto index_batch = [&](const Item& w, unsigned (&idx)[8]) {
           const f2_t BX = pk(w.bx, w.bx), BY = pk(w.by, w.by), NBY = pk(-w.by, -w.by);
 #pragma unroll
-          for (int u = 0; u < 2; ++u) {
-            const float4 a = s.sA[rb][w.q0 + u], bq = s.sB[rb][w.q0 + u];
-            const float2 cq = *reinterpret_cast<const float2*>(&s.sC[rb][w.q0 + u]);
-            const f2_t Z2 = pk(a.x, a.y), Z = pk(a.z, a.w), W = pk(bq.x, bq.y), X = pk(bq.z, bq.w);
-            const f2_t Y = pk(cq.x, cq.y);
-            // quat_apply_yaw (shifu/utils/terrain.py:202-206) on (bx, by, 0):
-            //   t = 2(q x b) = (-2z*by, 2z*bx);  out = (b + w*t) + q x t,  q x t = (-z*ty, z*tx)
-            // Products that feed an add are written fma(a, b, -0): ptxas contracts
-            // mul.rn.f32x2 + add.rn.f32x2 into one FFMA2 (single rounding) even under --fmad=false,
-            // which flips ~0.3 % of the cell indices; fma(a, b, -0) == RN(a*b) exactly and cannot be
-            // contracted again (NZ comes from a kernel parameter, so it is not constant-folded).
-            const f2_t tx = mul2(Z2, NBY), ty = mul2(Z2, BX);
-            const f2_t rx = sub2(add2(BX, fma2(W, tx, NZ)), fma2(Z, ty, NZ));
-            const f2_t ry = add2(add2(BY, fma2(W, ty, NZ)), fma2(Z, tx, NZ));
-            // + base xy, + border (isaac_gym.py:416-420)
-            cell_pair(add2(add2(rx, X), BORDER), add2(add2(ry, Y), BORDER), idx[4 * u], idx[4 * u + 1]);
-            // the mirror point: rotation = (-rx, -ry) exactly, and RN(-r + X) == RN(X - r)
-            cell_pair(add2(sub2(X, rx), BORDER), add2(sub2(Y, ry), BORDER), idx[4 * u + 2], idx[4 * u + 3]);
-          }
+          for (int u = 0; u < 2; ++u)
+            point_pair_cells<EXACT_DIV>(sk, BX, BY, NBY, s.sA[rb][w.q0 + u], s.sB[rb][w.q0 + u],
+                                        *reinterpret_cast<const float2*>(&s.sC[rb][w.q0 + u]), idx + 4 * u);
         };
         auto load_batch = [&](const unsigned (&idx)[8], int (&h)[8]) {
 #pragma unroll
@@ -430,7 +311,7 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           float* mb = HAS_MROW ? io.measured_heights + (e0 + 2 * w.q0) * A1_POINTS + w.pt : nullptr;
           // one packed pair of cells -> (z - 0.5) - h*vertical_scale, clipped, to rows r and r+1
           auto emit = [&](float2 zb, int h0, int h1, float* o, float* m) {
-            const f2_t hg2 = fma2(pk((float)h0, (float)h1), VS, NZ);            // * vertical_scale, :433
+            const f2_t hg2 = fma2(pk((float)h0, (float)h1), VS, sk.nz);         // * vertical_scale, :433
             float v0, v1;
             upk(sub2(pk(zb.x, zb.y), hg2), v0, v1);                             // a1_conditional.py:132
             __stcs(o, clampf(v0, -hclip, hclip));

@@ -61,7 +61,7 @@ struct A1K {
   int band_w;             // banded layout: entries per map row inside a band (tcols padded to 8)
   int tiled;              // 1: banded (T[px>>3][py][px&7], a 128-B line = 8x8 cells), 0: row-major (pitch = tcols)
   double* stats;          // SHIFU_NUM_STATS accumulators
-  float neg_zero;         // -0.0f, opaque to ptxas: see the fma(a, b, -0) products in a1_fused_tma.cuh
+  float neg_zero;         // -0.0f, opaque to ptxas: see the fma(a, b, -0) products in scan_pairs.cuh
 };
 
 __device__ __forceinline__ float hdivide(float x, const A1K& k) {

@@ -212,9 +212,10 @@ def test_fused_step_term_lists_vs_oracle(list_name, n, carry, heights):
 
 @pytest.mark.parametrize("list_name", ["L1", "L2", "L3"])
 def test_eval_terms_is_what_the_step_accumulates(list_name):
-    """terms.verify_a1_terms compares user hooks with shifu_a1_eval_terms (the phased a1_eval_term); full
-    tiles of a step run v3_eval_term in the pipelined kernel.  On the simulator state of a live step, every
-    non-reset env's episode sums must grow by exactly the eval_terms values, and rew must be their sum."""
+    """terms.verify_a1_terms compares user hooks with shifu_a1_eval_terms; full tiles of a step run the
+    pipelined kernel, which stages its rows and accumulates the terms its own way (both evaluate
+    a1_reward_term).  On the simulator state of a live step, every non-reset env's episode sums must grow
+    by exactly the eval_terms values, and rew must be their sum."""
     from shifu_b200.sim.synthetic import a1_snapshot
     n = 32 * 300                                     # full tiles only: every env goes through the pipelined kernel
     kw = util.term_list(list_name)
