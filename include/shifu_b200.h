@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SHIFU_ABI_VERSION 2
+#define SHIFU_ABI_VERSION 3
 
 #define SHIFU_MAX_DOF 12
 #define SHIFU_MAX_LEG_BODIES 8
@@ -258,9 +258,12 @@ int shifu_set_level_sum(ShifuCtx* ctx, const int64_t* terrain_levels, void* stre
 /* ---- row a1/a2: action clip + PD torque substep --------------------------------------------
  * a1_conditional.py:66-67 (+ :123 and env.py:87 when actions_out != NULL: actions_out =
  * clip(action_scale*actions_in, +-clip_actions) is written and used; otherwise actions_in is used
- * as is).  Called once per decimation substep; PhysX runs between calls. */
+ * as is).  Called once per decimation substep; PhysX runs between calls.  substep is the 0-based
+ * decimation substep (negative: SHIFU_E_RANGE).  It changes no result: the library uses it only
+ * to choose the order in which the envs are swept, so that consecutive substeps reuse what the
+ * previous one left in L2. */
 int shifu_pd_torque(ShifuCtx* ctx, const float* actions_in, float* actions_out, const float* dof_state,
-                    float* torques, void* stream);
+                    float* torques, int32_t substep, void* stream);
 
 /* ---- row a3: LeggedRobot.post_step (shifu/units/robot.py:222-229) -------------------------- */
 /* Root row of env e = root_state[(root_offset + e*root_stride)*13 ..]; works on any ctx. */

@@ -12,7 +12,7 @@ import os
 from typing import Optional
 
 MAX_DOF, MAX_LEG, MAX_PX, MAX_PY, MAX_TERMS, NUM_STATS = 12, 8, 17, 11, 8, 16
-ABI_VERSION = 2
+ABI_VERSION = 3
 
 # enum ShifuRewardTerm
 REW_TRACKING_LIN_VEL, REW_TRACKING_ANG_VEL, REW_STABILIZING_BASE, REW_SMOOTHING_ACTION = 0, 1, 2, 3
@@ -142,7 +142,7 @@ SIGNATURES = {
     "shifu_abi_version": [],
     "shifu_set_height_map": [_VP, _VP, _I32, _I32, _VP],
     "shifu_set_level_sum": [_VP, _VP, _VP],
-    "shifu_pd_torque": [_VP, _VP, _VP, _VP, _VP, _VP],
+    "shifu_pd_torque": [_VP, _VP, _VP, _VP, _VP, _I32, _VP],
     "shifu_body_frame": [_VP, _VP, _I32, _I32, _I32, _VP, _VP, _VP, _VP, _VP],
     "shifu_get_heights": [_VP, _VP, _VP, _VP, _VP],
     "shifu_a1_post_physics": [_VP, C.POINTER(A1StepIO), _VP],

@@ -105,15 +105,44 @@ __global__ void build_scan_table_kernel(const short* __restrict__ H, int rows, i
 // One thread per group of 4 consecutive dofs (3 groups per env): one 128-bit action load, two
 // 128-bit dof_state loads (4 x (pos, vel)), one 128-bit torque store — all fully coalesced.
 // Pure streaming: 192 B/env per substep (240 B when the clipped actions are written too).
+// descending != 0 sweeps the quads from the last one down (loop counter i processes quad
+// total-1-i), so a launch can start on the rows the launch before it touched last, which are
+// still in L2.  A warp still covers a contiguous span, so the accesses stay coalesced; which
+// launch sweeps which way is decided in capi.cu (shifu_pd_torque).  The first half of every
+// sweep is the half the next, reversed sweep reaches last, long after it has left L2: its loads
+// and stores carry an L2 evict_first policy, so that the second half, which the next sweep
+// starts on, keeps more of L2.
 // ------------------------------------------------------------------------------------------
 __device__ __forceinline__ float pd_one(float a, float q0, float kp, float kd, float lim, float q, float qd) {
   const float e = sub_rn(add_rn(a, q0), q);
   return clampf(sub_rn(mul_rn(kp, e), mul_rn(kd, qd)), -lim, lim);
 }
 
+__device__ __forceinline__ unsigned long long l2_policy_evict_first() {
+  unsigned long long p;
+  asm("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
+  return p;
+}
+__device__ __forceinline__ unsigned long long l2_policy_evict_normal() {
+  unsigned long long p;
+  asm("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(p));
+  return p;
+}
+// read-only (non-coherent) 128-bit load / 128-bit store with an L2 cache policy
+__device__ __forceinline__ float4 ldg_l2(const float4* p, unsigned long long pol) {
+  float4 v;
+  asm volatile("ld.global.nc.L2::cache_hint.v4.f32 {%0, %1, %2, %3}, [%4], %5;"
+               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol));
+  return v;
+}
+__device__ __forceinline__ void stg_l2(float4* p, float4 v, unsigned long long pol) {
+  asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;"
+               :: "l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "l"(pol) : "memory");
+}
+
 __global__ void __launch_bounds__(256)
 pd_torque_kernel(const __grid_constant__ A1K k, const float4* __restrict__ a_in, float4* __restrict__ a_out,
-                 const float4* __restrict__ dof, float4* __restrict__ tau) {
+                 const float4* __restrict__ dof, float4* __restrict__ tau, int descending) {
   __shared__ __align__(16) float c_q0[A1_DOF], c_kp[A1_DOF], c_kd[A1_DOF], c_lim[A1_DOF];
   if (threadIdx.x < A1_DOF) {
     c_q0[threadIdx.x] = k.q0[threadIdx.x];
@@ -124,15 +153,18 @@ pd_torque_kernel(const __grid_constant__ A1K k, const float4* __restrict__ a_in,
   __syncthreads();
   const unsigned total = (unsigned)k.n * (A1_DOF / 4);          // <= 3 * 2^31 / 4 quads
   const float sc = k.action_scale, ca = k.clip_actions;
-  for (unsigned q = blockIdx.x * blockDim.x + threadIdx.x; q < total; q += gridDim.x * blockDim.x) {
+  const unsigned long long pol_first = l2_policy_evict_first(), pol_normal = l2_policy_evict_normal();
+  for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+    const unsigned q = descending ? total - 1u - i : i;           // the quad this iteration processes
     const unsigned g = q % 3u;                                    // which third of the env's 12 dofs
-    float4 a = __ldg(a_in + q);
+    const unsigned long long pol = i < total / 2u ? pol_first : pol_normal;
+    float4 a = ldg_l2(a_in + q, pol);
     if (a_out != nullptr) {                                       // a1_conditional.py:123, env.py:87
       a.x = clampf(mul_rn(a.x, sc), -ca, ca); a.y = clampf(mul_rn(a.y, sc), -ca, ca);
       a.z = clampf(mul_rn(a.z, sc), -ca, ca); a.w = clampf(mul_rn(a.w, sc), -ca, ca);
-      a_out[q] = a;
+      stg_l2(a_out + q, a, pol);
     }
-    const float4 s0 = __ldg(dof + 2 * (size_t)q), s1 = __ldg(dof + 2 * (size_t)q + 1);
+    const float4 s0 = ldg_l2(dof + 2 * (size_t)q, pol), s1 = ldg_l2(dof + 2 * (size_t)q + 1, pol);
     const float4 q0 = reinterpret_cast<const float4*>(c_q0)[g], kp = reinterpret_cast<const float4*>(c_kp)[g];
     const float4 kd = reinterpret_cast<const float4*>(c_kd)[g], lm = reinterpret_cast<const float4*>(c_lim)[g];
     float4 t;
@@ -140,7 +172,7 @@ pd_torque_kernel(const __grid_constant__ A1K k, const float4* __restrict__ a_in,
     t.y = pd_one(a.y, q0.y, kp.y, kd.y, lm.y, s0.z, s0.w);
     t.z = pd_one(a.z, q0.z, kp.z, kd.z, lm.z, s1.x, s1.y);
     t.w = pd_one(a.w, q0.w, kp.w, kd.w, lm.w, s1.z, s1.w);
-    tau[q] = t;
+    stg_l2(tau + q, t, pol);
   }
 }
 

@@ -370,15 +370,22 @@ extern "C" int shifu_set_level_sum(ShifuCtx* c, const int64_t* levels, void* str
   return SHIFU_OK;
 }
 
-extern "C" int shifu_pd_torque(ShifuCtx* c, const float* a_in, float* a_out, const float* dof, float* tau, void* stream) {
+extern "C" int shifu_pd_torque(ShifuCtx* c, const float* a_in, float* a_out, const float* dof, float* tau,
+                               int32_t substep, void* stream) {
   REQUIRE_PTR(c); REQUIRE_PTR(a_in); REQUIRE_PTR(dof); REQUIRE_PTR(tau);
   if (!c->is_a1) return fail(SHIFU_E_STATE, "shifu_pd_torque needs an A1 ctx");
+  if (substep < 0) return fail(SHIFU_E_RANGE, "shifu_pd_torque: substep must be >= 0 (got %d)", substep);
   REQUIRE_ALIGNED(dof, 16); REQUIRE_ALIGNED(a_in, 16); REQUIRE_ALIGNED(tau, 16);
   if (a_out != nullptr) REQUIRE_ALIGNED(a_out, 16);
   const long long quads = (long long)c->a1.num_envs * (A1_DOF / 4);
+  // The four substeps and the fused kernel all stream the same dof_state / actions / torques
+  // (~200 MB at 1 Mi envs, more than L2).  Odd substeps sweep downward, so each launch starts on
+  // the rows the previous one touched last, and the last substep ends on env 0, where the fused
+  // kernel's first tiles start.
+  const int descending = substep & 1;
   pd_torque_kernel<<<grid_for(quads, 256, c->sm_count, 8), 256, 0, S(stream)>>>(
       c->a1k, reinterpret_cast<const float4*>(a_in), reinterpret_cast<float4*>(a_out),
-      reinterpret_cast<const float4*>(dof), reinterpret_cast<float4*>(tau));
+      reinterpret_cast<const float4*>(dof), reinterpret_cast<float4*>(tau), descending);
   CUDA_TRY(cudaGetLastError());
   return SHIFU_OK;
 }

@@ -392,6 +392,7 @@ class A1HotPath(_StepStats):
         self.swing_time = torch.zeros(n, max(desc.num_feet, 1), **f)
         self.last_contacts = torch.zeros(n, max(desc.num_feet, 1), device=dev, dtype=torch.bool)
         self.step_counter = 0
+        self._pd_substep = -1            # decimation substep of the last pd_torque call
         self._init_stats(dev)
         self._graph, self._graph_warm, self._dev_step, self._graph_actions = None, 0, -1, None
         self._fork = None
@@ -465,14 +466,17 @@ class A1HotPath(_StepStats):
 
     # -- individual rows -------------------------------------------------
     def pd_torque(self, raw_actions: Optional[torch.Tensor] = None):
-        """Row a2 (+a1 when ``raw_actions`` is given: env.actions = clip(0.5*a, +-1) is produced too)."""
+        """Row a2 (+a1 when ``raw_actions`` is given: env.actions = clip(0.5*a, +-1) is produced too).
+        A call with ``raw_actions`` is decimation substep 0, one without is the previous substep + 1;
+        the library picks each substep's sweep order from that number (the results do not depend on it)."""
         s = nv.current_stream()
+        self._pd_substep = 0 if raw_actions is not None else self._pd_substep + 1
         if raw_actions is not None:
             nv.check(self.lib.shifu_pd_torque(self.ctx.handle, nv.ptr(raw_actions), nv.ptr(self.actions),
-                                              nv.ptr(self.dof_state), nv.ptr(self.torques), s))
+                                              nv.ptr(self.dof_state), nv.ptr(self.torques), self._pd_substep, s))
         else:
             nv.check(self.lib.shifu_pd_torque(self.ctx.handle, nv.ptr(self.actions), None,
-                                              nv.ptr(self.dof_state), nv.ptr(self.torques), s))
+                                              nv.ptr(self.dof_state), nv.ptr(self.torques), self._pd_substep, s))
 
     def body_frame(self):
         """Row a3: LeggedRobot.post_step on the CURRENT content of root_state (S_prev, D7)."""
