@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SHIFU_ABI_VERSION 3
+#define SHIFU_ABI_VERSION 4
 
 #define SHIFU_MAX_DOF 12
 #define SHIFU_MAX_LEG_BODIES 8
@@ -37,6 +37,7 @@ extern "C" {
 #define SHIFU_MAX_POINTS_Y 11
 #define SHIFU_MAX_REWARD_TERMS 8
 #define SHIFU_NUM_STATS 16
+#define SHIFU_OBS_HEAD 72       /* observation columns before the 187 heights */
 
 enum {
   SHIFU_OK = 0,
@@ -72,6 +73,18 @@ enum ShifuRewardTerm {
                                      STATEFUL: swing_time / last_contacts (a1_conditional.py:99-102) are
                                      updated exactly like legged_gym's _reward_feet_air_time */
   SHIFU_REW_COUNT = 16
+};
+
+/* Source of one 3-column vector slot of the A1 observation (columns 3i..3i+2, i < 4) when
+ * ShifuA1Desc.obs_layout == 1.  The reference observation is COMMAND, BASE_LIN_VEL, BASE_ANG_VEL,
+ * GRAVITY_VEC (a1_conditional.py:131-144). */
+enum ShifuObsVec {
+  SHIFU_OBS_COMMAND = 0,            /* command_buf */
+  SHIFU_OBS_BASE_LIN_VEL = 1,       /* base_lin_vel (the carried S_prev value, D7) */
+  SHIFU_OBS_BASE_ANG_VEL = 2,       /* base_ang_vel */
+  SHIFU_OBS_GRAVITY_VEC = 3,        /* the constant (0, 0, -1) */
+  SHIFU_OBS_PROJECTED_GRAVITY = 4,  /* projected_gravity as it is when the step starts (robot.py:222-229 on S_prev) */
+  SHIFU_OBS_VEC_COUNT = 5
 };
 
 /* Index of each statistic in the stats vector (double[SHIFU_NUM_STATS]) that
@@ -148,6 +161,14 @@ typedef struct ShifuA1Desc {
   float air_time_cmd_min;                           /* term is 0 unless |cmd_xy| > this (0.1) */
   float air_time_dt;                                /* control dt added to swing_time every step (isaac_gym.py:26) */
   int32_t air_time_reset;                           /* !=0: reset_idx zeroes swing_time / last_contacts of the env */
+  /* observation layout (legged_gym's obs_scales / commands_scale, projected gravity, slot order) */
+  int32_t obs_layout;                               /* 0: the reference observation (a1_conditional.py:131-144); the
+                                                       fields below are ignored.  1: as below */
+  int32_t obs_vec_src[4];                           /* enum ShifuObsVec, source of columns 3i..3i+2 */
+  float obs_scale[SHIFU_OBS_HEAD];                  /* obs[j] = clip(x_j * obs_scale[j], +-clip_obs), j < 72;
+                                                       x_j of the dof-position columns is dof_pos - q0 */
+  float obs_height_scale;                           /* heights = clip(clip(z - height_offset - h, +-height_clip) * this,
+                                                       +-clip_obs) */
 } ShifuA1Desc;
 
 /* Tensors of one A1 step.  "rw" = read and written in place. */

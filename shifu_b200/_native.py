@@ -12,13 +12,16 @@ import os
 from typing import Optional
 
 MAX_DOF, MAX_LEG, MAX_PX, MAX_PY, MAX_TERMS, NUM_STATS = 12, 8, 17, 11, 8, 16
-ABI_VERSION = 3
+ABI_VERSION = 4
+OBS_HEAD = 72
 
 # enum ShifuRewardTerm
 REW_TRACKING_LIN_VEL, REW_TRACKING_ANG_VEL, REW_STABILIZING_BASE, REW_SMOOTHING_ACTION = 0, 1, 2, 3
 REW_LEG_COLLISION, REW_TORQUES, REW_ABB_REACHING, REW_ABB_SUCCESS = 4, 5, 6, 7
 REW_LIN_VEL_Z, REW_ANG_VEL_XY, REW_ORIENTATION, REW_DOF_VEL, REW_ACTION_RATE, REW_BASE_HEIGHT = 8, 9, 10, 11, 12, 13
 REW_DOF_POS_LIMITS, REW_FEET_AIR_TIME = 14, 15
+# enum ShifuObsVec
+OBS_COMMAND, OBS_BASE_LIN_VEL, OBS_BASE_ANG_VEL, OBS_GRAVITY_VEC, OBS_PROJECTED_GRAVITY, OBS_VEC_COUNT = range(6)
 STAT_TERM0, STAT_NRESET, STAT_LEVEL_SUM, STAT_SUCCESS, STAT_NENVS = 0, 8, 9, 10, 11
 
 E_NULL, E_RANGE, E_STATE, E_NODEVICE, E_ALIGN = -1, -2, -3, -4, -5
@@ -55,6 +58,8 @@ class A1Desc(C.Structure):
         ("dof_pos_limit_low", C.c_float * MAX_DOF), ("dof_pos_limit_high", C.c_float * MAX_DOF),
         ("num_feet", C.c_int32), ("feet_bodies", C.c_int32 * 4), ("feet_contact_force", C.c_float),
         ("air_time_cmd_min", C.c_float), ("air_time_dt", C.c_float), ("air_time_reset", C.c_int32),
+        ("obs_layout", C.c_int32), ("obs_vec_src", C.c_int32 * 4), ("obs_scale", C.c_float * OBS_HEAD),
+        ("obs_height_scale", C.c_float),
     ]
 
 

@@ -8,7 +8,8 @@
 //       does termination, warp 5 the yaw-quaternion normalisation for the height scan
 //   B2  warp 0 (lane = env): ordered reward / episode-sum accumulation, flag and ep_len stores,
 //       reset of flagged envs (curriculum, Philox draws, state rewrite), per-step log sums
-//   B3  all threads: obs head (72 columns), history push, carried body-frame velocities
+//   B3  all threads: obs head (72 columns, laid out and scaled by A1Obs), history push, carried
+//       body-frame velocities
 //   D   coalesced write-back of the obs head and the history tile
 //   C   thread t owns scan point t: 187-point height scan per env, obs columns 72..258 streamed
 //       straight to HBM (a warp writes 128 contiguous bytes per env)
@@ -218,15 +219,21 @@ __device__ __noinline__ float a1_eval_term(int q, const A1K& k, const A1Smem& s,
   return a1_reward_term<true>(k.terms[q], q, k.rp[q][0], k.rp[q][1], k, s, e, io, ge);
 }
 
+// The observation layout `o` is applied at run time for every layout (this kernel takes the ragged tail
+// and the fallback layouts); for the reference layout it is the identity, and x * 1.0f plus the
+// composed clips are exact, so the reference observation comes out unchanged.
 template <bool TILED, bool EXACT_DIV>
 __global__ void __launch_bounds__(A1_THREADS, 5)
-a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io) {
+a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io,
+                       const __grid_constant__ A1Obs o) {
   __shared__ __align__(16) A1Smem s;
+  // projected gravity at the start of the step: warp 5 overwrites io.projected_gravity in phase B3
+  // (carry_body_frame) while the other threads build the head
+  __shared__ float pg0[A1_TILE][3];
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const long long step = (io.step_dev != nullptr) ? *io.step_dev : io.step;
   // scan point owned by this thread (threads 187..191 idle in phase C)
   const float bx = k.px[t % A1_NX], by = k.py[(t / A1_NX) % A1_NY];
-  const float hclip = fminf(k.h_clip, k.clip_obs);     // clip(clip(v,+-a),+-b) == clip(v,+-min(a,b))
   const unsigned max_px = (unsigned)(k.trows - 1), max_py = (unsigned)(k.tcols - 1);
 
   for (int e0 = blockIdx.x * A1_TILE; e0 < k.n; e0 += gridDim.x * A1_TILE) {
@@ -250,6 +257,8 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
       for (int j = 0; j < SHIFU_MAX_REWARD_TERMS; ++j) esum[j] = (j < k.n_terms) ? io.ep_sums[j][ge] : 0.0f;
     }
     a1_stage_rows(s, k, io, e0, ne, t);
+    if (o.uses_pg)
+      for (int i = t; i < ne * 3; i += A1_THREADS) (&pg0[0][0])[i] = io.projected_gravity[e0 * 3LL + i];
     if (warp == 0 && lane_env) {
 #pragma unroll
       for (int j = 0; j < 9; ++j) s.cla[j / 3][lane][j % 3] = c9[j];
@@ -322,22 +331,21 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
       for (int i = t; i < ne * A1_DOF; i += A1_THREADS) {
         const int e = i / A1_DOF, d = i - e * A1_DOF;
         float* h = s.head[e];
-        h[12 + d] = clampf(sub_rn(s.dof[e][2 * d], k.q0[d]), -c, c);
-        h[24 + d] = clampf(s.dof[e][2 * d + 1], -c, c);
+        h[12 + d] = clampf(mul_rn(sub_rn(s.dof[e][2 * d], k.q0[d]), o.scale[12 + d]), -c, c);
+        h[24 + d] = clampf(mul_rn(s.dof[e][2 * d + 1], o.scale[24 + d]), -c, c);
         const float a0 = s.hist[e][d * A1_HIST + 0], a1 = s.hist[e][d * A1_HIST + 1],
                     a2 = s.hist[e][d * A1_HIST + 2];
-        h[36 + d] = clampf(a0, -c, c);                 // HistoryRecorder.flatten: slot-major
-        h[48 + d] = clampf(a1, -c, c);
-        h[60 + d] = clampf(a2, -c, c);
+        h[36 + d] = clampf(mul_rn(a0, o.scale[36 + d]), -c, c);    // HistoryRecorder.flatten: slot-major
+        h[48 + d] = clampf(mul_rn(a1, o.scale[48 + d]), -c, c);
+        h[60 + d] = clampf(mul_rn(a2, o.scale[60 + d]), -c, c);
         s.hist[e][d * A1_HIST + 2] = a1;               // HistoryRecorder.add
         s.hist[e][d * A1_HIST + 1] = a0;
         s.hist[e][d * A1_HIST + 0] = s.act[e][d];
       }
-      // (env, j < 12): command, body-frame velocities, gravity_vec
+      // (env, j < 12): the four vector slots (reference: command, body-frame velocities, gravity_vec)
       for (int i = t; i < ne * 12; i += A1_THREADS) {
         const int e = i / 12, j = i - e * 12;
-        const float v = (j < 9) ? s.cla[j / 3][e][j % 3] : ((j == 11) ? -1.0f : 0.0f);
-        s.head[e][j] = clampf(v, -c, c);
+        s.head[e][j] = clampf(mul_rn(a1_obs_vec(o, j, s.cla, e, pg0[e][j % 3]), o.scale[j]), -c, c);
       }
       // carried body-frame velocities for the next control step (robot.py:222-229, D7)
       if (io.carry_body_frame && warp == 5 && lane_env) {
@@ -368,7 +376,7 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
                  A1_THREADS);
     }
 
-    // ---- phase C: 187-point scan; obs[., 72 + t] = clip((z - 0.5) - h, +-1) --------------------
+    // ---- phase C: 187-point scan; obs[., 72 + t] = clip(clip((z - 0.5) - h, +-1) * h_scale, +-clip_obs)
     if (t < A1_POINTS) {
       float* orow = io.obs_buf + (long long)e0 * A1_OBS + A1_HEAD + t;
       float* mrow = (io.measured_heights != nullptr) ? io.measured_heights + (long long)e0 * A1_POINTS + t
@@ -397,7 +405,7 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
           idx = (int)(px * (unsigned)k.tcols + py);
         }
         const float hgt = mul_rn((float)__ldg(table + idx), k.vscale);      // isaac_gym.py:427-433
-        const float v = clampf(sub_rn(ps.z, hgt), -hclip, hclip);
+        const float v = clampf(mul_rn(clampf(sub_rn(ps.z, hgt), -k.h_clip, k.h_clip), o.h_scale), -k.clip_obs, k.clip_obs);
         __stcs(orow + (long long)e * A1_OBS, v);
         if (mrow != nullptr) __stcs(mrow + (long long)e * A1_POINTS, hgt);
       }

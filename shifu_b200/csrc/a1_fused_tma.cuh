@@ -20,7 +20,8 @@
 //   scan group (12 warps; thread = scan point + its mirror point, warp w: point pairs 32*(w%3)..,
 //                        env pairs 4*(w/3) .. +3 in two items of 4 envs)
 //                        first item's index arithmetic + gathers, then the obs head from the
-//                        post-reset rows (a1_conditional.py:131-144), history push (train.py:12-14),
+//                        post-reset rows (a1_conditional.py:131-144, or the A1Obs layout with OBS),
+//                        history push (train.py:12-14),
 //                        then the rest of the 187-point height scan (isaac_gym.py:393-433) with
 //                        packed fp32x2 arithmetic (two envs per instruction, one yaw rotation per
 //                        point pair), streamed with st.global.cs
@@ -111,9 +112,12 @@ __device__ __forceinline__ void v3_issue_loads(V3In& in, const A1K& k, const Shi
 // the barrier-phased kernel).  Requires root_stride == 1 and 16-byte aligned tensors.
 // HAS_EXTRA: the term list holds a code >= SHIFU_REW_LIN_VEL_Z.  The reference's own six terms run the
 // instantiation without that code (its presence alone cost the B group 5-10 % of the kernel).
-template <bool EXACT_DIV, bool HAS_MROW, bool HAS_EXTRA>
+// OBS: the observation follows the layout `o` (slot sources, column scales, height scale); without it
+// `o` is not read and the reference observation is built.
+template <bool EXACT_DIV, bool HAS_MROW, bool HAS_EXTRA, bool OBS>
 __global__ void __launch_bounds__(V3_THREADS, V3_CTAS_PER_SM)
-a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io, int num_tiles) {
+a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io, int num_tiles,
+                           const __grid_constant__ A1Obs o) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   V3Smem& s = *reinterpret_cast<V3Smem*>(smem_raw);
   const int t = threadIdx.x;
@@ -265,7 +269,8 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
   {
     const int p = t - V3_SCAN_BASE;                          // index in the scan group
     const int sw = p >> 5, lane = p & 31;
-    const float hclip = fminf(k.h_clip, k.clip_obs);         // clip(clip(v,+-a),+-b) == clip(v,+-min(a,b))
+    // clip(clip(v,+-a),+-b) == clip(v,+-min(a,b)); with OBS, clip(clip(v,+-a)*s,+-b) == clip(v*s,+-h_bound)
+    const float hclip = OBS ? o.h_bound : fminf(k.h_clip, k.clip_obs);
     const short* __restrict__ table = k.table;
     const PairScanK sk = pair_scan_k(k);
     const f2_t VS = pk(k.vscale, k.vscale);
@@ -307,15 +312,17 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           for (int u = 0; u < 8; ++u) h[u] = __ldg(table + idx[u]);          // isaac_gym.py:427-431 (folded)
         };
         auto store_batch = [&](const Item& w, const int (&h)[8]) {
-          float* ob = io.obs_buf + (e0 + 2 * w.q0) * A1_OBS + A1_HEAD + w.pt;
+          float* orow = io.obs_buf + (e0 + 2 * w.q0) * A1_OBS + A1_HEAD + w.pt;
           float* mb = HAS_MROW ? io.measured_heights + (e0 + 2 * w.q0) * A1_POINTS + w.pt : nullptr;
           // one packed pair of cells -> (z - 0.5) - h*vertical_scale, clipped, to rows r and r+1
-          auto emit = [&](float2 zb, int h0, int h1, float* o, float* m) {
+          auto emit = [&](float2 zb, int h0, int h1, float* ob, float* m) {
             const f2_t hg2 = fma2(pk((float)h0, (float)h1), VS, sk.nz);         // * vertical_scale, :433
             float v0, v1;
-            upk(sub2(pk(zb.x, zb.y), hg2), v0, v1);                             // a1_conditional.py:132
-            __stcs(o, clampf(v0, -hclip, hclip));
-            __stcs(o + A1_OBS, clampf(v1, -hclip, hclip));
+            f2_t d2 = sub2(pk(zb.x, zb.y), hg2);                                  // a1_conditional.py:132
+            if (OBS) d2 = mul2(d2, pk(o.h_scale, o.h_scale));
+            upk(d2, v0, v1);
+            __stcs(ob, clampf(v0, -hclip, hclip));
+            __stcs(ob + A1_OBS, clampf(v1, -hclip, hclip));
             if (HAS_MROW) {
               float g0, g1;
               upk(hg2, g0, g1);
@@ -328,8 +335,8 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
 #pragma unroll
             for (int u = 0; u < 2; ++u) {
               const float2 zb = *reinterpret_cast<const float2*>(&s.sC[rb][w.q0 + u].z);
-              emit(zb, h[4 * u], h[4 * u + 1], ob + (2 * u) * A1_OBS, mb + (2 * u) * A1_POINTS);
-              emit(zb, h[4 * u + 2], h[4 * u + 3], ob + (2 * u) * A1_OBS + mir, mb + (2 * u) * A1_POINTS + mir);
+              emit(zb, h[4 * u], h[4 * u + 1], orow + (2 * u) * A1_OBS, mb + (2 * u) * A1_POINTS);
+              emit(zb, h[4 * u + 2], h[4 * u + 3], orow + (2 * u) * A1_OBS + mir, mb + (2 * u) * A1_POINTS + mir);
             }
           }
         };
@@ -343,6 +350,13 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
         Item cur = item(0);
         index_batch(cur, idx);
         load_batch(idx, h);
+        // with OBS, a slot of projected_gravity reads its pre-step value from global memory, issued here to
+        // hide the latency: this tile's rows are bulk-stored over only after this thread's h_done arrival
+        float pgv = 0.0f;
+        if (OBS) {
+          const int pe = p / A1_DOF, pd = p - pe * A1_DOF;
+          if (o.src[pd / 3] == SHIFU_OBS_PROJECTED_GRAVITY) pgv = io.projected_gravity[(e0 + pe) * 3 + pd % 3];
+        }
         // ---- obs head (a1_conditional.py:131-144) + history push (train.py:12-14): post-reset rows
         pipe::mbar_wait<32>(&s.b_done[b], par);
         {
@@ -359,18 +373,22 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           const float2 qd = *reinterpret_cast<const float2*>(&in.dof[e][2 * d]);
           const float a0 = in.hist[e][d * A1_HIST + 0], a1 = in.hist[e][d * A1_HIST + 1],
                       a2 = in.hist[e][d * A1_HIST + 2];
-          const float v = (d < 9) ? in.cla[d / 3][e][d % 3] : ((d == 11) ? -1.0f : 0.0f);   // command, velocities, gravity_vec
+          // command, velocities, gravity_vec; with OBS the slot's source
+          const float v = OBS ? a1_obs_vec(o, d, in.cla, e, pgv)
+                              : (d < 9) ? in.cla[d / 3][e][d % 3] : ((d == 11) ? -1.0f : 0.0f);
           in.hist[e][d * A1_HIST + 2] = a1;              // HistoryRecorder.add (train.py:12-14)
           in.hist[e][d * A1_HIST + 1] = a0;
           in.hist[e][d * A1_HIST + 0] = in.act[e][d];
           pipe::fence_proxy_async();                            // pushed history -> visible to the TMA store
           pipe::mbar_arrive(&s.h_done[b]);
-          __stcs(hrow + d, clampf(v, -c, c));
-          __stcs(hrow + 12 + d, clampf(sub_rn(qd.x, k.q0[d]), -c, c));
-          __stcs(hrow + 24 + d, clampf(qd.y, -c, c));
-          __stcs(hrow + 36 + d, clampf(a0, -c, c));             // HistoryRecorder.flatten: slot-major
-          __stcs(hrow + 48 + d, clampf(a1, -c, c));
-          __stcs(hrow + 60 + d, clampf(a2, -c, c));
+          // with OBS: x_j * scale[j] before the clip
+          auto sc = [&](float x, int j) { return OBS ? mul_rn(x, o.scale[j]) : x; };
+          __stcs(hrow + d, clampf(sc(v, d), -c, c));
+          __stcs(hrow + 12 + d, clampf(sc(sub_rn(qd.x, k.q0[d]), 12 + d), -c, c));
+          __stcs(hrow + 24 + d, clampf(sc(qd.y, 24 + d), -c, c));
+          __stcs(hrow + 36 + d, clampf(sc(a0, 36 + d), -c, c));   // HistoryRecorder.flatten: slot-major
+          __stcs(hrow + 48 + d, clampf(sc(a1, 48 + d), -c, c));
+          __stcs(hrow + 60 + d, clampf(sc(a2, 60 + d), -c, c));
         }
 #pragma unroll 1
         for (int it = 1; it < V3_ITEMS; ++it) {

@@ -64,6 +64,34 @@ struct A1K {
   float neg_zero;         // -0.0f, opaque to ptxas: see the fma(a, b, -0) products in scan_pairs.cuh
 };
 
+// Observation layout of the fused step (ShifuA1Desc.obs_layout = 1): a separate __grid_constant__
+// parameter appended after the existing ones, so that A1K and the parameter offsets of the
+// reference-layout instantiations stay as they are.  Identity (src = 0, 1, 2, 3, every scale 1) for
+// the reference observation.
+static_assert(A1_HEAD == SHIFU_OBS_HEAD, "observation head width");
+struct A1Obs {
+  int src[4];             // enum ShifuObsVec of columns 3i..3i+2
+  float scale[A1_HEAD];   // obs[j] = clip(x_j * scale[j], +-clip_obs)
+  float h_scale;          // heights: clip(clip(z - h_off - h, +-h_clip) * h_scale, +-clip_obs)
+  float h_bound;          // min(h_clip * |h_scale|, clip_obs): the same heights as clip((z - h_off - h) * h_scale,
+                          // +-h_bound), because rounding the product is monotonic and sign-symmetric
+  int uses_pg;            // some slot reads projected_gravity
+};
+
+// Value of head column j < 12 of env e: slot j / 3, component j % 3.  cla = command, base lin vel,
+// base ang vel of the env; pg = component j % 3 of its projected gravity when the step started.
+template <class Cla>
+__device__ __forceinline__ float a1_obs_vec(const A1Obs& o, int j, const Cla& cla, int e, float pg) {
+  const int c = j % 3;
+  switch (o.src[j / 3]) {
+    case SHIFU_OBS_COMMAND: return cla[0][e][c];
+    case SHIFU_OBS_BASE_LIN_VEL: return cla[1][e][c];
+    case SHIFU_OBS_BASE_ANG_VEL: return cla[2][e][c];
+    case SHIFU_OBS_GRAVITY_VEC: return c == 2 ? -1.0f : 0.0f;
+    default: return pg;
+  }
+}
+
 __device__ __forceinline__ float hdivide(float x, const A1K& k) {
   return k.exact_div ? div_rn(x, k.hdiv.d) : div_const(x, k.hdiv);
 }

@@ -55,6 +55,8 @@ struct ShifuCtx {
   ShifuA1Desc a1{};
   ShifuAbbDesc abb{};
   A1K a1k{};
+  A1Obs a1o{};                     // observation layout (identity for the reference observation)
+  bool obs_custom = false;         // a1o differs from the reference: the OBS instantiations of the pipelined kernel
   AbbK abbk{};
   short* d_table = nullptr;
   double* d_stats = nullptr;         // SHIFU_NUM_STATS accumulators + [SHIFU_NUM_STATS] = level sum
@@ -71,13 +73,23 @@ struct ShifuCtx {
 
 static inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
-// the pipelined kernel's instantiations, index = 4*EXACT_DIV + 2*HAS_MROW + HAS_EXTRA
+// the pipelined kernel's instantiations, index = 8*OBS + 4*EXACT_DIV + 2*HAS_MROW + HAS_EXTRA
+constexpr int A1_TMA_VARIANTS = 16;
+template <bool OBS>
+static void a1_tma_fill(const void** t) {
+  t[0] = (const void*)a1_post_physics_tma_kernel<false, false, false, OBS>;
+  t[1] = (const void*)a1_post_physics_tma_kernel<false, false, true, OBS>;
+  t[2] = (const void*)a1_post_physics_tma_kernel<false, true, false, OBS>;
+  t[3] = (const void*)a1_post_physics_tma_kernel<false, true, true, OBS>;
+  t[4] = (const void*)a1_post_physics_tma_kernel<true, false, false, OBS>;
+  t[5] = (const void*)a1_post_physics_tma_kernel<true, false, true, OBS>;
+  t[6] = (const void*)a1_post_physics_tma_kernel<true, true, false, OBS>;
+  t[7] = (const void*)a1_post_physics_tma_kernel<true, true, true, OBS>;
+}
 static const void* const* a1_tma_variants() {
-  static const void* const table[8] = {
-      (const void*)a1_post_physics_tma_kernel<false, false, false>, (const void*)a1_post_physics_tma_kernel<false, false, true>,
-      (const void*)a1_post_physics_tma_kernel<false, true, false>,  (const void*)a1_post_physics_tma_kernel<false, true, true>,
-      (const void*)a1_post_physics_tma_kernel<true, false, false>,  (const void*)a1_post_physics_tma_kernel<true, false, true>,
-      (const void*)a1_post_physics_tma_kernel<true, true, false>,   (const void*)a1_post_physics_tma_kernel<true, true, true>};
+  static const void* table[A1_TMA_VARIANTS];
+  static const bool filled = (a1_tma_fill<false>(table), a1_tma_fill<true>(table + 8), true);
+  (void)filled;
   return table;
 }
 
@@ -92,6 +104,36 @@ static float sqrt_threshold(float thr) {
   while (s > 0.0f && std::sqrt(s) > thr) s = std::nextafter(s, 0.0f);
   while (std::sqrt(std::nextafter(s, INFINITY)) <= thr) s = std::nextafter(s, INFINITY);
   return s;
+}
+
+// Observation layout of the descriptor -> o (identity for layout 0); custom = it differs from the reference.
+static int fill_a1obs(const ShifuA1Desc& d, A1Obs& o, bool& custom) {
+  if (d.obs_layout != 0 && d.obs_layout != 1) return fail(SHIFU_E_RANGE, "obs_layout=%d must be 0 or 1", d.obs_layout);
+  std::memset(&o, 0, sizeof(o));
+  for (int i = 0; i < 4; ++i) o.src[i] = i;                // COMMAND, BASE_LIN_VEL, BASE_ANG_VEL, GRAVITY_VEC
+  for (int j = 0; j < A1_HEAD; ++j) o.scale[j] = 1.0f;
+  o.h_scale = 1.0f;
+  o.h_bound = std::fmin(d.height_clip, d.clip_obs);
+  custom = false;
+  if (d.obs_layout == 0) return SHIFU_OK;
+  for (int i = 0; i < 4; ++i) {
+    if (d.obs_vec_src[i] < 0 || d.obs_vec_src[i] >= SHIFU_OBS_VEC_COUNT)
+      return fail(SHIFU_E_RANGE, "obs_vec_src[%d]=%d is not an enum ShifuObsVec value", i, d.obs_vec_src[i]);
+    custom |= d.obs_vec_src[i] != i;
+    o.src[i] = d.obs_vec_src[i];
+    o.uses_pg |= d.obs_vec_src[i] == SHIFU_OBS_PROJECTED_GRAVITY;
+  }
+  for (int j = 0; j < A1_HEAD; ++j) {
+    if (!std::isfinite(d.obs_scale[j])) return fail(SHIFU_E_RANGE, "obs_scale[%d]=%g is not finite", j, (double)d.obs_scale[j]);
+    custom |= d.obs_scale[j] != 1.0f;
+    o.scale[j] = d.obs_scale[j];
+  }
+  if (!std::isfinite(d.obs_height_scale))
+    return fail(SHIFU_E_RANGE, "obs_height_scale=%g is not finite", (double)d.obs_height_scale);
+  custom |= d.obs_height_scale != 1.0f;
+  o.h_scale = d.obs_height_scale;
+  o.h_bound = std::fmin(d.height_clip * std::fabs(o.h_scale), d.clip_obs);
+  return SHIFU_OK;
 }
 
 static int fill_a1k(const ShifuA1Desc& d, A1K& k) {
@@ -232,8 +274,12 @@ extern "C" int shifu_ctx_create_util(int device, int32_t num_envs, ShifuCtx** ou
 
 static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc* abb, int util_envs, ShifuCtx** out) {
   // validate the descriptor before touching the device so argument errors surface without a GPU
-  A1K a1k; AbbK abbk;
-  if (a1 != nullptr) { int rc = fill_a1k(*a1, a1k); if (rc) return rc; }
+  A1K a1k; AbbK abbk; A1Obs a1o; bool obs_custom = false;
+  if (a1 != nullptr) {
+    int rc = fill_a1k(*a1, a1k);
+    if (rc == SHIFU_OK) rc = fill_a1obs(*a1, a1o, obs_custom);
+    if (rc) return rc;
+  }
   else if (abb != nullptr) { int rc = fill_abbk(*abb, abbk); if (rc) return rc; }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) {
@@ -251,7 +297,7 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
   c->sm_count = prop.multiProcessorCount;
   int n = 0;
   if (a1 != nullptr) {
-    c->is_a1 = true; c->a1 = *a1; c->a1k = a1k; n = a1->num_envs;
+    c->is_a1 = true; c->a1 = *a1; c->a1k = a1k; c->a1o = a1o; c->obs_custom = obs_custom; n = a1->num_envs;
     c->grid_symmetric = true;
     for (int i = 0; i < A1_NX; ++i) c->grid_symmetric &= (a1k.px[i] == -a1k.px[A1_NX - 1 - i]);
     for (int i = 0; i < A1_NY; ++i) c->grid_symmetric &= (a1k.py[i] == -a1k.py[A1_NY - 1 - i]);
@@ -293,14 +339,14 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
       carve = (int)((need * 100 + smem_sm - 1) / smem_sm);
       if (carve > 100) carve = 100;
     }
-    for (int v = 0; v < 8 && e == cudaSuccess; ++v) {
+    for (int v = 0; v < A1_TMA_VARIANTS && e == cudaSuccess; ++v) {
       e = cudaFuncSetAttribute(tma_variants[v], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(V3Smem));
       if (e == cudaSuccess)
         e = cudaFuncSetAttribute(tma_variants[v], cudaFuncAttributePreferredSharedMemoryCarveout, carve);
     }
     int tocc = 0;
     if (e == cudaSuccess)
-      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tocc, a1_post_physics_tma_kernel<false, false, false>, V3_THREADS,
+      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tocc, a1_post_physics_tma_kernel<false, false, false, false>, V3_THREADS,
                                                         sizeof(V3Smem));
     c->tma_occ = tocc;
     const char* kern = getenv("SHIFU_A1_KERNEL");
@@ -468,9 +514,9 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     bool extra = false;
     for (int q = 0; q < c->a1k.n_terms; ++q) extra |= c->a1k.terms[q] >= SHIFU_REW_LIN_VEL_Z;
     int tiles_arg = full_tiles;
-    void* args[3] = {(void*)&c->a1k, const_cast<ShifuA1StepIO*>(io), (void*)&tiles_arg};
-    CUDA_TRY(cudaLaunchKernel(a1_tma_variants()[(exact ? 4 : 0) + (mrow ? 2 : 0) + (extra ? 1 : 0)], grid, block, args, smem,
-                              S(stream)));
+    void* args[4] = {(void*)&c->a1k, const_cast<ShifuA1StepIO*>(io), (void*)&tiles_arg, (void*)&c->a1o};
+    const int variant = (c->obs_custom ? 8 : 0) + (exact ? 4 : 0) + (mrow ? 2 : 0) + (extra ? 1 : 0);
+    CUDA_TRY(cudaLaunchKernel(a1_tma_variants()[variant], grid, block, args, smem, S(stream)));
   }
   const int done = full_tiles * A1_TILE;
   if (done < n) {
@@ -495,10 +541,11 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     const int tiles = (k.n + A1_TILE - 1) / A1_TILE;
     const int cap = c->sm_count * (c->a1_occ > 0 ? c->a1_occ : 1);
     const dim3 grid(tiles < cap ? tiles : cap), block(A1_THREADS);
-    if (tiled && !exact) a1_post_physics_kernel<true, false><<<grid, block, 0, S(stream)>>>(k, t);
-    else if (tiled && exact) a1_post_physics_kernel<true, true><<<grid, block, 0, S(stream)>>>(k, t);
-    else if (!tiled && !exact) a1_post_physics_kernel<false, false><<<grid, block, 0, S(stream)>>>(k, t);
-    else a1_post_physics_kernel<false, true><<<grid, block, 0, S(stream)>>>(k, t);
+    const A1Obs& o = c->a1o;
+    if (tiled && !exact) a1_post_physics_kernel<true, false><<<grid, block, 0, S(stream)>>>(k, t, o);
+    else if (tiled && exact) a1_post_physics_kernel<true, true><<<grid, block, 0, S(stream)>>>(k, t, o);
+    else if (!tiled && !exact) a1_post_physics_kernel<false, false><<<grid, block, 0, S(stream)>>>(k, t, o);
+    else a1_post_physics_kernel<false, true><<<grid, block, 0, S(stream)>>>(k, t, o);
     CUDA_TRY(cudaGetLastError());
   }
   return SHIFU_OK;

@@ -10,7 +10,8 @@ of the fused kernels computes.  The proof has three parts, none of which reads s
   sampling, curriculum, the PD loop — they are stochastic or call the simulator) the set of
   attribute names and literals their code objects reference (``co_names`` / ``co_consts``;
   stable across Python versions, unlike bytecode);
-* **term compilation** (``shifu_b200.terms``): reward hooks -> (opcode, constants) by probing;
+* **term compilation** (``shifu_b200.terms``): reward hooks -> (opcode, constants) and the observation
+  hook -> its layout (slot sources, column scales, height scale), by probing;
 * **numerical check**: reward hooks against ``shifu_a1_eval_terms``; observation and termination
   hooks against the layout / predicates the kernel implements, on a seeded random state.
 
@@ -27,8 +28,7 @@ from shifu_b200 import hotpath, terms
 from shifu_b200 import _native as nv
 
 
-class NotFusable(Exception):
-    pass
+NotFusable = terms.NotFusable
 
 
 def _code(fn):
@@ -90,15 +90,7 @@ def _overridden(obj, name: str, base) -> bool:
     return getattr(type(obj), name, None) is not getattr(base, name, None)
 
 
-def _close(a: torch.Tensor, b: torch.Tensor, what: str, rtol=1e-6, atol=1e-7):
-    if a.shape != b.shape:
-        raise NotFusable(f"{what}: shape {tuple(a.shape)} != {tuple(b.shape)}")
-    if a.dtype == torch.bool or b.dtype == torch.bool:
-        bad = int((a.bool() != b.bool()).sum())
-    else:
-        bad = int(((a.float() - b.float()).abs() > atol + rtol * b.float().abs()).sum())
-    if bad:
-        raise NotFusable(f"{what}: the Python hook differs from the fused kernel's definition on {bad} entries")
+_close = terms.check_close
 
 
 # =============================================================================================
@@ -163,6 +155,8 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
     # ---- reward terms: match + fit ------------------------------------------------------------
     compiled = terms.compile_a1_terms(env, env.reward_functions)
     names = [t.name for t in compiled]
+    # ---- observation: slot sources and scales -------------------------------------------------
+    obs = terms.compile_a1_obs(env)
     # ---- the hot path over the env's own tensors -----------------------------------------------
     desc = hotpath.a1_desc(
         env.num_envs, env_offset=getattr(env, "env_offset", 0), rng_seed=rng_seed,
@@ -178,7 +172,7 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
         force_body=force_body, root_stride=layout[0], root_offset=layout[1],
         action_scale=1.0,                        # a subclass step() has already scaled (a1_conditional.py:122-124)
         clip_actions=float(env.clip_actions), clip_obs=float(env.clip_obs),
-        air_time_reset=air_time_reset,
+        air_time_reset=air_time_reset, obs=obs,
         **terms.desc_extras(compiled))
     desc.push_force_max = float(forces[0])
     desc.cmd_low[0], desc.cmd_high[0] = env.cmd_lin_vel_x
@@ -199,25 +193,19 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
         hp.adopt(swing_time=air[0], last_contacts=air[1])
     # ---- numerical checks ----------------------------------------------------------------------
     terms.verify_a1_terms(env, hp, env.reward_functions, compiled)
-    _check_a1_obs_and_termination(env)
+    terms.verify_a1_obs(env, obs)
+    _check_a1_termination(env)
     return hp
 
 
-def _check_a1_obs_and_termination(env):
-    """compute_observations / compute_termination against the kernel's definition (a1_conditional.py:
-    131-150) on a random state."""
+def _check_a1_termination(env):
+    """compute_termination against the kernel's definition (a1_conditional.py:146-150) on a random state."""
     rb, isg = env.robot, env.isg_env
     with terms.A1Probe(env) as pr:
         pr.randomize(4321)
         had = isg.__dict__.get("_measured_heights")
         isg.measured_heights = torch.randn(env.num_envs, isg.num_height_points, device=env.device)
         try:
-            env.compute_observations()
-            heights = torch.clip(rb.base_pose[:, 2].unsqueeze(1) - 0.5 - isg.measured_heights, -1, 1.)
-            want = torch.cat([env.command_buf, rb.base_lin_vel, rb.base_ang_vel, rb.gravity_vec,
-                              rb.dof_pos - rb.default_dof_pos, rb.dof_vel, env.actions_recorder.flatten(), heights],
-                             dim=1)
-            _close(env.obs_buf, want, "compute_observations")
             env.compute_termination()
             force = rb.contact_forces[:, int(env.contact_terminate_indices), :]
             contact = torch.norm(force, dim=-1) > 1.

@@ -12,8 +12,11 @@ class API; tests and ``bench.py`` may also drive them directly.
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, List, Optional, Sequence
+import math
+from dataclasses import dataclass
+from typing import Dict, List, Optional, Sequence, Tuple
 
+import numpy as np
 import torch
 
 from . import _native as nv
@@ -37,6 +40,45 @@ A1_TERM_PARAMS = {
 ABB_TERM_CODES = {"reward_reaching": nv.REW_ABB_REACHING, "reward_success": nv.REW_ABB_SUCCESS}
 # examples/abb_pushbox_vision/a_prior_stage.py:118-131
 ABB_TERM_PARAMS = {"reward_reaching": (0.1, 0.05), "reward_success": (200.0, 0.02)}
+
+
+# enum ShifuObsVec: the sources a 3-column vector slot of the observation head can take
+OBS_SOURCES = {"COMMAND": nv.OBS_COMMAND, "BASE_LIN_VEL": nv.OBS_BASE_LIN_VEL, "BASE_ANG_VEL": nv.OBS_BASE_ANG_VEL,
+               "GRAVITY_VEC": nv.OBS_GRAVITY_VEC, "PROJECTED_GRAVITY": nv.OBS_PROJECTED_GRAVITY}
+A1_OBS_SLOTS = ("COMMAND", "BASE_LIN_VEL", "BASE_ANG_VEL", "GRAVITY_VEC")      # a1_conditional.py:137-140
+
+
+@dataclass(frozen=True)
+class ObsLayout:
+    """Layout of the 259-column A1 observation the fused kernel builds.
+
+    Columns 0-11 are four 3-column slots, ``slots[i]`` naming the source of columns 3i..3i+2 (a key of
+    ``OBS_SOURCES``); every head column j < 72 is ``clip(x_j * scales[j], +-clip_obs)`` (the dof-position
+    columns' x_j is ``dof_pos - default_dof_pos``); the 187 heights are
+    ``clip(clip(z - 0.5 - h, +-1) * height_scale, +-clip_obs)``, legged_gym's clip-then-scale order.
+    PROJECTED_GRAVITY is the value the tensor holds when the step starts (``LeggedRobot.post_step`` on
+    the previous state, like the body-frame velocities).  Scales are kept as fp32 values."""
+    slots: Tuple[str, str, str, str] = A1_OBS_SLOTS
+    scales: Tuple[float, ...] = (1.0,) * nv.OBS_HEAD
+    height_scale: float = 1.0
+
+    def __post_init__(self):
+        slots = tuple(self.slots)
+        if len(slots) != 4 or any(s not in OBS_SOURCES for s in slots):
+            raise ValueError(f"slots must be 4 names out of {sorted(OBS_SOURCES)}, got {slots}")
+        scales = tuple(float(np.float32(v)) for v in self.scales)
+        if len(scales) != nv.OBS_HEAD:
+            raise ValueError(f"{len(scales)} column scales: the observation head has {nv.OBS_HEAD} columns")
+        hs = float(np.float32(self.height_scale))
+        if not all(math.isfinite(v) for v in (*scales, hs)):
+            raise ValueError("observation scales must be finite")
+        object.__setattr__(self, "slots", slots)
+        object.__setattr__(self, "scales", scales)
+        object.__setattr__(self, "height_scale", hs)
+
+    def is_reference(self) -> bool:
+        """The reference observation (a1_conditional.py:131-144): identity scales, reference slots."""
+        return self.slots == A1_OBS_SLOTS and all(v == 1.0 for v in self.scales) and self.height_scale == 1.0
 
 
 def compile_reward_terms(names: Sequence[str], codes: Dict[str, int], params: Dict[str, tuple]):
@@ -72,8 +114,9 @@ def a1_desc(num_envs: int, *, env_offset: int = 0, rng_seed: int = 0x5EED,
             leg_bodies=(2, 3, 6, 7, 10, 11, 14, 15), force_body=0, root_stride=1, root_offset=0,
             action_scale=0.5, clip_actions=1., clip_obs=100.,
             dof_pos_limits=None, feet_bodies=(4, 8, 12, 16), feet_contact_force=1.0, air_time_cmd_min=0.1,
-            air_time_dt=0.02, air_time_reset=True) -> nv.A1Desc:
-    """Defaults = the constants of ``examples/a1_conditional`` (SURVEY.md Appendix A)."""
+            air_time_dt=0.02, air_time_reset=True, obs: Optional[ObsLayout] = None) -> nv.A1Desc:
+    """Defaults = the constants of ``examples/a1_conditional`` (SURVEY.md Appendix A).  ``obs``: the
+    observation layout; ``None`` or the reference layout writes ``obs_layout = 0``."""
     d = nv.A1Desc()
     d.abi_version = nv.ABI_VERSION
     d.num_envs, d.env_offset, d.rng_seed = num_envs, env_offset, rng_seed
@@ -121,6 +164,13 @@ def a1_desc(num_envs: int, *, env_offset: int = 0, rng_seed: int = 0x5EED,
     for i, (code, p0, p1) in enumerate(comp):
         d.reward_terms[i] = code
         d.reward_params[i][0], d.reward_params[i][1] = p0, p1
+    if obs is not None and not obs.is_reference():
+        d.obs_layout = 1
+        for i, name in enumerate(obs.slots):
+            d.obs_vec_src[i] = OBS_SOURCES[name]
+        for j, v in enumerate(obs.scales):
+            d.obs_scale[j] = v
+        d.obs_height_scale = obs.height_scale
     return d
 
 

@@ -165,6 +165,16 @@ class A1Conditional(ShifuVecEnv):
         if layout is None:
             raise NotImplementedError("the fused A1 kernel needs affine root_indices")
         names = [fn.__name__ for fn in self.reward_functions]
+        obs = None
+        if type(self).compute_observations is not A1Conditional.compute_observations:
+            # an edited observation hook: fused only when the kernel's observation layout expresses it,
+            # never silently replaced by the reference observation
+            from shifu_b200 import terms
+            try:
+                obs = terms.compile_a1_obs(self)
+                terms.verify_a1_obs(self, obs)
+            except terms.NotFusable as exc:
+                raise NotImplementedError(f"{exc} (fused=False runs any observation hook)") from exc
         desc = hotpath.a1_desc(
             self.num_envs, env_offset=self.env_offset, rng_seed=self.rng_seed, terms=names,
             q0=tuple(rb.cfg.default_dof_pos), kp=tuple(float(v) for v in rb.cfg.dof_stiffness),
@@ -178,7 +188,7 @@ class A1Conditional(ShifuVecEnv):
             env_length=isg.terrain.env_length, base_body=int(self.contact_terminate_indices),
             leg_bodies=tuple(rb.leg_indices.tolist()), force_body=rb.rigid_body_dict['base'],
             root_stride=layout[0], root_offset=layout[1], clip_actions=float(self.clip_actions),
-            clip_obs=float(self.clip_obs))
+            clip_obs=float(self.clip_obs), obs=obs)
         hp = hotpath.A1HotPath(desc, root_state=isg.root_state, dof_state=isg.dof_state,
                                contact_state=isg.contact_state, height_samples=isg.height_samples,
                                terrain_origins=isg.terrain_origins, terrain_types=isg.terrain_types,

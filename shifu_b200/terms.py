@@ -1,4 +1,5 @@
-"""Reward-term compiler (SURVEY.md §8f row N1): ``build_reward_functions()`` lists -> fused term descriptors.
+"""Reward / observation term compiler (SURVEY.md §8f row N1): ``build_reward_functions()`` lists -> fused term
+descriptors, ``compute_observations`` -> the fused observation layout (:func:`compile_a1_obs`).
 
 The reference's "registry" is a plain list of bound methods whose weights are literals inside each
 body (``shifu/gym/env.py:78-80,160-166,180-185``; ``a1_conditional.py:152-192``).  To fuse such a
@@ -28,12 +29,29 @@ from typing import Callable, Dict, List, Optional, Sequence, Tuple
 import torch
 
 from . import _native as nv
+from .hotpath import OBS_SOURCES, ObsLayout
 
 RTOL, ATOL = 2e-5, 2e-6
 
 
 class TermMismatch(Exception):
     """The user's hook is not (numerically) the library term it was matched to."""
+
+
+class NotFusable(Exception):
+    """A hook of the env is not what the fused kernel computes; the message names the hook and the reason."""
+
+
+def check_close(a: torch.Tensor, b: torch.Tensor, what: str, rtol=1e-6, atol=1e-7):
+    """Raise NotFusable unless the hook's result ``a`` is the fused definition ``b``."""
+    if a.shape != b.shape:
+        raise NotFusable(f"{what}: shape {tuple(a.shape)} != {tuple(b.shape)}")
+    if a.dtype == torch.bool or b.dtype == torch.bool:
+        bad = int((a.bool() != b.bool()).sum())
+    else:
+        bad = int(((a.float() - b.float()).abs() > atol + rtol * b.float().abs()).sum())
+    if bad:
+        raise NotFusable(f"{what}: the Python hook differs from the fused kernel's definition on {bad} entries")
 
 
 @dataclass
@@ -94,6 +112,7 @@ class A1Probe:
         rb, isg = self.robot, self.isg
         self.tensors = {
             "command": env.command_buf, "lin": rb.base_lin_vel, "ang": rb.base_ang_vel, "pg": rb.projected_gravity,
+            "gvec": rb.gravity_vec,
             "history": env.actions_recorder.history_buf, "contact": isg.contact_state, "torques": rb.torques,
             "dof": isg.dof_state, "root": isg.root_state, "actions": env.actions,
             "ep_len": env.episode_length_buf,
@@ -321,3 +340,169 @@ def verify_a1_terms(env, hot, functions: Sequence[Callable], terms: Sequence[Com
             raise TermMismatch(f"reward term {term.name!r}: the Python hook and the fused term (code {term.code}, "
                                f"p0={term.p0:g}, p1={term.p1:g}) differ on {bad} of {err.numel()} envs "
                                f"(max abs err {float(err.max()):.3e})")
+
+
+# ---------------------------------------------------------------------------------------------
+# Observation layout (ObsLayout): which source feeds each vector slot, and every column's scale
+# ---------------------------------------------------------------------------------------------
+
+_OBS_PROBE = {"COMMAND": ("command", "command_buf"), "BASE_LIN_VEL": ("lin", "base_lin_vel"),
+              "BASE_ANG_VEL": ("ang", "base_ang_vel"), "GRAVITY_VEC": ("gvec", "gravity_vec"),
+              "PROJECTED_GRAVITY": ("pg", "projected_gravity")}
+assert set(_OBS_PROBE) == set(OBS_SOURCES)
+
+
+def _exact_offset(q0: float) -> float:
+    """A power of two v with fp32 (q0 + v) - q0 == v: a dof-position probe whose dof_pos - q0 is exact."""
+    q = torch.tensor(q0, dtype=torch.float)
+    for k in range(0, 40):
+        v = 2.0 ** -k
+        if float((q + v) - q) == v:
+            return v
+    raise NotFusable(f"compute_observations: no exact dof-position probe around {q0}")
+
+
+def compile_a1_obs(env) -> ObsLayout:
+    """``env.compute_observations`` -> ObsLayout, by probing.  At the zero state (every input zero,
+    dof_pos = default_dof_pos, base 0.5 above flat terrain) the observation must be all zeros; then each
+    input is set alone to a power of two and must reach exactly one column of its block, the three
+    components of a vector in order in one slot; the column's value over the input is its scale.  The
+    heights are probed at z - 0.5 - h = 0.5 and 3, which fixes their scale and the clip-then-scale order.
+    Anything else raises NotFusable naming the column and the reason."""
+    rb, isg = env.robot, env.isg_env
+    n_head = nv.OBS_HEAD
+    had = isg.__dict__.get("_measured_heights")
+    with A1Probe(env) as pr:
+        t = pr.tensors
+        heights = torch.zeros(env.num_envs, isg.num_height_points, device=env.device)
+        dof = t["dof"].view(env.num_envs, -1, 2)
+        q0 = rb.default_dof_pos
+        rows0 = rb.root_indices[0]
+
+        def zero_state():
+            pr.zero()
+            dof[:, :, 0] = q0
+            t["root"][rb.root_indices, 2] = 0.5
+            heights.zero_()
+
+        def observe():
+            isg.measured_heights = heights
+            env.compute_observations()
+            obs = env.obs_buf
+            if tuple(obs.shape) != (env.num_envs, n_head + heights.shape[1]):
+                raise NotFusable(f"compute_observations: shape {tuple(obs.shape)}, the fused observation is "
+                                 f"({env.num_envs}, {n_head + heights.shape[1]})")
+            return obs[0].float().cpu()
+
+        def lit(o, lo=0, hi=n_head):
+            return [(j, float(o[j])) for j in torch.nonzero(o[lo:hi]).flatten().add(lo).tolist()]
+
+        try:
+            zero_state()
+            for j, v in lit(observe(), 0, None):
+                raise NotFusable(f"compute_observations: column {j} is {v:g} with every input at zero (dof_pos = "
+                                 "default_dof_pos, base height 0.5 above the terrain): the fused observation has "
+                                 "no additive offsets")
+            slots, scales = [None] * 4, [None] * n_head
+            for name, (key, label) in _OBS_PROBE.items():
+                cols = []
+                for c in range(3):
+                    zero_state()
+                    t[key][0, c] = 1.0
+                    cols.append(lit(observe(), 0, None))
+                if not any(cols):
+                    continue                                        # source not observed
+                for c, hits in enumerate(cols):
+                    if len(hits) != 1:
+                        raise NotFusable(f"compute_observations: {label}[:, {c}] reaches columns "
+                                         f"{[j for j, _ in hits]}; it must reach exactly one column")
+                    j = hits[0][0]
+                    if j >= 12 or j % 3 != c or j // 3 != cols[0][0][0] // 3:
+                        raise NotFusable(f"compute_observations: column {j} reads {label}[:, {c}]; the fused "
+                                         "observation takes a vector whole, in order, into one of the slots at "
+                                         "columns 0-2, 3-5, 6-8, 9-11")
+                slot = cols[0][0][0] // 3
+                if slots[slot] is not None:
+                    raise NotFusable(f"compute_observations: columns {3 * slot}-{3 * slot + 2} read both "
+                                     f"{_OBS_PROBE[slots[slot]][1]} and {label}; a column takes one source")
+                slots[slot] = name
+                for c in range(3):
+                    scales[3 * slot + c] = cols[c][0][1]
+            for i, src in enumerate(slots):
+                if src is None:
+                    raise NotFusable(f"compute_observations: columns {3 * i}-{3 * i + 2} follow none of "
+                                     f"{[label for _, label in _OBS_PROBE.values()]}")
+            # dof positions (dof_pos - default_dof_pos), dof velocities, history slot-major
+            probes = []
+            for d in range(12):
+                probes.append((12 + d, f"dof_pos[:, {d}] - default_dof_pos[{d}]", ("dof", d, 0)))
+                probes.append((24 + d, f"dof_vel[:, {d}]", ("dof", d, 1)))
+                for h in range(3):
+                    probes.append((36 + 12 * h + d, f"actions_recorder.get_last({h})[:, {d}]", ("history", d, h)))
+            for col, label, (key, a, b) in probes:
+                zero_state()
+                if key == "dof" and b == 0:
+                    x = _exact_offset(float(q0[a]))
+                    dof[0, a, 0] = float(torch.tensor(float(q0[a]), dtype=torch.float) + x)
+                else:
+                    x = 1.0
+                    (dof if key == "dof" else t["history"])[0, a, b] = x
+                hits = lit(observe(), 0, None)
+                if len(hits) != 1 or hits[0][0] != col:
+                    raise NotFusable(f"compute_observations: {label} reaches columns {[j for j, _ in hits]}; the "
+                                     f"fused observation has it in column {col} alone")
+                scales[col] = hits[0][1] / x
+            # heights: clip(z - 0.5 - h, +-1) * height_scale
+            zero_state()
+            heights[0] = -0.5
+            o = observe()
+            for j, v in lit(o):
+                raise NotFusable(f"compute_observations: column {j} follows the measured heights")
+            hv = o[n_head:]
+            hs = float(hv[0]) / 0.5
+            if hs == 0.0 or not bool((hv == hv[0]).all()):
+                raise NotFusable("compute_observations: the height columns are not one scale times "
+                                 "clip(base z - 0.5 - measured_heights, -1, 1)")
+            heights[0] = -3.0
+            hv = observe()[n_head:]
+            bad = torch.nonzero(hv != hs).flatten().tolist()
+            if bad:
+                raise NotFusable(f"compute_observations: height column {n_head + bad[0]} is {float(hv[bad[0]]):g} at "
+                                 f"z - 0.5 - h = 3, not clip(3, -1, 1) * {hs:g}: heights must be clipped to +-1 "
+                                 "before they are scaled")
+        finally:
+            if had is None:
+                del isg.measured_heights
+            else:
+                isg.measured_heights = had
+    return ObsLayout(tuple(slots), tuple(scales), hs)
+
+
+def a1_obs_definition(env, layout: ObsLayout) -> torch.Tensor:
+    """The observation the fused kernel builds under ``layout``, in torch on the env's tensors (before the
+    final clip to +-clip_obs that the base class applies)."""
+    rb, isg = env.robot, env.isg_env
+    src = {name: getattr(rb if key != "command" else env, label) for name, (key, label) in _OBS_PROBE.items()}
+    head = torch.cat([src[name] for name in layout.slots]
+                     + [rb.dof_pos - rb.default_dof_pos, rb.dof_vel, env.actions_recorder.flatten()], dim=1)
+    head = head * torch.tensor(layout.scales, dtype=torch.float, device=head.device)
+    heights = torch.clip(rb.base_pose[:, 2].unsqueeze(1) - 0.5 - isg.measured_heights, -1, 1.) * layout.height_scale
+    return torch.cat([head, heights], dim=1)
+
+
+def verify_a1_obs(env, layout: ObsLayout, seed: int = 4321):
+    """``env.compute_observations`` against the layout's definition on a seeded random state."""
+    isg = env.isg_env
+    had = isg.__dict__.get("_measured_heights")
+    with A1Probe(env) as pr:
+        pr.randomize(seed)
+        g = torch.Generator(device=env.device).manual_seed(seed)
+        isg.measured_heights = torch.randn(env.num_envs, isg.num_height_points, generator=g, device=env.device)
+        try:
+            env.compute_observations()
+            check_close(env.obs_buf, a1_obs_definition(env, layout), "compute_observations")
+        finally:
+            if had is None:
+                del isg.measured_heights
+            else:
+                isg.measured_heights = had
