@@ -17,6 +17,10 @@ of the fused kernels computes.  The proof has three parts, none of which reads s
 
 Anything that fails leaves the env in user-hook mode (eager torch hooks on CUDA tensors, with the
 base-class rows still done by kernels) and records the reason in ``env.fusion_report``.
+
+The task classes of ``shifu_b200.tasks`` fuse explicitly, without the proof, through the same
+pieces: the descriptor builders (``a1_env_desc``, ``abb_hot_path``), the bindings (``bind_a1``,
+``bind_abb``) and ``install``, which routes ``step`` / ``reset_idx`` to the fused kernels.
 """
 from __future__ import annotations
 
@@ -158,31 +162,11 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
     # ---- observation: slot sources and scales -------------------------------------------------
     obs = terms.compile_a1_obs(env)
     # ---- the hot path over the env's own tensors -----------------------------------------------
-    desc = hotpath.a1_desc(
-        env.num_envs, env_offset=getattr(env, "env_offset", 0), rng_seed=rng_seed,
-        terms=[(t.name, t.code, t.p0, t.p1) for t in compiled],
-        q0=tuple(rb.cfg.default_dof_pos), kp=tuple(float(v) for v in rb.p_gains.tolist()),
-        kd=tuple(float(v) for v in rb.d_gains.tolist()), torque_limit=tuple(rb.torque_limits.tolist()),
-        points_x=tuple(tc.measured_points_x), points_y=tuple(tc.measured_points_y),
-        border_size=float(tc.border_size), horizontal_scale=tc.horizontal_scale, vertical_scale=tc.vertical_scale,
-        max_episode_length=int(env.max_episode_length), max_episode_length_s=float(env.max_episode_length_s),
-        default_root=tuple(rb.cfg.default_pos) + tuple(rb.cfg.default_quat), curriculum=tc.curriculum,
-        max_terrain_level=isg.max_terrain_level, num_terrain_types=tc.num_cols, env_length=isg.terrain.env_length,
-        base_body=int(env.contact_terminate_indices), leg_bodies=tuple(rb.leg_indices.tolist()),
-        force_body=force_body, root_stride=layout[0], root_offset=layout[1],
-        action_scale=1.0,                        # a subclass step() has already scaled (a1_conditional.py:122-124)
-        clip_actions=float(env.clip_actions), clip_obs=float(env.clip_obs),
-        air_time_reset=air_time_reset, obs=obs,
-        **terms.desc_extras(compiled))
-    desc.push_force_max = float(forces[0])
-    desc.cmd_low[0], desc.cmd_high[0] = env.cmd_lin_vel_x
-    desc.cmd_low[1], desc.cmd_high[1] = env.cmd_lin_vel_y
-    desc.cmd_low[2], desc.cmd_high[2] = env.cmd_ang_vel_yaw
-    hp = hotpath.A1HotPath(desc, root_state=isg.root_state, dof_state=isg.dof_state, contact_state=isg.contact_state,
-                           height_samples=isg.height_samples, terrain_origins=isg.terrain_origins,
-                           terrain_types=isg.terrain_types, env_origins=isg.env_origins, terms=names,
-                           carry_body_frame=carry_body_frame,
-                           want_measured_heights=bool(getattr(cfg, "store_measured_heights", False)))
+    desc = a1_env_desc(env, [(t.name, t.code, t.p0, t.p1) for t in compiled], rng_seed=rng_seed, obs=obs,
+                       action_scale=1.0,         # a subclass step() has already scaled (a1_conditional.py:122-124)
+                       force_body=force_body, push_force_max=float(forces[0]), air_time_reset=air_time_reset,
+                       **terms.desc_extras(compiled))
+    hp = a1_hot_path(env, desc, names, carry_body_frame, bool(getattr(cfg, "store_measured_heights", False)))
     # the probes below run the user's hooks on the env's CURRENT tensors: point the hot path at them
     hp.adopt(actions=env.actions, history=env.actions_recorder.history_buf, command=env.command_buf,
              torques=rb.torques, base_lin_vel=rb.base_lin_vel, base_ang_vel=rb.base_ang_vel,
@@ -219,8 +203,44 @@ def _check_a1_termination(env):
                 isg.measured_heights = had
 
 
+def a1_env_desc(env, terms, *, rng_seed: int, force_body: int, push_force_max: float, **kw) -> nv.A1Desc:
+    """``hotpath.a1_desc`` of an A1-shaped env: dof gains and limits from its robot, the point grid and
+    terrain scales from its config, curriculum, levels and env length from its gym env, and its episode
+    lengths, clips and command ranges.  ``terms`` and ``kw`` (``obs``, ``action_scale``, ``air_time_reset``,
+    the compiled terms' extras) go to ``a1_desc`` as they are."""
+    rb, isg, tc = env.robot, env.isg_env, env.cfg.terrain
+    stride, offset = rb.affine_root_layout()
+    desc = hotpath.a1_desc(
+        env.num_envs, env_offset=env.env_offset, rng_seed=rng_seed, terms=terms,
+        q0=tuple(rb.cfg.default_dof_pos), kp=tuple(float(v) for v in rb.p_gains.tolist()),
+        kd=tuple(float(v) for v in rb.d_gains.tolist()), torque_limit=tuple(rb.torque_limits.tolist()),
+        points_x=tuple(tc.measured_points_x), points_y=tuple(tc.measured_points_y),
+        border_size=float(tc.border_size), horizontal_scale=tc.horizontal_scale, vertical_scale=tc.vertical_scale,
+        max_episode_length=int(env.max_episode_length), max_episode_length_s=float(env.max_episode_length_s),
+        default_root=tuple(rb.cfg.default_pos) + tuple(rb.cfg.default_quat), curriculum=tc.curriculum,
+        max_terrain_level=isg.max_terrain_level, num_terrain_types=tc.num_cols, env_length=isg.terrain.env_length,
+        base_body=int(env.contact_terminate_indices), leg_bodies=tuple(rb.leg_indices.tolist()),
+        force_body=force_body, root_stride=stride, root_offset=offset,
+        clip_actions=float(env.clip_actions), clip_obs=float(env.clip_obs), **kw)
+    desc.push_force_max = push_force_max
+    desc.cmd_low[0], desc.cmd_high[0] = env.cmd_lin_vel_x
+    desc.cmd_low[1], desc.cmd_high[1] = env.cmd_lin_vel_y
+    desc.cmd_low[2], desc.cmd_high[2] = env.cmd_ang_vel_yaw
+    return desc
+
+
+def a1_hot_path(env, desc: nv.A1Desc, names, carry_body_frame: bool, want_measured_heights: bool) -> hotpath.A1HotPath:
+    """An ``A1HotPath`` for ``desc`` over the env's gym tensors."""
+    isg = env.isg_env
+    return hotpath.A1HotPath(desc, root_state=isg.root_state, dof_state=isg.dof_state, contact_state=isg.contact_state,
+                             height_samples=isg.height_samples, terrain_origins=isg.terrain_origins,
+                             terrain_types=isg.terrain_types, env_origins=isg.env_origins, terms=names,
+                             carry_body_frame=carry_body_frame, want_measured_heights=want_measured_heights)
+
+
 def bind_a1(env, hp):
-    """Make the env / robot attributes BE the tensors the kernel reads and writes."""
+    """Make the env / robot attributes BE the tensors the kernel reads and writes, and derive the
+    body-frame velocities the first step reads from the current root rows."""
     rb, isg = env.robot, env.isg_env
     env.actions, env.obs_buf, env.rew_buf, env.reset_buf = hp.actions, hp.obs_buf, hp.rew_buf, hp.reset_buf
     env._episode_length_buf = hp.ep_len
@@ -234,6 +254,7 @@ def bind_a1(env, hp):
     isg.measured_heights = hp.measured_heights          # None unless cfg.store_measured_heights: filled on demand
     isg.__dict__["_heights_on_demand"] = hp.measured_heights is None
     env.extras.update(hp.extras())
+    hp.body_frame()
 
 
 def _resident_state(env) -> bool:
@@ -268,25 +289,9 @@ def a1_fused_step(env, hp, actions: torch.Tensor):
     isg.refresh_state()
     hp.post_physics()
     hp.finalize(env.stats_allreduce)
-    if getattr(gym, "needs_indexed_resets", True):
-        ids = hp.reset_id_list()
-        if len(ids):
-            rb.push_dof_reset(ids)
-            isg.push_root_reset(ids)
+    push_resets(env, hp)
     env.extras.update(hp.extras())
     return env.obs_buf, env.privileged_obs_buf, env.rew_buf, env.reset_buf, env.extras
-
-
-def a1_fused_reset_idx(env, hp, env_ids):
-    hp.step_counter = env.common_step_counter
-    hp.reset_idx(env_ids, env.stats_allreduce)
-    gym = env.isg_env.gym
-    if getattr(gym, "needs_indexed_resets", True):
-        ids = torch.arange(env.num_envs, device=env.device) if env_ids is None else env_ids
-        if len(ids):
-            env.robot.push_dof_reset(ids)
-            env.isg_env.push_root_reset(ids)
-    env.extras.update(hp.extras())
 
 
 # =============================================================================================
@@ -295,7 +300,7 @@ def a1_fused_reset_idx(env, hp, env_ids):
 
 def fuse_abb(env, rng_seed: int = 0x5EED):
     from shifu_b200.units import ArmRobot, Box
-    isg, cfg = env.isg_env, env.cfg
+    cfg = env.cfg
     rb = getattr(env, "robot", None)
     if not isinstance(rb, ArmRobot) or not all(isinstance(getattr(env, a, None), Box) for a in ("table", "cube", "goal")):
         raise NotFusable("needs an ArmRobot with table / cube / goal boxes")
@@ -313,11 +318,19 @@ def fuse_abb(env, rng_seed: int = 0x5EED):
     names = [fn.__name__ for fn in env.reward_functions]
     if names != ["reward_reaching", "reward_success"]:
         raise NotFusable(f"reward list {names} is not [reward_reaching, reward_success]")
-    params = _fit_abb_terms(env)
-    desc = hotpath.abb_desc(env.num_envs, env_offset=getattr(env, "env_offset", 0), rng_seed=rng_seed, terms=names,
-                            term_params=params)
+    return abb_hot_path(env, rng_seed, _fit_abb_terms(env))
+
+
+def abb_hot_path(env, rng_seed: int, term_params: Dict[str, tuple]) -> hotpath.AbbHotPath:
+    """An ``AbbHotPath`` over the env's gym tensors, its descriptor read off the 4-actor scene (layout,
+    robot and table poses, end-effector box, cube and goal ranges) with the given reward constants."""
+    isg, rb = env.isg_env, env.robot
+    actors = [rb, env.table, env.cube, env.goal]
+    names = [fn.__name__ for fn in env.reward_functions]
+    desc = hotpath.abb_desc(env.num_envs, env_offset=env.env_offset, rng_seed=rng_seed, terms=names,
+                            term_params=term_params)
     desc.num_actors = len(actors)
-    desc.robot_actor, desc.table_actor, desc.cube_actor, desc.goal_actor = (l[1] for l in layouts)
+    desc.robot_actor, desc.table_actor, desc.cube_actor, desc.goal_actor = (a.affine_root_layout()[1] for a in actors)
     desc.num_bodies = sum(a.num_bodies for a in actors)
     desc.num_dof, desc.ee_body = rb.num_dof, int(rb.ee_indices[0])
     for i in range(3):
@@ -330,7 +343,7 @@ def fuse_abb(env, rng_seed: int = 0x5EED):
     for i, v in enumerate([*env.table.cfg.default_pos, *env.table.cfg.default_quat]):
         desc.table_root[i] = v
     desc.goal_z = env.goal.pos_range["low"][2]
-    desc.success_distance = params["reward_success"][1]
+    desc.success_distance = term_params["reward_success"][1]
     desc.max_episode_length, desc.max_episode_length_s = int(env.max_episode_length), float(env.max_episode_length_s)
     desc.clip_obs = float(env.clip_obs)
     return hotpath.AbbHotPath(desc, root_state=isg.root_state, body_state=isg.body_state, dof_state=isg.dof_state,
@@ -418,12 +431,20 @@ def abb_fused_step(env, hp, actions: torch.Tensor):
     hp.step_counter = env.common_step_counter - 1
     hp.post_physics()
     hp.finalize(env.stats_allreduce)
-    _push_abb(env, hp, None)
+    push_resets(env, hp)
     env.extras.update(hp.extras())
     return env.obs_buf, env.privileged_obs_buf, env.rew_buf, env.reset_buf, env.extras
 
 
-def _push_abb(env, hp, env_ids):
+# =============================================================================================
+# both recipes
+# =============================================================================================
+
+def push_resets(env, hp, env_ids: Optional[torch.Tensor] = None):
+    """Indexed setters of the simulator for the rows the kernel rewrote (isaac_gym.py:70-73,
+    robot.py:78-86): ``env_ids``, or the step's compacted reset ids when None.  They need the id count
+    on the host (one sync, like the reference's ``nonzero``); the stand-in simulator has no hidden
+    state and skips this."""
     if not getattr(env.isg_env.gym, "needs_indexed_resets", True):
         return
     ids = hp.reset_id_list() if env_ids is None else env_ids
@@ -432,28 +453,38 @@ def _push_abb(env, hp, env_ids):
         env.isg_env.push_root_reset(ids)
 
 
-def abb_fused_reset_idx(env, hp, env_ids):
+def fused_reset_idx(env, hp, env_ids: Optional[torch.Tensor]):
+    """``reset_idx`` of a fused env in one launch (env.py:114-130 with the task's reset hooks);
+    ``None`` = all envs.  ``extras`` keeps pointing at the hot path's ring, never a detached dict."""
     hp.step_counter = env.common_step_counter
     hp.reset_idx(env_ids, env.stats_allreduce)
-    _push_abb(env, hp, torch.arange(env.num_envs, device=env.device) if env_ids is None else env_ids)
+    push_resets(env, hp, torch.arange(env.num_envs, device=env.device) if env_ids is None else env_ids)
     env.extras.update(hp.extras())
 
 
-RECIPES = (("a1", fuse_a1, bind_a1, a1_fused_step, a1_fused_reset_idx),
-           ("abb", fuse_abb, bind_abb, abb_fused_step, abb_fused_reset_idx))
+RECIPES = {"a1": (fuse_a1, bind_a1, a1_fused_step), "abb": (fuse_abb, bind_abb, abb_fused_step)}
+
+
+def install(env, recipe: str, hp):
+    """Run the env on ``hp``: bind its attributes to the hot path's tensors, and route ``step`` (through
+    ``ShifuVecEnv.step``) and ``reset_idx`` (which a subclass may override: it is part of what got
+    fused) to the fused kernels."""
+    _, bind, step = RECIPES[recipe]
+    bind(env, hp)
+    env.hot, env._fusion, env._fusion_tried = hp, (recipe, hp, step), True
+    env.reset_idx = lambda env_ids: fused_reset_idx(env, hp, env_ids)
 
 
 def try_fuse(env, **kw):
-    """(recipe name, hot path, step fn, reset_idx fn) or None; the reasons go to env.fusion_report."""
+    """Installs the first recipe whose proof holds; the reasons go to env.fusion_report."""
     report = []
-    for name, fuse, bind, step, reset_idx in RECIPES:
+    for name, (fuse, _, _) in RECIPES.items():
         try:
             hp = fuse(env, **{k: v for k, v in kw.items() if k in fuse.__code__.co_varnames})
         except (NotFusable, terms.TermMismatch, KeyError, AttributeError) as exc:
             report.append(f"{name}: {exc}")
             continue
-        bind(env, hp)
+        install(env, name, hp)
         env.fusion_report = f"fused: {name}"
-        return name, hp, step, reset_idx
+        return
     env.fusion_report = "user-hook mode — " + "; ".join(report)
-    return None

@@ -13,9 +13,11 @@ Two execution modes, both CUDA-only (no CPU fallback):
 * **user-hook mode** (default): the hooks are arbitrary torch code on CUDA tensors and this class
   runs the reference's orchestration (env.py:85-130) around them, with the rows it owns itself —
   action / obs clip, reset-id compaction, history push — done by the ``libshifu_b200`` kernels;
-* **fused mode**: a task that declares its reward terms to the registry
-  (``shifu_b200.hotpath.compile_reward_terms``) replaces ``post_step`` by one fused kernel
-  (see ``shifu_b200/tasks``).
+* **fused mode**: ``post_step`` becomes one fused kernel.  A subclass whose hooks provably are what
+  the kernel computes is fused on its first ``reset()`` / ``step()`` (``autofuse.py``); the task
+  classes of ``shifu_b200/tasks`` fuse explicitly at construction.  Both ways build the descriptor,
+  bind the env's tensors and dispatch ``step`` / ``reset_idx`` with the same code
+  (``autofuse.install``).
 """
 from __future__ import annotations
 
@@ -54,7 +56,7 @@ class ShifuVecEnv(VecEnv):
         self.stats_allreduce: Optional[Callable] = None    # sums a tensor over ranks (sharded runs)
         self.extras: Dict = {}
         self.fusion_report = "not attempted"
-        self._fusion = None            # (recipe, hot path, step fn, reset_idx fn) once fused
+        self._fusion = None            # (recipe, hot path, step fn) once fused (autofuse.install)
         self._fusion_tried = False
         self._allocate()
         self.reward_functions: List[Callable] = self.build_reward_functions()
@@ -115,22 +117,13 @@ class ShifuVecEnv(VecEnv):
     # ------------------------------------------------------------------ automatic fusion
     def _maybe_fuse(self):
         """First reset()/step(): replace the hooks by a fused kernel when they provably are what the kernel
-        computes (autofuse.py).  Tasks that manage their own fusion (shifu_b200.tasks) set ``hot``."""
-        if self._fusion_tried:
-            return self._fusion
-        self._fusion_tried = True
-        if not self.auto_fuse or getattr(self, "hot", None) is not None or not hasattr(self, "robot"):
-            return None
-        from shifu_b200.gym import autofuse
-        self._fusion = autofuse.try_fuse(self, rng_seed=getattr(self.cfg, "rng_seed", 0x5EED),
-                                         carry_body_frame=getattr(self.cfg, "carry_body_frame", True))
-        if self._fusion is not None:
-            recipe, hp, step_fn, reset_fn = self._fusion
-            self.hot = hp
-            # a subclass reset_idx (curriculum + command sampling in torch) is part of what got fused
-            self.reset_idx = lambda env_ids: reset_fn(self, hp, env_ids)
-            if recipe == "a1":
-                hp.body_frame()
+        computes (autofuse.py).  Tasks that fuse explicitly (shifu_b200.tasks) have installed theirs."""
+        if not self._fusion_tried:
+            self._fusion_tried = True
+            if self.auto_fuse and hasattr(self, "robot"):
+                from shifu_b200.gym import autofuse
+                autofuse.try_fuse(self, rng_seed=getattr(self.cfg, "rng_seed", 0x5EED),
+                                  carry_body_frame=getattr(self.cfg, "carry_body_frame", True))
         return self._fusion
 
     # ------------------------------------------------------------------ orchestration, user-hook mode

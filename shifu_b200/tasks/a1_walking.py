@@ -6,7 +6,10 @@ Counterpart of ``examples/a1_conditional`` of the reference: same classes (``A1R
 * ``fused=True`` (default): the reward list is handed to the reward-term registry and
   ``post_step`` is ONE CUDA kernel (``shifu_a1_post_physics``) — PD torques, body-frame
   velocities, height scan, termination, rewards + episode sums, reset with Philox draws,
-  observation, history push and clips never go through torch;
+  observation, history push and clips never go through torch.  The descriptor builder, the
+  binding of the env's tensors, the fused step and the ``reset_idx`` dispatch are automatic
+  fusion's (``shifu_b200.gym.autofuse``), without its proof: the named terms run the reference
+  constants;
 * ``fused=False``: the hooks below run as ordinary torch code on the same CUDA tensors through
   ``ShifuVecEnv``'s user-hook orchestration (what an unmodified user subclass gets).  Random
   draws come from the same counter-based Philox streams so the two modes can be compared.
@@ -19,7 +22,6 @@ import numpy as np
 import torch
 from isaacgym import gymapi
 
-from shifu_b200 import hotpath
 from shifu_b200.configs import LeggedRobotActorConfig, PPOConfig, TerrainEnvConfig
 from shifu_b200.gym import ShifuVecEnv
 from shifu_b200.units import LeggedRobot
@@ -133,7 +135,7 @@ class A1Conditional(ShifuVecEnv):
                  env_offset: int = 0, num_envs_global: int = None, store_measured_heights: bool = False,
                  use_cuda_graph: bool = True):
         super().__init__(cfg, env_offset=env_offset, num_envs_global=num_envs_global)
-        self.auto_fuse = False          # this class wires its own fusion (explicit fused= switch)
+        self.auto_fuse = False          # this class fuses explicitly (fused= switch)
         self.fused = fused
         self.rng_seed = rng_seed
         self.use_cuda_graph = use_cuda_graph
@@ -160,68 +162,26 @@ class A1Conditional(ShifuVecEnv):
     # fused mode
     # ------------------------------------------------------------------------------------------
     def _fuse(self, carry_body_frame):
-        isg, rb, tc = self.isg_env, self.robot, self.cfg.terrain
-        layout = rb.affine_root_layout()
-        if layout is None:
+        from shifu_b200 import terms
+        from shifu_b200.gym import autofuse
+        if self.robot.affine_root_layout() is None:
             raise NotImplementedError("the fused A1 kernel needs affine root_indices")
         names = [fn.__name__ for fn in self.reward_functions]
         obs = None
         if type(self).compute_observations is not A1Conditional.compute_observations:
             # an edited observation hook: fused only when the kernel's observation layout expresses it,
             # never silently replaced by the reference observation
-            from shifu_b200 import terms
             try:
                 obs = terms.compile_a1_obs(self)
                 terms.verify_a1_obs(self, obs)
             except terms.NotFusable as exc:
                 raise NotImplementedError(f"{exc} (fused=False runs any observation hook)") from exc
-        desc = hotpath.a1_desc(
-            self.num_envs, env_offset=self.env_offset, rng_seed=self.rng_seed, terms=names,
-            q0=tuple(rb.cfg.default_dof_pos), kp=tuple(float(v) for v in rb.cfg.dof_stiffness),
-            kd=tuple(float(v) for v in rb.cfg.dof_damping), torque_limit=tuple(rb.torque_limits.tolist()),
-            points_x=tuple(tc.measured_points_x), points_y=tuple(tc.measured_points_y),
-            border_size=float(tc.border_size), horizontal_scale=tc.horizontal_scale,
-            vertical_scale=tc.vertical_scale, max_episode_length=int(self.max_episode_length),
-            max_episode_length_s=float(self.max_episode_length_s),
-            default_root=tuple(rb.cfg.default_pos) + tuple(rb.cfg.default_quat), curriculum=tc.curriculum,
-            max_terrain_level=isg.max_terrain_level, num_terrain_types=tc.num_cols,
-            env_length=isg.terrain.env_length, base_body=int(self.contact_terminate_indices),
-            leg_bodies=tuple(rb.leg_indices.tolist()), force_body=rb.rigid_body_dict['base'],
-            root_stride=layout[0], root_offset=layout[1], clip_actions=float(self.clip_actions),
-            clip_obs=float(self.clip_obs), obs=obs)
-        hp = hotpath.A1HotPath(desc, root_state=isg.root_state, dof_state=isg.dof_state,
-                               contact_state=isg.contact_state, height_samples=isg.height_samples,
-                               terrain_origins=isg.terrain_origins, terrain_types=isg.terrain_types,
-                               env_origins=isg.env_origins, terms=names, carry_body_frame=carry_body_frame,
-                               want_measured_heights=self._store_heights)
-        self.hot = hp
-        # the env / robot attributes ARE the tensors the kernel reads and writes
-        self.actions, self.obs_buf, self.rew_buf, self.reset_buf = hp.actions, hp.obs_buf, hp.rew_buf, hp.reset_buf
-        self._episode_length_buf = hp.ep_len
-        self.time_out_buf, self.contact_terminate_buf = hp.time_out_buf, hp.contact_terminate_buf
-        self.episode_rewards = hp.ep_sums
-        self.command_buf, self.terrain_levels = hp.command, hp.terrain_levels
-        if hp.swing_time.shape == self.swing_time.shape:
-            self.swing_time, self.last_contacts = hp.swing_time, hp.last_contacts
-        self.actions_recorder.history_buf = hp.history
-        rb.torques, rb.dof_targets, rb.rand_force_buf = hp.torques, hp.dof_targets, hp.rand_force
-        rb.base_lin_vel, rb.base_ang_vel = hp.base_lin_vel, hp.base_ang_vel
-        rb.projected_gravity, rb.gravity_vec = hp.projected_gravity, hp.gravity_vec
-        isg.measured_heights = hp.measured_heights      # None unless store_measured_heights: filled on demand
-        isg.__dict__["_heights_on_demand"] = hp.measured_heights is None
-        self.extras = hp.extras()
-        hp.body_frame()
-
-    def _push_resets_to_sim(self, env_ids=None):
-        """Indexed setters of the simulator for rows the kernel rewrote (isaac_gym.py:70-73,
-        robot.py:78-86).  They need the id count on the host (one sync, like the reference's
-        ``nonzero``); the stand-in simulator has no hidden state and skips this."""
-        if not getattr(self.isg_env.gym, "needs_indexed_resets", True):
-            return
-        ids = self.hot.reset_id_list() if env_ids is None else env_ids
-        if len(ids):
-            self.robot.push_dof_reset(ids)
-            self.isg_env.push_root_reset(ids)
+        # reference constants: the named terms' (hotpath.A1_TERM_PARAMS) and the push force
+        # (a1_conditional.py:82-87); step() hands the kernel raw actions, which a1_desc's default
+        # action_scale scales (a1_conditional.py:122-124)
+        desc = autofuse.a1_env_desc(self, names, rng_seed=self.rng_seed, obs=obs,
+                                    force_body=self.robot.rigid_body_dict['base'], push_force_max=5.0)
+        autofuse.install(self, "a1", autofuse.a1_hot_path(self, desc, names, carry_body_frame, self._store_heights))
 
     def step(self, actions: torch.Tensor):
         if not self.fused:
@@ -229,20 +189,7 @@ class A1Conditional(ShifuVecEnv):
         from shifu_b200.gym import autofuse
         return autofuse.a1_fused_step(self, self.hot, actions)       # kernel launches, or one graph replay
 
-    def reset(self):
-        if not self.fused:
-            return super().reset()
-        self.reset_idx(None)
-        obs, pri, _, _, _ = self.step(torch.zeros(self.num_envs, self.num_actions, device=self.device))
-        return obs, pri
-
-    def reset_idx(self, env_ids):
-        if self.fused:
-            self.hot.step_counter = self.common_step_counter
-            self.hot.reset_idx(env_ids, self.stats_allreduce)
-            self._push_resets_to_sim(torch.arange(self.num_envs, device=self.device) if env_ids is None else env_ids)
-            self.extras.update(self.hot.extras())
-            return
+    def reset_idx(self, env_ids):                   # user-hook mode; fused mode installs the kernel's
         if self.cfg.terrain.curriculum:
             self.update_terrain_curriculum(env_ids)
         super().reset_idx(env_ids)

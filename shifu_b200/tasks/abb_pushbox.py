@@ -153,7 +153,6 @@ class AbbPushBox(ShifuVecEnv):
 
     def __init__(self, cfg, rng_seed: int = 0x5EED, env_offset: int = 0):
         super().__init__(cfg, env_offset=env_offset)
-        self.auto_fuse = False          # this class wires its own fusion
         self.rng_seed = rng_seed
         self.robot = AbbRobot(AbbRobotConfig())
         self.table = Box(TableConfig())
@@ -169,66 +168,15 @@ class AbbPushBox(ShifuVecEnv):
         return []
 
     def _fuse(self):
-        isg = self.isg_env
-        names = [fn.__name__ for fn in self.reward_functions]
-        desc = hotpath.abb_desc(self.num_envs, env_offset=self.env_offset, rng_seed=self.rng_seed, terms=names)
+        """Step and reset_idx (env.py:85-130) of the 4-actor scene run ``shifu_abb_post_physics`` /
+        ``shifu_abb_reset_idx``: default robot / table poses and Philox-drawn cube and goal poses
+        (a_prior_stage.py:39-51) with the reference's reward constants."""
+        from shifu_b200.gym import autofuse
         actors = [self.robot, self.table, self.cube, self.goal]
         layouts = [a.affine_root_layout() for a in actors]
         if any(l is None or l[0] != len(actors) for l in layouts):
             raise NotImplementedError("the fused ABB kernel needs the 4-actor interleaved root layout")
-        desc.num_actors = len(actors)
-        desc.robot_actor, desc.table_actor, desc.cube_actor, desc.goal_actor = (l[1] for l in layouts)
-        desc.num_bodies = sum(a.num_bodies for a in actors)
-        desc.num_dof, desc.ee_body = self.robot.num_dof, int(self.robot.ee_indices[0])
-        for i in range(3):
-            desc.min_ee_pos[i], desc.max_ee_pos[i] = self.robot.cfg.min_ee_pos[i], self.robot.cfg.max_ee_pos[i]
-            desc.box_pos_low[i], desc.box_pos_high[i] = self.cube.pos_range["low"][i], self.cube.pos_range["high"][i]
-        desc.goal_z = self.goal.pos_range["low"][2]
-        desc.max_episode_length, desc.max_episode_length_s = int(self.max_episode_length), float(self.max_episode_length_s)
-        desc.clip_obs = float(self.clip_obs)
-        hp = hotpath.AbbHotPath(desc, root_state=isg.root_state, body_state=isg.body_state,
-                                dof_state=isg.dof_state, terms=names)
-        self.hot = hp
-        self.obs_buf, self.rew_buf, self.reset_buf = hp.obs_buf, hp.rew_buf, hp.reset_buf
-        self._episode_length_buf, self.time_out_buf, self.success_buf = hp.ep_len, hp.time_out_buf, hp.success_buf
-        self.episode_rewards = hp.ep_sums
-        self.robot.dof_targets = hp.dof_targets
-        self.extras = hp.extras()
-
-    def step(self, actions: torch.Tensor):
-        k = self.isg_env.kernels()
-        self.actions = k.clip(actions, self.clip_actions, out=self.actions)      # env.py:87
-        self.isg_env.step(self.actions)                                          # shifu_arm_ik (row N2) + sim
-        self.common_step_counter += 1
-        self.hot.step_counter = self.common_step_counter - 1
-        self.hot.post_physics()
-        self.hot.finalize(self.stats_allreduce)
-        self._push_resets_to_sim()
-        self.extras.update(self.hot.extras())      # this step's own slot of the extras ring (fresh inner dict)
-        return self.obs_buf, self.privileged_obs_buf, self.rew_buf, self.reset_buf, self.extras
-
-    def _push_resets_to_sim(self, env_ids=None):
-        """Indexed setters of the simulator for the rows the kernel rewrote (isaac_gym.py:70-73)."""
-        if not getattr(self.isg_env.gym, "needs_indexed_resets", True):
-            return
-        ids = self.hot.reset_id_list() if env_ids is None else env_ids
-        if len(ids):
-            self.robot.push_dof_reset(ids)
-            self.isg_env.push_root_reset(ids)
-
-    def reset(self):                                                             # env.py:108-112
-        self.reset_idx(None)
-        obs, pri, *_ = self.step(torch.zeros(self.num_envs, self.num_actions, device=self.device))
-        return obs, pri
-
-    def reset_idx(self, env_ids):
-        """env.py:114-130 for the 4-actor scene in one launch (``shifu_abb_reset_idx``): default robot /
-        table poses, Philox-drawn cube and goal poses (a_prior_stage.py:39-51), episode bookkeeping and
-        the logged means — ``extras`` keeps pointing at the hot path's ring, never a detached dict."""
-        self.hot.step_counter = self.common_step_counter
-        self.hot.reset_idx(env_ids, self.stats_allreduce)
-        self._push_resets_to_sim(torch.arange(self.num_envs, device=self.device) if env_ids is None else env_ids)
-        self.extras.update(self.hot.extras())
+        autofuse.install(self, "abb", autofuse.abb_hot_path(self, self.rng_seed, hotpath.ABB_TERM_PARAMS))
 
     # hooks: the names feed the reward-term registry (a_prior_stage.py:112-127)
     def build_reward_functions(self):

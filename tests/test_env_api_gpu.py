@@ -119,6 +119,26 @@ def test_abb_class_api_replays_golden():
         util.compare_a1(got, want, f"abb api/s{t}", skip=("dof_targets",))
 
 
+def test_task_classes_carry_the_reference_descriptor():
+    """The fused task classes on their default configs hand the kernel exactly the reference's constants:
+    the descriptor builders they share with automatic fusion read every value off the env, its robot,
+    its scene and its config, and the default config has the constants ``a1_desc`` / ``abb_desc`` default to."""
+    from shifu_b200 import hotpath
+    n, offset, seed = 64, 4096, 99
+    _install()
+    from shifu_b200.tasks.a1_walking import A1Conditional, A1EnvConfig
+    cfg = A1EnvConfig()
+    cfg.num_envs, cfg.device = n, "cuda:0"
+    env = A1Conditional(cfg, rng_seed=seed, env_offset=offset, num_envs_global=offset + n)
+    assert bytes(env.hot.desc) == bytes(hotpath.a1_desc(n, env_offset=offset, rng_seed=seed))
+    _install()
+    from shifu_b200.tasks.abb_pushbox import AbbPushBox, PriorStageEnvConfig
+    cfg = PriorStageEnvConfig()
+    cfg.num_envs, cfg.device = n, "cuda:0"
+    env = AbbPushBox(cfg, rng_seed=seed, env_offset=offset)
+    assert bytes(env.hot.desc) == bytes(hotpath.abb_desc(n, env_offset=offset, rng_seed=seed))
+
+
 def test_abb_robot_step_uses_arm_ik_kernel():
     """AbbRobot.step (a_prior_stage.py:67-73) through the class API == oracle restatement."""
     import json, os
