@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SHIFU_ABI_VERSION 4
+#define SHIFU_ABI_VERSION 5
 
 #define SHIFU_MAX_DOF 12
 #define SHIFU_MAX_LEG_BODIES 8
@@ -38,6 +38,22 @@ extern "C" {
 #define SHIFU_MAX_REWARD_TERMS 8
 #define SHIFU_NUM_STATS 16
 #define SHIFU_OBS_HEAD 72       /* observation columns before the 187 heights */
+
+/* Philox stream of the observation noise (ShifuA1Desc.obs_noise / obs_height_noise).  Counter
+ * (global env id, step, SHIFU_STREAM_OBS_NOISE, word), key rng_seed, u = (x >> 8) * 2^-24 like every other
+ * draw; step is the one the step's reset draws use.  65 words (0-64) cover the 259 columns:
+ *   head, words 0-17: column d + 12m (d < 12, m < 6) is lane (d & 1) + 2 (m & 1) of word 3 (d >> 1) + (m >> 1),
+ *     i.e. word 3i + r holds columns 2i + 24r, 2i + 1 + 24r, 2i + 24r + 12, 2i + 1 + 24r + 12 in x, y, z, w;
+ *   heights, words 18-64: point pair k = (point k, point 186 - k), k = 0..93, is word 18 + (k >> 1): for even
+ *     k, x = point k and y = point 186 - k; for odd k, z = point k and w = point 186 - k; the centre point 93
+ *     uses z only.
+ * The map follows the pipelined kernel's work split.  The two scan lanes of head columns d = 2i, 2i+1 each
+ * evaluate one of words 3i, 3i+1 and swap halves; both evaluate word 3i+2 and each uses its half (a warp
+ * issues that evaluation in the same slots whether one lane or two run it): 24 evaluations for the 18 head
+ * words.  The two lanes of height point pairs k, k^1 each evaluate word 18 + (k >> 1) for one env of an env
+ * pair and swap halves, so every lane of those evaluations is used; the two idle scan lanes evaluate word 64
+ * for nothing. */
+#define SHIFU_STREAM_OBS_NOISE 8
 
 enum {
   SHIFU_OK = 0,
@@ -169,6 +185,11 @@ typedef struct ShifuA1Desc {
                                                        x_j of the dof-position columns is dof_pos - q0 */
   float obs_height_scale;                           /* heights = clip(clip(z - height_offset - h, +-height_clip) * this,
                                                        +-clip_obs) */
+  /* uniform observation noise (legged_gym's noise_scale_vec), added before the clip to +-clip_obs:
+   * obs[j] = clip(x_j * obs_scale[j] + (2u_j - 1) * obs_noise[j], +-clip_obs), heights likewise with
+   * obs_height_noise, u_j drawn on SHIFU_STREAM_OBS_NOISE.  All zero: no noise.  Needs obs_layout = 1. */
+  float obs_noise[SHIFU_OBS_HEAD];
+  float obs_height_noise;
 } ShifuA1Desc;
 
 /* Tensors of one A1 step.  "rw" = read and written in place. */

@@ -12,7 +12,7 @@ import os
 from typing import Optional
 
 MAX_DOF, MAX_LEG, MAX_PX, MAX_PY, MAX_TERMS, NUM_STATS = 12, 8, 17, 11, 8, 16
-ABI_VERSION = 4
+ABI_VERSION = 5
 OBS_HEAD = 72
 
 # enum ShifuRewardTerm
@@ -59,7 +59,7 @@ class A1Desc(C.Structure):
         ("num_feet", C.c_int32), ("feet_bodies", C.c_int32 * 4), ("feet_contact_force", C.c_float),
         ("air_time_cmd_min", C.c_float), ("air_time_dt", C.c_float), ("air_time_reset", C.c_int32),
         ("obs_layout", C.c_int32), ("obs_vec_src", C.c_int32 * 4), ("obs_scale", C.c_float * OBS_HEAD),
-        ("obs_height_scale", C.c_float),
+        ("obs_height_scale", C.c_float), ("obs_noise", C.c_float * OBS_HEAD), ("obs_height_noise", C.c_float),
     ]
 
 

@@ -221,8 +221,10 @@ __device__ __noinline__ float a1_eval_term(int q, const A1K& k, const A1Smem& s,
 
 // The observation layout `o` is applied at run time for every layout (this kernel takes the ragged tail
 // and the fallback layouts); for the reference layout it is the identity, and x * 1.0f plus the
-// composed clips are exact, so the reference observation comes out unchanged.
-template <bool TILED, bool EXACT_DIV>
+// composed clips are exact, so the reference observation comes out unchanged.  NOISE (the host sets it
+// when o.noisy): observation noise from the same words as the pipelined kernel, one evaluation per
+// column; a compile-time flag, so that the noiseless instantiations keep their registers and code.
+template <bool TILED, bool EXACT_DIV, bool NOISE>
 __global__ void __launch_bounds__(A1_THREADS, 5)
 a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io,
                        const __grid_constant__ A1Obs o) {
@@ -327,17 +329,21 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
     // ---- phase B3: obs head (a1_conditional.py:131-144), history push (train.py:12-14) --------
     {
       const float c = k.clip_obs;
+      // + the column's noise before the clip to +-clip_obs
+      auto nz = [&](float x, int e, int j) {
+        return NOISE ? add_rn(x, obs_noise_at(o, k.seed, k.env_offset + e0 + e, step, j)) : x;
+      };
       // (env, dof) items: dof columns and history columns (+ in-place push)
       for (int i = t; i < ne * A1_DOF; i += A1_THREADS) {
         const int e = i / A1_DOF, d = i - e * A1_DOF;
         float* h = s.head[e];
-        h[12 + d] = clampf(mul_rn(sub_rn(s.dof[e][2 * d], k.q0[d]), o.scale[12 + d]), -c, c);
-        h[24 + d] = clampf(mul_rn(s.dof[e][2 * d + 1], o.scale[24 + d]), -c, c);
+        h[12 + d] = clampf(nz(mul_rn(sub_rn(s.dof[e][2 * d], k.q0[d]), o.scale[12 + d]), e, 12 + d), -c, c);
+        h[24 + d] = clampf(nz(mul_rn(s.dof[e][2 * d + 1], o.scale[24 + d]), e, 24 + d), -c, c);
         const float a0 = s.hist[e][d * A1_HIST + 0], a1 = s.hist[e][d * A1_HIST + 1],
                     a2 = s.hist[e][d * A1_HIST + 2];
-        h[36 + d] = clampf(mul_rn(a0, o.scale[36 + d]), -c, c);    // HistoryRecorder.flatten: slot-major
-        h[48 + d] = clampf(mul_rn(a1, o.scale[48 + d]), -c, c);
-        h[60 + d] = clampf(mul_rn(a2, o.scale[60 + d]), -c, c);
+        h[36 + d] = clampf(nz(mul_rn(a0, o.scale[36 + d]), e, 36 + d), -c, c);    // HistoryRecorder.flatten: slot-major
+        h[48 + d] = clampf(nz(mul_rn(a1, o.scale[48 + d]), e, 48 + d), -c, c);
+        h[60 + d] = clampf(nz(mul_rn(a2, o.scale[60 + d]), e, 60 + d), -c, c);
         s.hist[e][d * A1_HIST + 2] = a1;               // HistoryRecorder.add
         s.hist[e][d * A1_HIST + 1] = a0;
         s.hist[e][d * A1_HIST + 0] = s.act[e][d];
@@ -345,7 +351,7 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
       // (env, j < 12): the four vector slots (reference: command, body-frame velocities, gravity_vec)
       for (int i = t; i < ne * 12; i += A1_THREADS) {
         const int e = i / 12, j = i - e * 12;
-        s.head[e][j] = clampf(mul_rn(a1_obs_vec(o, j, s.cla, e, pg0[e][j % 3]), o.scale[j]), -c, c);
+        s.head[e][j] = clampf(nz(mul_rn(a1_obs_vec(o, j, s.cla, e, pg0[e][j % 3]), o.scale[j]), e, j), -c, c);
       }
       // carried body-frame velocities for the next control step (robot.py:222-229, D7)
       if (io.carry_body_frame && warp == 5 && lane_env) {
@@ -376,13 +382,13 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
                  A1_THREADS);
     }
 
-    // ---- phase C: 187-point scan; obs[., 72 + t] = clip(clip((z - 0.5) - h, +-1) * h_scale, +-clip_obs)
+    // ---- phase C: 187-point scan; obs[., 72 + t] = clip(clip((z - 0.5) - h, +-1) * h_scale [+ noise], +-clip_obs)
     if (t < A1_POINTS) {
       float* orow = io.obs_buf + (long long)e0 * A1_OBS + A1_HEAD + t;
       float* mrow = (io.measured_heights != nullptr) ? io.measured_heights + (long long)e0 * A1_POINTS + t
                                                      : nullptr;
       const short* __restrict__ table = k.table;
-#pragma unroll 4
+#pragma unroll (NOISE ? 1 : 4)            // with NOISE: a Philox evaluation per env, unrolled it spills
       for (int e = 0; e < ne; ++e) {
         const float4 ev = s.ev[e];          // (2z, z, w, -)
         const float4 ps = s.pos[e];         // (x, y, zb, -)
@@ -405,7 +411,9 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
           idx = (int)(px * (unsigned)k.tcols + py);
         }
         const float hgt = mul_rn((float)__ldg(table + idx), k.vscale);      // isaac_gym.py:427-433
-        const float v = clampf(mul_rn(clampf(sub_rn(ps.z, hgt), -k.h_clip, k.h_clip), o.h_scale), -k.clip_obs, k.clip_obs);
+        float v = mul_rn(clampf(sub_rn(ps.z, hgt), -k.h_clip, k.h_clip), o.h_scale);
+        if (NOISE) v = add_rn(v, obs_noise_at(o, k.seed, k.env_offset + e0 + e, step, A1_HEAD + t));
+        v = clampf(v, -k.clip_obs, k.clip_obs);
         __stcs(orow + (long long)e * A1_OBS, v);
         if (mrow != nullptr) __stcs(mrow + (long long)e * A1_POINTS, hgt);
       }

@@ -114,7 +114,9 @@ __device__ __forceinline__ void v3_issue_loads(V3In& in, const A1K& k, const Shi
 // instantiation without that code (its presence alone cost the B group 5-10 % of the kernel).
 // OBS: the observation follows the layout `o` (slot sources, column scales, height scale); without it
 // `o` is not read and the reference observation is built.
-template <bool EXACT_DIV, bool HAS_MROW, bool HAS_EXTRA, bool OBS>
+// NOISE (only with OBS): uniform noise o.noise / o.h_noise is added before the clip to +-clip_obs, drawn
+// on STREAM_OBS_NOISE with the word map of include/shifu_b200.h.
+template <bool EXACT_DIV, bool HAS_MROW, bool HAS_EXTRA, bool OBS, bool NOISE>
 __global__ void __launch_bounds__(V3_THREADS, V3_CTAS_PER_SM)
 a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io, int num_tiles,
                            const __grid_constant__ A1Obs o) {
@@ -270,7 +272,9 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
     const int p = t - V3_SCAN_BASE;                          // index in the scan group
     const int sw = p >> 5, lane = p & 31;
     // clip(clip(v,+-a),+-b) == clip(v,+-min(a,b)); with OBS, clip(clip(v,+-a)*s,+-b) == clip(v*s,+-h_bound)
-    const float hclip = OBS ? o.h_bound : fminf(k.h_clip, k.clip_obs);
+    // (with NOISE the noise sits between the two clips: heights are clipped to +-h_clip, scaled, noised
+    // and clipped to +-clip_obs)
+    const float hclip = NOISE ? k.clip_obs : OBS ? o.h_bound : fminf(k.h_clip, k.clip_obs);
     const short* __restrict__ table = k.table;
     const PairScanK sk = pair_scan_k(k);
     const f2_t VS = pk(k.vscale, k.vscale);
@@ -280,6 +284,14 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
     // point-symmetric to the phased kernel.)
     static_assert(V3_SCAN_WARPS % 3 == 0 && 8 % (V3_SCAN_WARPS / 3) == 0, "scan warps: 3 pair groups x rows");
     constexpr int V3_ITEMS = 8 / (V3_SCAN_WARPS / 3);
+    // with NOISE: the noise scales of this thread's six head columns d + 12m, loaded once (a lane-dependent
+    // index into the parameter space would serialise the loads in the tile loop)
+    float hns[6];
+    if (NOISE) {
+      const int pd = p % A1_DOF;
+#pragma unroll
+      for (int m = 0; m < 6; ++m) hns[m] = o.noise[pd + 12 * m];
+    }
     for (int j = 0; j < my_tiles; ++j) {
       const int b = j % V3_STAGES;
       const uint32_t par = (j / V3_STAGES) & 1;
@@ -315,11 +327,19 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           float* orow = io.obs_buf + (e0 + 2 * w.q0) * A1_OBS + A1_HEAD + w.pt;
           float* mb = HAS_MROW ? io.measured_heights + (e0 + 2 * w.q0) * A1_POINTS + w.pt : nullptr;
           // one packed pair of cells -> (z - 0.5) - h*vertical_scale, clipped, to rows r and r+1
-          auto emit = [&](float2 zb, int h0, int h1, float* ob, float* m) {
+          auto emit = [&](float2 zb, int h0, int h1, float* ob, float* m, f2_t noise) {
             const f2_t hg2 = fma2(pk((float)h0, (float)h1), VS, sk.nz);         // * vertical_scale, :433
             float v0, v1;
             f2_t d2 = sub2(pk(zb.x, zb.y), hg2);                                  // a1_conditional.py:132
-            if (OBS) d2 = mul2(d2, pk(o.h_scale, o.h_scale));
+            if (NOISE) {
+              // fma(a, b, -0) is the product rounded once; a mul2 followed by the add2 would be contracted
+              // into one FFMA2 (DESIGN.md section 2)
+              upk(d2, v0, v1);
+              d2 = pk(clampf(v0, -k.h_clip, k.h_clip), clampf(v1, -k.h_clip, k.h_clip));
+              d2 = add2(fma2(d2, pk(o.h_scale, o.h_scale), sk.nz), noise);
+            } else if (OBS) {
+              d2 = mul2(d2, pk(o.h_scale, o.h_scale));
+            }
             upk(d2, v0, v1);
             __stcs(ob, clampf(v0, -hclip, hclip));
             __stcs(ob + A1_OBS, clampf(v1, -hclip, hclip));
@@ -330,13 +350,29 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
               __stcs(m + A1_POINTS, g1);
             }
           };
-          if (w.live) {
-            const int mir = (A1_POINTS - 1) - 2 * w.pt;                         // column of the mirror point
+          if (NOISE || w.live) {                                                // NOISE: every lane shuffles
+            const int mir = (A1_POINTS - 1) - 2 * w.pt;                           // column of the mirror point
 #pragma unroll
             for (int u = 0; u < 2; ++u) {
-              const float2 zb = *reinterpret_cast<const float2*>(&s.sC[rb][w.q0 + u].z);
-              emit(zb, h[4 * u], h[4 * u + 1], orow + (2 * u) * A1_OBS, mb + (2 * u) * A1_POINTS);
-              emit(zb, h[4 * u + 2], h[4 * u + 3], orow + (2 * u) * A1_OBS + mir, mb + (2 * u) * A1_POINTS + mir);
+              // with NOISE: the envs 2(q0+u), +1 and the point pairs k, k^1 of this lane and its neighbour share
+              // word 18 + (k >> 1); lane k&1 evaluates it for env 2(q0+u) + (k&1) and swaps the neighbour's half
+              f2_t npt = 0, nmir = 0;
+              if (NOISE) {
+                const int c = lane & 1;                                             // = k & 1
+                const U4 q = obs_noise_word(k.seed, k.env_offset + e0 + 2 * (w.q0 + u) + c, step, 18 + (w.pt >> 1));
+                const uint32_t r0 = __shfl_xor_sync(~0u, c ? q.x : q.z, 1), r1 = __shfl_xor_sync(~0u, c ? q.y : q.w, 1);
+                const uint32_t o0 = c ? q.z : q.x, o1 = c ? q.w : q.y;            // (point, mirror) of own env
+                const float sh = o.h_noise;
+                const float p0 = mul_rn(u_pm1(c ? r0 : o0), sh), p1 = mul_rn(u_pm1(c ? o0 : r0), sh);
+                npt = pk(p0, p1);
+                nmir = (w.pt == A1_POINTS / 2) ? npt                              // the centre is its own mirror
+                                                : pk(mul_rn(u_pm1(c ? r1 : o1), sh), mul_rn(u_pm1(c ? o1 : r1), sh));
+              }
+              if (!NOISE || w.live) {
+                const float2 zb = *reinterpret_cast<const float2*>(&s.sC[rb][w.q0 + u].z);
+                emit(zb, h[4 * u], h[4 * u + 1], orow + (2 * u) * A1_OBS, mb + (2 * u) * A1_POINTS, npt);
+                emit(zb, h[4 * u + 2], h[4 * u + 3], orow + (2 * u) * A1_OBS + mir, mb + (2 * u) * A1_POINTS + mir, nmir);
+              }
             }
           }
         };
@@ -356,6 +392,20 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
         if (OBS) {
           const int pe = p / A1_DOF, pd = p - pe * A1_DOF;
           if (o.src[pd / 3] == SHIFU_OBS_PROJECTED_GRAVITY) pgv = io.projected_gravity[(e0 + pe) * 3 + pd % 3];
+        }
+        // with NOISE, this thread's six head noise values: words 3(d>>1) .. +2 of its env, shared with the
+        // lane of column d^1 (the first word is split between the two lanes, the third read by both)
+        float hn[6];
+        if (NOISE) {
+          const int pe = p / A1_DOF, pd = p - pe * A1_DOF, c = pd & 1;
+          const long long gid = k.env_offset + e0 + pe;
+          const U4 wa = obs_noise_word(k.seed, gid, step, 3 * (pd >> 1) + c);
+          const U4 wc = obs_noise_word(k.seed, gid, step, 3 * (pd >> 1) + 2);
+          const uint32_t r0 = __shfl_xor_sync(~0u, c ? wa.x : wa.y, 1), r1 = __shfl_xor_sync(~0u, c ? wa.z : wa.w, 1);
+          const uint32_t o0 = c ? wa.y : wa.x, o1 = c ? wa.w : wa.z;
+          const uint32_t x[6] = {c ? r0 : o0, c ? r1 : o1, c ? o0 : r0, c ? o1 : r1, c ? wc.y : wc.x, c ? wc.w : wc.z};
+#pragma unroll
+          for (int m = 0; m < 6; ++m) hn[m] = mul_rn(u_pm1(x[m]), hns[m]);
         }
         // ---- obs head (a1_conditional.py:131-144) + history push (train.py:12-14): post-reset rows
         pipe::mbar_wait<32>(&s.b_done[b], par);
@@ -382,13 +432,17 @@ a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant_
           pipe::fence_proxy_async();                            // pushed history -> visible to the TMA store
           pipe::mbar_arrive(&s.h_done[b]);
           // with OBS: x_j * scale[j] before the clip
-          auto sc = [&](float x, int j) { return OBS ? mul_rn(x, o.scale[j]) : x; };
-          __stcs(hrow + d, clampf(sc(v, d), -c, c));
-          __stcs(hrow + 12 + d, clampf(sc(sub_rn(qd.x, k.q0[d]), 12 + d), -c, c));
-          __stcs(hrow + 24 + d, clampf(sc(qd.y, 24 + d), -c, c));
-          __stcs(hrow + 36 + d, clampf(sc(a0, 36 + d), -c, c));   // HistoryRecorder.flatten: slot-major
-          __stcs(hrow + 48 + d, clampf(sc(a1, 48 + d), -c, c));
-          __stcs(hrow + 60 + d, clampf(sc(a2, 60 + d), -c, c));
+          // with NOISE: + noise of column d + 12m before the clip
+          auto sc = [&](float x, int m) {
+            const float y = OBS ? mul_rn(x, o.scale[d + 12 * m]) : x;
+            return NOISE ? add_rn(y, hn[m]) : y;
+          };
+          __stcs(hrow + d, clampf(sc(v, 0), -c, c));
+          __stcs(hrow + 12 + d, clampf(sc(sub_rn(qd.x, k.q0[d]), 1), -c, c));
+          __stcs(hrow + 24 + d, clampf(sc(qd.y, 2), -c, c));
+          __stcs(hrow + 36 + d, clampf(sc(a0, 3), -c, c));   // HistoryRecorder.flatten: slot-major
+          __stcs(hrow + 48 + d, clampf(sc(a1, 4), -c, c));
+          __stcs(hrow + 60 + d, clampf(sc(a2, 5), -c, c));
         }
 #pragma unroll 1
         for (int it = 1; it < V3_ITEMS; ++it) {

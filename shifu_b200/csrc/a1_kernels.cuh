@@ -76,7 +76,23 @@ struct A1Obs {
   float h_bound;          // min(h_clip * |h_scale|, clip_obs): the same heights as clip((z - h_off - h) * h_scale,
                           // +-h_bound), because rounding the product is monotonic and sign-symmetric
   int uses_pg;            // some slot reads projected_gravity
+  // uniform noise, added before the clip to +-clip_obs (0 everywhere: none).  With noise the heights are
+  // clip(clip(clip(z - h_off - h, +-h_clip) * h_scale + n, +-clip_obs)): h_bound does not apply.
+  float noise[A1_HEAD];   // head column j: n = (2u - 1) * noise[j]
+  float h_noise;          // every height column
+  int noisy;              // some noise scale is non-zero
 };
+static_assert(STREAM_OBS_NOISE == SHIFU_STREAM_OBS_NOISE, "observation-noise stream");
+
+// Noise n = (2u - 1) * s of head column j < 72 or height column j >= 72 of env gid (the phased kernel's
+// form: one Philox evaluation per column; the pipelined kernel shares the words between lanes).
+__device__ __forceinline__ float obs_noise_at(const A1Obs& o, unsigned long long seed, long long gid, long long step,
+                                              int j) {
+  uint32_t word;
+  int lane;
+  obs_noise_slot(j, word, lane);
+  return mul_rn(u_pm1(u4_lane(obs_noise_word(seed, gid, step, word), lane)), j < A1_HEAD ? o.noise[j] : o.h_noise);
+}
 
 // Value of head column j < 12 of env e: slot j / 3, component j % 3.  cla = command, base lin vel,
 // base ang vel of the env; pg = component j % 3 of its projected gravity when the step started.

@@ -73,22 +73,24 @@ struct ShifuCtx {
 
 static inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
-// the pipelined kernel's instantiations, index = 8*OBS + 4*EXACT_DIV + 2*HAS_MROW + HAS_EXTRA
-constexpr int A1_TMA_VARIANTS = 16;
-template <bool OBS>
+// the pipelined kernel's instantiations, index = 8*(OBS + NOISE) + 4*EXACT_DIV + 2*HAS_MROW + HAS_EXTRA
+// (NOISE only with OBS)
+constexpr int A1_TMA_VARIANTS = 24;
+template <bool OBS, bool NOISE>
 static void a1_tma_fill(const void** t) {
-  t[0] = (const void*)a1_post_physics_tma_kernel<false, false, false, OBS>;
-  t[1] = (const void*)a1_post_physics_tma_kernel<false, false, true, OBS>;
-  t[2] = (const void*)a1_post_physics_tma_kernel<false, true, false, OBS>;
-  t[3] = (const void*)a1_post_physics_tma_kernel<false, true, true, OBS>;
-  t[4] = (const void*)a1_post_physics_tma_kernel<true, false, false, OBS>;
-  t[5] = (const void*)a1_post_physics_tma_kernel<true, false, true, OBS>;
-  t[6] = (const void*)a1_post_physics_tma_kernel<true, true, false, OBS>;
-  t[7] = (const void*)a1_post_physics_tma_kernel<true, true, true, OBS>;
+  t[0] = (const void*)a1_post_physics_tma_kernel<false, false, false, OBS, NOISE>;
+  t[1] = (const void*)a1_post_physics_tma_kernel<false, false, true, OBS, NOISE>;
+  t[2] = (const void*)a1_post_physics_tma_kernel<false, true, false, OBS, NOISE>;
+  t[3] = (const void*)a1_post_physics_tma_kernel<false, true, true, OBS, NOISE>;
+  t[4] = (const void*)a1_post_physics_tma_kernel<true, false, false, OBS, NOISE>;
+  t[5] = (const void*)a1_post_physics_tma_kernel<true, false, true, OBS, NOISE>;
+  t[6] = (const void*)a1_post_physics_tma_kernel<true, true, false, OBS, NOISE>;
+  t[7] = (const void*)a1_post_physics_tma_kernel<true, true, true, OBS, NOISE>;
 }
 static const void* const* a1_tma_variants() {
   static const void* table[A1_TMA_VARIANTS];
-  static const bool filled = (a1_tma_fill<false>(table), a1_tma_fill<true>(table + 8), true);
+  static const bool filled = (a1_tma_fill<false, false>(table), a1_tma_fill<true, false>(table + 8),
+                              a1_tma_fill<true, true>(table + 16), true);
   (void)filled;
   return table;
 }
@@ -115,6 +117,14 @@ static int fill_a1obs(const ShifuA1Desc& d, A1Obs& o, bool& custom) {
   o.h_scale = 1.0f;
   o.h_bound = std::fmin(d.height_clip, d.clip_obs);
   custom = false;
+  for (int j = 0; j <= A1_HEAD; ++j) {
+    const float v = j < A1_HEAD ? d.obs_noise[j] : d.obs_height_noise;
+    if (!std::isfinite(v))
+      return j < A1_HEAD ? fail(SHIFU_E_RANGE, "obs_noise[%d]=%g is not finite", j, (double)v)
+                         : fail(SHIFU_E_RANGE, "obs_height_noise=%g is not finite", (double)v);
+    if (v != 0.0f && d.obs_layout == 0)
+      return fail(SHIFU_E_RANGE, "observation noise needs obs_layout = 1 (obs_layout = 0 ignores the layout fields)");
+  }
   if (d.obs_layout == 0) return SHIFU_OK;
   for (int i = 0; i < 4; ++i) {
     if (d.obs_vec_src[i] < 0 || d.obs_vec_src[i] >= SHIFU_OBS_VEC_COUNT)
@@ -133,6 +143,10 @@ static int fill_a1obs(const ShifuA1Desc& d, A1Obs& o, bool& custom) {
   custom |= d.obs_height_scale != 1.0f;
   o.h_scale = d.obs_height_scale;
   o.h_bound = std::fmin(d.height_clip * std::fabs(o.h_scale), d.clip_obs);
+  for (int j = 0; j < A1_HEAD; ++j) { o.noise[j] = d.obs_noise[j]; o.noisy |= d.obs_noise[j] != 0.0f; }
+  o.h_noise = d.obs_height_noise;
+  o.noisy |= d.obs_height_noise != 0.0f;
+  custom |= o.noisy != 0;
   return SHIFU_OK;
 }
 
@@ -314,14 +328,16 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
   if (e == cudaSuccess && c->is_a1) {
     // all four instantiations share resources; ask for the full shared-memory carve-out so the
     // resident-CTA count is bounded by registers/threads, not by the default L1/smem split
-    const void* variants[4] = {
-        (const void*)a1_post_physics_kernel<true, false>, (const void*)a1_post_physics_kernel<true, true>,
-        (const void*)a1_post_physics_kernel<false, false>, (const void*)a1_post_physics_kernel<false, true>};
-    for (int v = 0; v < 4 && e == cudaSuccess; ++v)
+    const void* variants[8] = {
+        (const void*)a1_post_physics_kernel<true, false, false>, (const void*)a1_post_physics_kernel<true, true, false>,
+        (const void*)a1_post_physics_kernel<false, false, false>, (const void*)a1_post_physics_kernel<false, true, false>,
+        (const void*)a1_post_physics_kernel<true, false, true>, (const void*)a1_post_physics_kernel<true, true, true>,
+        (const void*)a1_post_physics_kernel<false, false, true>, (const void*)a1_post_physics_kernel<false, true, true>};
+    for (int v = 0; v < 8 && e == cudaSuccess; ++v)
       e = cudaFuncSetAttribute(variants[v], cudaFuncAttributePreferredSharedMemoryCarveout, 75);
     int occ = 0;
     if (e == cudaSuccess)
-      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, a1_post_physics_kernel<true, false>, A1_THREADS, 0);
+      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, a1_post_physics_kernel<true, false, false>, A1_THREADS, 0);
     const int tiles = (n + A1_TILE - 1) / A1_TILE;
     const int cap = c->sm_count * (occ > 0 ? occ : 1);
     c->a1_grid = tiles < cap ? tiles : cap;
@@ -346,7 +362,7 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
     }
     int tocc = 0;
     if (e == cudaSuccess)
-      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tocc, a1_post_physics_tma_kernel<false, false, false, false>, V3_THREADS,
+      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tocc, a1_post_physics_tma_kernel<false, false, false, false, false>, V3_THREADS,
                                                         sizeof(V3Smem));
     c->tma_occ = tocc;
     const char* kern = getenv("SHIFU_A1_KERNEL");
@@ -515,7 +531,7 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     for (int q = 0; q < c->a1k.n_terms; ++q) extra |= c->a1k.terms[q] >= SHIFU_REW_LIN_VEL_Z;
     int tiles_arg = full_tiles;
     void* args[4] = {(void*)&c->a1k, const_cast<ShifuA1StepIO*>(io), (void*)&tiles_arg, (void*)&c->a1o};
-    const int variant = (c->obs_custom ? 8 : 0) + (exact ? 4 : 0) + (mrow ? 2 : 0) + (extra ? 1 : 0);
+    const int variant = (c->obs_custom ? 8 : 0) + (c->a1o.noisy ? 8 : 0) + (exact ? 4 : 0) + (mrow ? 2 : 0) + (extra ? 1 : 0);
     CUDA_TRY(cudaLaunchKernel(a1_tma_variants()[variant], grid, block, args, smem, S(stream)));
   }
   const int done = full_tiles * A1_TILE;
@@ -542,10 +558,17 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     const int cap = c->sm_count * (c->a1_occ > 0 ? c->a1_occ : 1);
     const dim3 grid(tiles < cap ? tiles : cap), block(A1_THREADS);
     const A1Obs& o = c->a1o;
-    if (tiled && !exact) a1_post_physics_kernel<true, false><<<grid, block, 0, S(stream)>>>(k, t, o);
-    else if (tiled && exact) a1_post_physics_kernel<true, true><<<grid, block, 0, S(stream)>>>(k, t, o);
-    else if (!tiled && !exact) a1_post_physics_kernel<false, false><<<grid, block, 0, S(stream)>>>(k, t, o);
-    else a1_post_physics_kernel<false, true><<<grid, block, 0, S(stream)>>>(k, t, o);
+    if (o.noisy) {
+      if (tiled && !exact) a1_post_physics_kernel<true, false, true><<<grid, block, 0, S(stream)>>>(k, t, o);
+      else if (tiled && exact) a1_post_physics_kernel<true, true, true><<<grid, block, 0, S(stream)>>>(k, t, o);
+      else if (!tiled && !exact) a1_post_physics_kernel<false, false, true><<<grid, block, 0, S(stream)>>>(k, t, o);
+      else a1_post_physics_kernel<false, true, true><<<grid, block, 0, S(stream)>>>(k, t, o);
+    } else {
+      if (tiled && !exact) a1_post_physics_kernel<true, false, false><<<grid, block, 0, S(stream)>>>(k, t, o);
+      else if (tiled && exact) a1_post_physics_kernel<true, true, false><<<grid, block, 0, S(stream)>>>(k, t, o);
+      else if (!tiled && !exact) a1_post_physics_kernel<false, false, false><<<grid, block, 0, S(stream)>>>(k, t, o);
+      else a1_post_physics_kernel<false, true, false><<<grid, block, 0, S(stream)>>>(k, t, o);
+    }
     CUDA_TRY(cudaGetLastError());
   }
   return SHIFU_OK;

@@ -159,7 +159,9 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
     # ---- reward terms: match + fit ------------------------------------------------------------
     compiled = terms.compile_a1_terms(env, env.reward_functions)
     names = [t.name for t in compiled]
-    # ---- observation: slot sources and scales -------------------------------------------------
+    # ---- observation: slot sources, scales and noise scales ------------------------------------
+    # (read once, here, like every fitted constant: a noise curriculum that changes noise_scale_vec
+    # later does not reach the kernel)
     obs = terms.compile_a1_obs(env)
     # ---- the hot path over the env's own tensors -----------------------------------------------
     desc = a1_env_desc(env, [(t.name, t.code, t.p0, t.p1) for t in compiled], rng_seed=rng_seed, obs=obs,

@@ -57,10 +57,17 @@ class ObsLayout:
     columns' x_j is ``dof_pos - default_dof_pos``); the 187 heights are
     ``clip(clip(z - 0.5 - h, +-1) * height_scale, +-clip_obs)``, legged_gym's clip-then-scale order.
     PROJECTED_GRAVITY is the value the tensor holds when the step starts (``LeggedRobot.post_step`` on
-    the previous state, like the body-frame velocities).  Scales are kept as fp32 values."""
+    the previous state, like the body-frame velocities).  Scales are kept as fp32 values.
+
+    ``noise`` / ``height_noise``: legged_gym's uniform observation noise (``noise_scale_vec``), one scale per
+    head column and one for all 187 heights.  Column j gets ``+ (2u - 1) * noise[j]`` before the clip to
+    +-clip_obs, u drawn per env, step and column from the kernels' Philox stream
+    (``shifu_b200.utils.philox.obs_noise_u01``).  All zero: no noise."""
     slots: Tuple[str, str, str, str] = A1_OBS_SLOTS
     scales: Tuple[float, ...] = (1.0,) * nv.OBS_HEAD
     height_scale: float = 1.0
+    noise: Tuple[float, ...] = (0.0,) * nv.OBS_HEAD
+    height_noise: float = 0.0
 
     def __post_init__(self):
         slots = tuple(self.slots)
@@ -72,13 +79,25 @@ class ObsLayout:
         hs = float(np.float32(self.height_scale))
         if not all(math.isfinite(v) for v in (*scales, hs)):
             raise ValueError("observation scales must be finite")
+        noise = tuple(float(np.float32(v)) for v in self.noise)
+        if len(noise) != nv.OBS_HEAD:
+            raise ValueError(f"{len(noise)} column noise scales: the observation head has {nv.OBS_HEAD} columns")
+        hn = float(np.float32(self.height_noise))
+        if not all(math.isfinite(v) for v in (*noise, hn)):
+            raise ValueError("observation noise scales must be finite")
         object.__setattr__(self, "slots", slots)
         object.__setattr__(self, "scales", scales)
         object.__setattr__(self, "height_scale", hs)
+        object.__setattr__(self, "noise", noise)
+        object.__setattr__(self, "height_noise", hn)
+
+    def has_noise(self) -> bool:
+        return any(v != 0.0 for v in self.noise) or self.height_noise != 0.0
 
     def is_reference(self) -> bool:
-        """The reference observation (a1_conditional.py:131-144): identity scales, reference slots."""
-        return self.slots == A1_OBS_SLOTS and all(v == 1.0 for v in self.scales) and self.height_scale == 1.0
+        """The reference observation (a1_conditional.py:131-144): identity scales, reference slots, no noise."""
+        return (self.slots == A1_OBS_SLOTS and all(v == 1.0 for v in self.scales) and self.height_scale == 1.0
+                and not self.has_noise())
 
 
 def compile_reward_terms(names: Sequence[str], codes: Dict[str, int], params: Dict[str, tuple]):
@@ -171,6 +190,9 @@ def a1_desc(num_envs: int, *, env_offset: int = 0, rng_seed: int = 0x5EED,
         for j, v in enumerate(obs.scales):
             d.obs_scale[j] = v
         d.obs_height_scale = obs.height_scale
+        for j, v in enumerate(obs.noise):
+            d.obs_noise[j] = v
+        d.obs_height_noise = obs.height_noise
     return d
 
 

@@ -362,12 +362,53 @@ def _exact_offset(q0: float) -> float:
     raise NotFusable(f"compute_observations: no exact dof-position probe around {q0}")
 
 
+@contextmanager
+def _obs_draws(env, u):
+    """While ``compute_observations`` runs: ``torch.rand_like`` of the whole observation returns ``u`` (a
+    number or a tensor of that shape), once per call; any other draw raises NotFusable.  legged_gym's noise
+    is ``obs_buf += (2 * torch.rand_like(obs_buf) - 1) * noise_scale_vec``, which the fused kernel adds."""
+    shape = (env.num_envs, nv.OBS_HEAD + env.isg_env.num_height_points)
+    calls = []
+
+    def rand_like(t, *args, **kwargs):
+        if tuple(t.shape) != shape:
+            raise NotFusable(f"compute_observations: torch.rand_like of a {tuple(t.shape)} tensor; the fused noise "
+                             f"draws one u per column of the whole {shape} observation")
+        calls.append(1)
+        if len(calls) > 1:
+            raise NotFusable("compute_observations: torch.rand_like is called more than once; the fused noise draws "
+                             "one u per column")
+        dtype = t.dtype if t.dtype.is_floating_point else torch.float
+        if isinstance(u, torch.Tensor):
+            return u.to(device=t.device, dtype=dtype)
+        return torch.full(shape, float(u), device=t.device, dtype=dtype)
+
+    def refuse(name):
+        def draw(*args, **kwargs):
+            raise NotFusable(f"compute_observations: draws with torch.{name}; the fused observation noise is "
+                             "uniform: (2 * torch.rand_like(obs_buf) - 1) * scale")
+        return draw
+
+    saved = {name: getattr(torch, name) for name in ("rand_like", "randn_like", "rand", "randn", "normal")}
+    patched = {name: (rand_like if name == "rand_like" else refuse(name)) for name in saved}
+    try:
+        for name, fn in patched.items():
+            setattr(torch, name, fn)
+        yield
+    finally:
+        for name, fn in saved.items():
+            setattr(torch, name, fn)
+
+
 def compile_a1_obs(env) -> ObsLayout:
     """``env.compute_observations`` -> ObsLayout, by probing.  At the zero state (every input zero,
     dof_pos = default_dof_pos, base 0.5 above flat terrain) the observation must be all zeros; then each
     input is set alone to a power of two and must reach exactly one column of its block, the three
     components of a vector in order in one slot; the column's value over the input is its scale.  The
     heights are probed at z - 0.5 - h = 0.5 and 3, which fixes their scale and the clip-then-scale order.
+    Every probe so far runs with ``torch.rand_like`` at u = 0.5, where uniform noise vanishes.  Then, at the
+    zero state, u = 1 gives each column's noise scale and u = 0 must give its negative; the heights share
+    one scale, added after their clip and scale (probed at z - 0.5 - h = 3).
     Anything else raises NotFusable naming the column and the reason."""
     rb, isg = env.robot, env.isg_env
     n_head = nv.OBS_HEAD
@@ -385,9 +426,10 @@ def compile_a1_obs(env) -> ObsLayout:
             t["root"][rb.root_indices, 2] = 0.5
             heights.zero_()
 
-        def observe():
+        def observe(u=0.5):
             isg.measured_heights = heights
-            env.compute_observations()
+            with _obs_draws(env, u):
+                env.compute_observations()
             obs = env.obs_buf
             if tuple(obs.shape) != (env.num_envs, n_head + heights.shape[1]):
                 raise NotFusable(f"compute_observations: shape {tuple(obs.shape)}, the fused observation is "
@@ -470,37 +512,72 @@ def compile_a1_obs(env) -> ObsLayout:
                 raise NotFusable(f"compute_observations: height column {n_head + bad[0]} is {float(hv[bad[0]]):g} at "
                                  f"z - 0.5 - h = 3, not clip(3, -1, 1) * {hs:g}: heights must be clipped to +-1 "
                                  "before they are scaled")
+            # noise: clean + (2u - 1) * s, so +s at u = 1 and -s at u = 0 on the all-zero observation
+            zero_state()
+            up, down = observe(1.0), observe(0.0)
+            bad = torch.nonzero(down != -up).flatten().tolist()
+            if bad:
+                j = bad[0]
+                raise NotFusable(f"compute_observations: column {j} is {float(up[j]):g} at u = 1 and {float(down[j]):g} "
+                                 "at u = 0 with every input at zero; the fused noise is (2u - 1) * scale with "
+                                 "u = torch.rand_like(obs_buf)")
+            hn = float(up[n_head])
+            bad = torch.nonzero(up[n_head:] != hn).flatten().tolist()
+            if bad:
+                raise NotFusable(f"compute_observations: height column {n_head + bad[0]} has noise scale "
+                                 f"{float(up[n_head + bad[0]]):g}, height column {n_head} {hn:g}; the fused observation "
+                                 "has one noise scale for all height columns")
+            if hn != 0.0:
+                heights[0] = -3.0
+                for u, sign in ((1.0, 1.0), (0.0, -1.0)):
+                    want = torch.tensor(hs, dtype=torch.float) + torch.tensor(sign * hn, dtype=torch.float)
+                    hv = observe(u)[n_head:]
+                    bad = torch.nonzero(hv != want).flatten().tolist()
+                    if bad:
+                        raise NotFusable(f"compute_observations: height column {n_head + bad[0]} is "
+                                         f"{float(hv[bad[0]]):g} at z - 0.5 - h = 3 and u = {u:g}, not "
+                                         f"clip(3, -1, 1) * {hs:g} {'+' if sign > 0 else '-'} {hn:g}: the noise must "
+                                         "be added after the heights are clipped and scaled")
+            noise = tuple(float(v) for v in up[:n_head])
         finally:
             if had is None:
                 del isg.measured_heights
             else:
                 isg.measured_heights = had
-    return ObsLayout(tuple(slots), tuple(scales), hs)
+    return ObsLayout(tuple(slots), tuple(scales), hs, noise, hn)
 
 
-def a1_obs_definition(env, layout: ObsLayout) -> torch.Tensor:
+def a1_obs_definition(env, layout: ObsLayout, u: Optional[torch.Tensor] = None) -> torch.Tensor:
     """The observation the fused kernel builds under ``layout``, in torch on the env's tensors (before the
-    final clip to +-clip_obs that the base class applies)."""
+    final clip to +-clip_obs that the base class applies).  ``u``: the noise draws, (num_envs, 259)."""
     rb, isg = env.robot, env.isg_env
     src = {name: getattr(rb if key != "command" else env, label) for name, (key, label) in _OBS_PROBE.items()}
     head = torch.cat([src[name] for name in layout.slots]
                      + [rb.dof_pos - rb.default_dof_pos, rb.dof_vel, env.actions_recorder.flatten()], dim=1)
     head = head * torch.tensor(layout.scales, dtype=torch.float, device=head.device)
     heights = torch.clip(rb.base_pose[:, 2].unsqueeze(1) - 0.5 - isg.measured_heights, -1, 1.) * layout.height_scale
-    return torch.cat([head, heights], dim=1)
+    obs = torch.cat([head, heights], dim=1)
+    if u is not None and layout.has_noise():
+        scale = torch.tensor(layout.noise + (layout.height_noise,) * heights.shape[1], dtype=torch.float,
+                             device=obs.device)
+        obs = obs + (2 * u - 1) * scale
+    return obs
 
 
 def verify_a1_obs(env, layout: ObsLayout, seed: int = 4321):
-    """``env.compute_observations`` against the layout's definition on a seeded random state."""
+    """``env.compute_observations`` against the layout's definition (noise included) on a seeded random
+    state, with the same seeded draws given to the hook's ``torch.rand_like`` and to the definition."""
     isg = env.isg_env
     had = isg.__dict__.get("_measured_heights")
     with A1Probe(env) as pr:
         pr.randomize(seed)
         g = torch.Generator(device=env.device).manual_seed(seed)
         isg.measured_heights = torch.randn(env.num_envs, isg.num_height_points, generator=g, device=env.device)
+        u = torch.rand(env.num_envs, nv.OBS_HEAD + isg.num_height_points, generator=g, device=env.device)
         try:
-            env.compute_observations()
-            check_close(env.obs_buf, a1_obs_definition(env, layout), "compute_observations")
+            with _obs_draws(env, u):
+                env.compute_observations()
+            check_close(env.obs_buf, a1_obs_definition(env, layout, u), "compute_observations")
         finally:
             if had is None:
                 del isg.measured_heights
