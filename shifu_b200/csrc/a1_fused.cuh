@@ -14,7 +14,7 @@
 //   C   thread t owns scan point t: 187-point height scan per env, obs columns 72..258 streamed
 //       straight to HBM (a warp writes 128 contiguous bytes per env)
 // HBM traffic is the algorithmic minimum (every state row read once, obs written once); the scan
-// table (tiled min-of-3 map, 5.4 MB) lives in L2/L1.
+// table (banded min-of-3 map, 5.4 MB) lives in L2/L1.
 #pragma once
 #include "a1_kernels.cuh"
 
@@ -30,8 +30,8 @@ struct A1Smem {
   float head[A1_TILE][A1_HEAD];
   float rterm[SHIFU_MAX_REWARD_TERMS][A1_TILE];   // reward term values, [term][env]
   float cla[3][A1_TILE][3];                         // command (post-reset), base lin vel, base ang vel
-  float4 ev[A1_TILE];                               // (2*zq, zq, wq, unused) of the PRE-reset pose
-  float4 pos[A1_TILE];                              // (x + 0, y + 0, zb = z_postreset - 0.5, unused)
+  ScanEnv ev[A1_TILE];                              // yaw and xy of the PRE-reset pose
+  float zb[A1_TILE];                                // z_postreset - h_off
 };
 
 // Copy `n` floats global -> shared with float4 when both sides are 16-byte aligned.
@@ -224,10 +224,12 @@ __device__ __noinline__ float a1_eval_term(int q, const A1K& k, const A1Smem& s,
 // composed clips are exact, so the reference observation comes out unchanged.  NOISE (the host sets it
 // when o.noisy): observation noise from the same words as the pipelined kernel, one evaluation per
 // column; a compile-time flag, so that the noiseless instantiations keep their registers and code.
-template <bool TILED, bool EXACT_DIV, bool NOISE>
+// The kernel starts at tile first_tile (the tiles before it are the pipelined kernel's); env indices
+// stay absolute, so k and io describe all k.n envs.
+template <bool EXACT_DIV, bool NOISE>
 __global__ void __launch_bounds__(A1_THREADS, 5)
 a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io,
-                       const __grid_constant__ A1Obs o) {
+                       const __grid_constant__ A1Obs o, int first_tile) {
   __shared__ __align__(16) A1Smem s;
   // projected gravity at the start of the step: warp 5 overwrites io.projected_gravity in phase B3
   // (carry_body_frame) while the other threads build the head
@@ -236,9 +238,8 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
   const long long step = (io.step_dev != nullptr) ? *io.step_dev : io.step;
   // scan point owned by this thread (threads 187..191 idle in phase C)
   const float bx = k.px[t % A1_NX], by = k.py[(t / A1_NX) % A1_NY];
-  const unsigned max_px = (unsigned)(k.trows - 1), max_py = (unsigned)(k.tcols - 1);
 
-  for (int e0 = blockIdx.x * A1_TILE; e0 < k.n; e0 += gridDim.x * A1_TILE) {
+  for (int e0 = (first_tile + blockIdx.x) * A1_TILE; e0 < k.n; e0 += gridDim.x * A1_TILE) {
     const int ne = min(A1_TILE, k.n - e0);
     const int ge = e0 + lane;                      // env of this lane in the lane = env phases
     const bool lane_env = (lane < ne);
@@ -274,13 +275,8 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
       for (int j = warp; j < k.n_terms; j += A1_THREADS / 32) s.rterm[j][lane] = a1_eval_term(j, k, s, lane, io, ge);
       if (warp == 0)                                                    // a1_conditional.py:146-148
         contact_term = force_exceeds(&s.contact[lane][k.base_body * 3], k.contact_thr_sq);
-      if (warp == 5) {
-        // heights are measured at the PRE-reset pose (isaac_gym.py:320-322 runs before post_step)
-        const ScanEnv ev = make_scan_env(s.root[lane]);
-        s.ev[lane] = make_float4(ev.z2, ev.z, ev.w, 0.0f);
-        s.pos[lane].x = ev.x;
-        s.pos[lane].y = ev.y;
-      }
+      if (warp == 5)    // heights are measured at the PRE-reset pose (isaac_gym.py:320-322 runs before post_step)
+        s.ev[lane] = make_scan_env(s.root[lane]);
     }
     __syncthreads();
 
@@ -320,7 +316,7 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
 #pragma unroll
         for (int j = 0; j < SHIFU_MAX_REWARD_TERMS; ++j)
           if (j < k.n_terms) io.ep_sums[j][ge] = esum[j];
-        s.pos[lane].z = sub_rn(s.root[lane][2], k.h_off);                  // post-reset base z (D8)
+        s.zb[lane] = sub_rn(s.root[lane][2], k.h_off);                     // post-reset base z (D8)
       }
       a1_log_sums(k, reset, st_sum, level_delta, lane);
     }
@@ -387,31 +383,11 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
       float* orow = io.obs_buf + (long long)e0 * A1_OBS + A1_HEAD + t;
       float* mrow = (io.measured_heights != nullptr) ? io.measured_heights + (long long)e0 * A1_POINTS + t
                                                      : nullptr;
-      const short* __restrict__ table = k.table;
 #pragma unroll (NOISE ? 1 : 4)            // with NOISE: a Philox evaluation per env, unrolled it spills
       for (int e = 0; e < ne; ++e) {
-        const float4 ev = s.ev[e];          // (2z, z, w, -)
-        const float4 ps = s.pos[e];         // (x, y, zb, -)
-        // quat_apply_yaw (shifu/utils/terrain.py:202-206) on (bx, by, 0)
-        const float tx = -mul_rn(ev.x, by);
-        const float ty = mul_rn(ev.x, bx);
-        const float rx = add_rn(add_rn(bx, mul_rn(ev.z, tx)), -mul_rn(ev.y, ty));
-        const float ry = add_rn(add_rn(by, mul_rn(ev.z, ty)), mul_rn(ev.y, tx));
-        // + base xy, + border, / horizontal_scale, .long(), clip (isaac_gym.py:416-425)
-        const float ax = add_rn(add_rn(rx, ps.x), k.border);
-        const float ay = add_rn(add_rn(ry, ps.y), k.border);
-        const float fx = EXACT_DIV ? div_rn(ax, k.hdiv.d) : div_const(ax, k.hdiv);
-        const float fy = EXACT_DIV ? div_rn(ay, k.hdiv.d) : div_const(ay, k.hdiv);
-        const unsigned px = min(__float2uint_rz(fx), max_px);
-        const unsigned py = min(__float2uint_rz(fy), max_py);
-        int idx;
-        if (TILED) {
-          idx = (int)((px & ~7u) * (unsigned)(k.band_w - 1) + px + (py << TILE_SHIFT));
-        } else {
-          idx = (int)(px * (unsigned)k.tcols + py);
-        }
-        const float hgt = mul_rn((float)__ldg(table + idx), k.vscale);      // isaac_gym.py:427-433
-        float v = mul_rn(clampf(sub_rn(ps.z, hgt), -k.h_clip, k.h_clip), o.h_scale);
+        unsigned px, py;
+        const float hgt = scan_point<EXACT_DIV>(s.ev[e], bx, by, k, &px, &py);
+        float v = mul_rn(clampf(sub_rn(s.zb[e], hgt), -k.h_clip, k.h_clip), o.h_scale);
         if (NOISE) v = add_rn(v, obs_noise_at(o, k.seed, k.env_offset + e0 + e, step, A1_HEAD + t));
         v = clampf(v, -k.clip_obs, k.clip_obs);
         __stcs(orow + (long long)e * A1_OBS, v);

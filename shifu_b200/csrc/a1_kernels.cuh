@@ -3,7 +3,7 @@
 // Everything here is HBM-/LSU-bound fp32 + integer work; there is no contraction, so no
 // tensor-core path.  The design rules that matter: one pass over every state tensor with
 // coalesced 128-bit loads, the obs row written once with streaming stores, grids sized by the
-// SM count, and the 187-point height scan served from an L2-resident tiled table.
+// SM count, and the 187-point height scan served from an L2-resident banded table.
 #pragma once
 #include "exact_math.cuh"
 #include "philox.cuh"
@@ -56,10 +56,9 @@ struct A1K {
   int term_count[A1K_TERM_WARPS], term_list[A1K_TERM_WARPS][SHIFU_MAX_REWARD_TERMS];
   float contact_thr_sq;
   // scan table
-  const short* table;     // tiled min-of-3 table
+  const short* table;     // banded min-of-3 table T[px>>3][py][px&7]: a 128-B line = 8x8 cells
   int trows, tcols;       // valid index range: px in [0, trows-1], py in [0, tcols-1]
-  int band_w;             // banded layout: entries per map row inside a band (tcols padded to 8)
-  int tiled;              // 1: banded (T[px>>3][py][px&7], a 128-B line = 8x8 cells), 0: row-major (pitch = tcols)
+  int band_w;             // entries per map row inside a band (tcols padded to 8)
   double* stats;          // SHIFU_NUM_STATS accumulators
   float neg_zero;         // -0.0f, opaque to ptxas: see the fma(a, b, -0) products in scan_pairs.cuh
 };
@@ -108,14 +107,9 @@ __device__ __forceinline__ float a1_obs_vec(const A1Obs& o, int j, const Cla& cl
   }
 }
 
-__device__ __forceinline__ float hdivide(float x, const A1K& k) {
-  return k.exact_div ? div_rn(x, k.hdiv.d) : div_const(x, k.hdiv);
-}
-
 __device__ __forceinline__ int table_index(unsigned px, unsigned py, const A1K& k) {
-  if (k.tiled)     // (px>>3)*8*W + py*8 + (px&7)  ==  (px & ~7)*(W-1) + px + 8*py      (3 integer ops)
-    return (int)((px & ~7u) * (unsigned)(k.band_w - 1) + px + (py << TILE_SHIFT));
-  return (int)(px * (unsigned)k.tcols + py);
+  // (px>>3)*8*W + py*8 + (px&7)  ==  (px & ~7)*(W-1) + px + 8*py      (3 integer ops)
+  return (int)((px & ~7u) * (unsigned)(k.band_w - 1) + px + (py << TILE_SHIFT));
 }
 
 // ------------------------------------------------------------------------------------------
@@ -123,7 +117,7 @@ __device__ __forceinline__ int table_index(unsigned px, unsigned py, const A1K& 
 // (shifu/gym/isaac_gym.py:427-431 folded; the map is static after create_ground()).
 // ------------------------------------------------------------------------------------------
 __global__ void build_scan_table_kernel(const short* __restrict__ H, int rows, int cols,
-                                        short* __restrict__ T, int band_w, int tiled) {
+                                        short* __restrict__ T, int band_w) {
   const int trows = rows - 1, tcols = cols - 1;
   const long long total = (long long)trows * tcols;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
@@ -132,14 +126,7 @@ __global__ void build_scan_table_kernel(const short* __restrict__ H, int rows, i
     const short a = H[(long long)px * cols + py];
     const short b = H[(long long)(px + 1) * cols + py];
     const short c = H[(long long)px * cols + py + 1];
-    const short m = min(min(a, b), c);
-    long long o;
-    if (tiled) {
-      o = (long long)(px >> TILE_SHIFT) * 8 * band_w + (long long)py * 8 + (px & 7);
-    } else {
-      o = (long long)px * tcols + py;
-    }
-    T[o] = m;
+    T[(long long)(px >> TILE_SHIFT) * 8 * band_w + (long long)py * 8 + (px & 7)] = min(min(a, b), c);
   }
 }
 
@@ -284,6 +271,8 @@ __device__ __forceinline__ ScanEnv make_scan_env(const float* root_row) {
   return ev;
 }
 
+// EXACT_DIV: / horizontal_scale as __fdiv_rn (A1K::exact_div), else the 3-op constant division
+template <bool EXACT_DIV>
 __device__ __forceinline__ float scan_point(const ScanEnv& ev, float bx, float by, const A1K& k,
                                             unsigned* opx, unsigned* opy) {
   // t = 2*(q_xyz x b) with q_xyz = (0,0,z), b = (bx,by,0)  ->  (-2z*by, 2z*bx, 0)
@@ -293,8 +282,10 @@ __device__ __forceinline__ float scan_point(const ScanEnv& ev, float bx, float b
   const float rx = add_rn(add_rn(bx, mul_rn(ev.w, tx)), -mul_rn(ev.z, ty));
   const float ry = add_rn(add_rn(by, mul_rn(ev.w, ty)), mul_rn(ev.z, tx));
   // + base xy, + border, / horizontal_scale, .long() (trunc), clip to [0, dim-2]
-  const float fx = hdivide(add_rn(add_rn(rx, ev.x), k.border), k);
-  const float fy = hdivide(add_rn(add_rn(ry, ev.y), k.border), k);
+  const float ax = add_rn(add_rn(rx, ev.x), k.border);
+  const float ay = add_rn(add_rn(ry, ev.y), k.border);
+  const float fx = EXACT_DIV ? div_rn(ax, k.hdiv.d) : div_const(ax, k.hdiv);
+  const float fy = EXACT_DIV ? div_rn(ay, k.hdiv.d) : div_const(ay, k.hdiv);
   // float->unsigned conversion truncates toward zero and saturates (negatives -> 0)
   const unsigned px = min(__float2uint_rz(fx), (unsigned)(k.trows - 1));
   const unsigned py = min(__float2uint_rz(fy), (unsigned)(k.tcols - 1));
@@ -319,7 +310,8 @@ get_heights_kernel(const __grid_constant__ A1K k, const float* __restrict__ root
     if (t < A1_POINTS) {
       for (int e = 0; e < ne; ++e) {
         unsigned px, py;
-        const float h = scan_point(s_ev[e], bx, by, k, &px, &py);
+        const float h = k.exact_div ? scan_point<true>(s_ev[e], bx, by, k, &px, &py)
+                                    : scan_point<false>(s_ev[e], bx, by, k, &px, &py);
         const long long o = (long long)(e0 + e) * A1_POINTS + t;
         mh[o] = h;
         if (cell_idx != nullptr) { cell_idx[2 * o] = (int)px; cell_idx[2 * o + 1] = (int)py; }

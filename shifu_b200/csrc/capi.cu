@@ -328,16 +328,14 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
   if (e == cudaSuccess && c->is_a1) {
     // all four instantiations share resources; ask for the full shared-memory carve-out so the
     // resident-CTA count is bounded by registers/threads, not by the default L1/smem split
-    const void* variants[8] = {
-        (const void*)a1_post_physics_kernel<true, false, false>, (const void*)a1_post_physics_kernel<true, true, false>,
-        (const void*)a1_post_physics_kernel<false, false, false>, (const void*)a1_post_physics_kernel<false, true, false>,
-        (const void*)a1_post_physics_kernel<true, false, true>, (const void*)a1_post_physics_kernel<true, true, true>,
-        (const void*)a1_post_physics_kernel<false, false, true>, (const void*)a1_post_physics_kernel<false, true, true>};
-    for (int v = 0; v < 8 && e == cudaSuccess; ++v)
+    const void* variants[4] = {
+        (const void*)a1_post_physics_kernel<false, false>, (const void*)a1_post_physics_kernel<true, false>,
+        (const void*)a1_post_physics_kernel<false, true>, (const void*)a1_post_physics_kernel<true, true>};
+    for (int v = 0; v < 4 && e == cudaSuccess; ++v)
       e = cudaFuncSetAttribute(variants[v], cudaFuncAttributePreferredSharedMemoryCarveout, 75);
     int occ = 0;
     if (e == cudaSuccess)
-      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, a1_post_physics_kernel<true, false, false>, A1_THREADS, 0);
+      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, a1_post_physics_kernel<false, false>, A1_THREADS, 0);
     const int tiles = (n + A1_TILE - 1) / A1_TILE;
     const int cap = c->sm_count * (occ > 0 ? occ : 1);
     c->a1_grid = tiles < cap ? tiles : cap;
@@ -402,23 +400,21 @@ extern "C" int shifu_set_height_map(ShifuCtx* c, const int16_t* hs, int32_t rows
   REQUIRE_PTR(c); REQUIRE_PTR(hs);
   if (!c->is_a1) return fail(SHIFU_E_STATE, "height map only applies to an A1 ctx");
   if (rows < 2 || cols < 2 || (long long)rows * cols > (1LL << 30)) return fail(SHIFU_E_RANGE, "map %dx%d out of range", rows, cols);
-  const char* layout = getenv("SHIFU_TABLE_LAYOUT");
-  const int tiled = (layout != nullptr && strcmp(layout, "rowmajor") == 0) ? 0 : 1;
   const int trows = rows - 1, tcols = cols - 1;
   // banded layout T[px>>3][py][px&7]: the 8 rows of a band are interleaved per column, so a 128-B
   // line still holds an 8x8-cell patch of the map while the index needs 3 integer ops
   const int bands = (trows + 7) / 8, band_w = ((tcols + 7) / 8) * 8;
-  const size_t elems = tiled ? (size_t)bands * 8 * band_w : (size_t)trows * tcols;
+  const size_t elems = (size_t)bands * 8 * band_w;
   CUDA_TRY(cudaStreamSynchronize(S(stream)));
   if (c->d_table != nullptr) { cudaFree(c->d_table); c->d_table = nullptr; }
   CUDA_TRY(cudaMalloc(&c->d_table, elems * sizeof(short)));
   CUDA_TRY(cudaMemsetAsync(c->d_table, 0, elems * sizeof(short), S(stream)));
   build_scan_table_kernel<<<grid_for((long long)trows * tcols, 256, c->sm_count, 8), 256, 0, S(stream)>>>(
-      hs, rows, cols, c->d_table, band_w, tiled);
+      hs, rows, cols, c->d_table, band_w);
   CUDA_TRY(cudaGetLastError());
   CUDA_TRY(cudaStreamSynchronize(S(stream)));
   c->a1k.table = c->d_table;
-  c->a1k.trows = trows; c->a1k.tcols = tcols; c->a1k.band_w = band_w; c->a1k.tiled = tiled;
+  c->a1k.trows = trows; c->a1k.tcols = tcols; c->a1k.band_w = band_w;
   return SHIFU_OK;
 }
 
@@ -468,8 +464,7 @@ extern "C" int shifu_get_heights(ShifuCtx* c, const float* root, float* mh, int3
   if (!c->is_a1) return fail(SHIFU_E_STATE, "shifu_get_heights needs an A1 ctx");
   if (c->d_table == nullptr) return fail(SHIFU_E_STATE, "call shifu_set_height_map first");
   const int tiles = (c->a1.num_envs + A1_TILE - 1) / A1_TILE;
-  if (cell_idx == nullptr && c->a1k.tiled && !c->a1k.exact_div && c->grid_symmetric &&
-      !(getenv("SHIFU_A1_KERNEL") != nullptr && strcmp(getenv("SHIFU_A1_KERNEL"), "phased") == 0)) {
+  if (cell_idx == nullptr && !c->a1k.exact_div && c->grid_symmetric && c->use_tma) {
     const int cap4 = c->sm_count * 4;                   // packed, one rotation per point pair (scan_pairs.cuh)
     get_heights_pairs_kernel<<<tiles < cap4 ? tiles : cap4, SP_THREADS, 0, S(stream)>>>(c->a1k, root, mh);
     CUDA_TRY(cudaGetLastError());
@@ -508,7 +503,7 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
   for (int j = 0; j < c->a1.num_reward_terms; ++j)
     if (io->ep_sums[j] == nullptr) return fail(SHIFU_E_NULL, "ep_sums[%d] is NULL", j);
   REQUIRE_ALIGNED(io->dof_state, 16);
-  const bool tiled = c->a1k.tiled != 0, exact = c->a1k.exact_div != 0;
+  const bool exact = c->a1k.exact_div != 0;
   const int n = c->a1.num_envs;
 
   // Pipelined TMA kernel for the full 32-env tiles when the layout allows bulk copies
@@ -516,7 +511,7 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
   // tail (< 32 envs) or everything when bulk copies are not possible.
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
   // the pipelined scan rotates once per point pair: it needs the point-symmetric grid (else: phased kernel)
-  const bool can_tma = c->use_tma && tiled && c->grid_symmetric && c->a1k.root_stride == 1 && c->a1k.root_offset == 0 && al16(io->root_state) &&
+  const bool can_tma = c->use_tma && c->grid_symmetric && c->a1k.root_stride == 1 && c->a1k.root_offset == 0 && al16(io->root_state) &&
                        al16(io->dof_state) && al16(io->contact_state) && al16(io->history) && al16(io->torques) &&
                        al16(io->actions) && al16(io->obs_buf) && al16(io->ep_len) && al16(io->command) &&
                        al16(io->base_lin_vel) && al16(io->base_ang_vel) && al16(io->projected_gravity) &&
@@ -534,40 +529,18 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     const int variant = (c->obs_custom ? 8 : 0) + (c->a1o.noisy ? 8 : 0) + (exact ? 4 : 0) + (mrow ? 2 : 0) + (extra ? 1 : 0);
     CUDA_TRY(cudaLaunchKernel(a1_tma_variants()[variant], grid, block, args, smem, S(stream)));
   }
-  const int done = full_tiles * A1_TILE;
-  if (done < n) {
-    A1K k = c->a1k;
-    ShifuA1StepIO t = *io;
-    if (done > 0) {                       // shift every per-env tensor to the first tail env
-      const size_t e = (size_t)done;
-      k.n = n - done;
-      k.env_offset += done;
-      t.root_state += e * 13; t.dof_state += e * (A1_DOF * 2); t.contact_state += e * (A1_BODIES * 3);
-      t.actions += e * A1_DOF; t.torques += e * A1_DOF; t.history += e * (A1_DOF * A1_HIST);
-      t.command += e * 3; t.ep_len += e;
-      for (int j = 0; j < SHIFU_MAX_REWARD_TERMS; ++j) if (t.ep_sums[j] != nullptr) t.ep_sums[j] += e;
-      t.base_lin_vel += e * 3; t.base_ang_vel += e * 3; t.projected_gravity += e * 3;
-      t.env_origins += e * 3; t.terrain_levels += e; t.terrain_types += e;
-      t.dof_targets += e * A1_DOF; t.rand_force += e * (A1_BODIES * 3);
-      t.obs_buf += e * A1_OBS; t.rew_buf += e; t.reset_buf += e; t.time_out_buf += e; t.contact_term_buf += e;
-      if (t.measured_heights != nullptr) t.measured_heights += e * A1_POINTS;
-      if (t.swing_time != nullptr) t.swing_time += e * k.n_feet;
-      if (t.last_contacts != nullptr) t.last_contacts += e * k.n_feet;
-    }
-    const int tiles = (k.n + A1_TILE - 1) / A1_TILE;
+  const int tiles = (n + A1_TILE - 1) / A1_TILE - full_tiles;    // the ragged tail, or every tile
+  if (tiles > 0) {
     const int cap = c->sm_count * (c->a1_occ > 0 ? c->a1_occ : 1);
     const dim3 grid(tiles < cap ? tiles : cap), block(A1_THREADS);
+    const A1K& k = c->a1k;
     const A1Obs& o = c->a1o;
     if (o.noisy) {
-      if (tiled && !exact) a1_post_physics_kernel<true, false, true><<<grid, block, 0, S(stream)>>>(k, t, o);
-      else if (tiled && exact) a1_post_physics_kernel<true, true, true><<<grid, block, 0, S(stream)>>>(k, t, o);
-      else if (!tiled && !exact) a1_post_physics_kernel<false, false, true><<<grid, block, 0, S(stream)>>>(k, t, o);
-      else a1_post_physics_kernel<false, true, true><<<grid, block, 0, S(stream)>>>(k, t, o);
+      if (exact) a1_post_physics_kernel<true, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      else a1_post_physics_kernel<false, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
     } else {
-      if (tiled && !exact) a1_post_physics_kernel<true, false, false><<<grid, block, 0, S(stream)>>>(k, t, o);
-      else if (tiled && exact) a1_post_physics_kernel<true, true, false><<<grid, block, 0, S(stream)>>>(k, t, o);
-      else if (!tiled && !exact) a1_post_physics_kernel<false, false, false><<<grid, block, 0, S(stream)>>>(k, t, o);
-      else a1_post_physics_kernel<false, true, false><<<grid, block, 0, S(stream)>>>(k, t, o);
+      if (exact) a1_post_physics_kernel<true, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      else a1_post_physics_kernel<false, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
     }
     CUDA_TRY(cudaGetLastError());
   }

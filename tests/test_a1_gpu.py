@@ -121,15 +121,6 @@ def test_height_cell_indices_bit_exact():
     want, widx = so.get_heights(p, root[:, :7], torch.from_numpy(hs), p.height_points(), return_idx=True)
     assert torch.equal(idx[:, 0].cpu().long(), widx[0]) and torch.equal(idx[:, 1].cpu().long(), widx[1])
     assert torch.equal(mh.cpu(), want)
-    # the row-major table layout must give the same answer as the tiled one
-    import os
-    os.environ["SHIFU_TABLE_LAYOUT"] = "rowmajor"
-    try:
-        hp2 = util.make_cuda_a1(n, hs, origins, types, env_origins)
-        hp2.root_state.copy_(root.cuda())
-        assert torch.equal(hp2.get_heights().cpu(), want)
-    finally:
-        del os.environ["SHIFU_TABLE_LAYOUT"]
 
 
 @pytest.mark.parametrize("n", [1, 31, 33, 4096 + 17, 65536])
