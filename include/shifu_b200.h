@@ -52,7 +52,8 @@ extern "C" {
  * issues that evaluation in the same slots whether one lane or two run it): 24 evaluations for the 18 head
  * words.  The two lanes of height point pairs k, k^1 each evaluate word 18 + (k >> 1) for one env of an env
  * pair and swap halves, so every lane of those evaluations is used; the two idle scan lanes evaluate word 64
- * for nothing. */
+ * for nothing.
+ * A 72-column (blind, num_obs = SHIFU_OBS_HEAD) observation draws words 0-17 only, with the same map. */
 #define SHIFU_STREAM_OBS_NOISE 8
 
 enum {
@@ -129,7 +130,10 @@ typedef struct ShifuA1Desc {
   int32_t num_dof;              /* 12 */
   int32_t num_bodies;           /* 17: contact rows per env */
   int32_t num_hist;             /* 3  (cfg.num_actions_history) */
-  int32_t num_obs;              /* 259 */
+  int32_t num_obs;              /* 259, or SHIFU_OBS_HEAD (72) for a blind task: obs_buf is (N,72), the
+                                   measured heights are neither scanned nor written (measured_heights must be
+                                   NULL), obs_height_scale is not read, obs_height_noise must be 0, and
+                                   shifu_a1_post_physics needs no shifu_set_height_map */
   int32_t base_body;            /* contact_terminate_indices, a1_conditional.py:98-99 */
   int32_t num_leg_bodies;       /* 8 */
   int32_t leg_bodies[SHIFU_MAX_LEG_BODIES]; /* a1_conditional.py:59-61 */
@@ -212,12 +216,12 @@ typedef struct ShifuA1StepIO {
   const float* terrain_origins;   /* (levels, types, 3) */
   float* dof_targets;             /* w on reset (N,12) (robot.py:75) */
   float* rand_force;              /* w on reset (N,17,3) (a1_conditional.py:82-87) */
-  float* obs_buf;                 /* w (N,259) already clipped to +-clip_obs */
+  float* obs_buf;                 /* w (N,num_obs) already clipped to +-clip_obs */
   float* rew_buf;                 /* w (N) */
   uint8_t* reset_buf;             /* w (N) bool */
   uint8_t* time_out_buf;          /* w (N) bool */
   uint8_t* contact_term_buf;      /* w (N) bool */
-  float* measured_heights;        /* optional w (N,187), may be NULL */
+  float* measured_heights;        /* optional w (N,187), may be NULL; must be NULL when num_obs = 72 */
   int64_t step;                   /* common_step_counter AFTER its increment (env.py:96): Philox counter */
   const int64_t* step_dev;        /* optional: when non-NULL the step is read from this device word
                                      instead (lets a captured CUDA graph replay with a moving

@@ -226,7 +226,9 @@ __device__ __noinline__ float a1_eval_term(int q, const A1K& k, const A1Smem& s,
 // column; a compile-time flag, so that the noiseless instantiations keep their registers and code.
 // The kernel starts at tile first_tile (the tiles before it are the pipelined kernel's); env indices
 // stay absolute, so k and io describe all k.n envs.
-template <bool EXACT_DIV, bool NOISE>
+// BLIND: the 72-column observation without the height scan (no phase C, obs rows of A1_HEAD floats);
+// EXACT_DIV does not apply.
+template <bool EXACT_DIV, bool NOISE, bool BLIND>
 __global__ void __launch_bounds__(A1_THREADS, 5)
 a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io,
                        const __grid_constant__ A1Obs o, int first_tile) {
@@ -236,6 +238,7 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
   __shared__ float pg0[A1_TILE][3];
   const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
   const long long step = (io.step_dev != nullptr) ? *io.step_dev : io.step;
+  constexpr int OW = BLIND ? A1_HEAD : A1_OBS;     // obs row stride
   // scan point owned by this thread (threads 187..191 idle in phase C)
   const float bx = k.px[t % A1_NX], by = k.py[(t / A1_NX) % A1_NY];
 
@@ -275,7 +278,7 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
       for (int j = warp; j < k.n_terms; j += A1_THREADS / 32) s.rterm[j][lane] = a1_eval_term(j, k, s, lane, io, ge);
       if (warp == 0)                                                    // a1_conditional.py:146-148
         contact_term = force_exceeds(&s.contact[lane][k.base_body * 3], k.contact_thr_sq);
-      if (warp == 5)    // heights are measured at the PRE-reset pose (isaac_gym.py:320-322 runs before post_step)
+      if (!BLIND && warp == 5)    // heights are measured at the PRE-reset pose (isaac_gym.py:320-322 runs before post_step)
         s.ev[lane] = make_scan_env(s.root[lane]);
     }
     __syncthreads();
@@ -368,18 +371,18 @@ a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ Sh
 
     // ---- phase D: obs head + history tile ------------------------------------------------------
     {
-      float* obase = io.obs_buf + (long long)e0 * A1_OBS;
+      float* obase = io.obs_buf + (long long)e0 * OW;
       const float* hsrc = &s.head[0][0];
       for (int i = t; i < ne * A1_HEAD; i += A1_THREADS) {
         const int e = i / A1_HEAD, j = i - e * A1_HEAD;
-        __stcs(obase + (long long)e * A1_OBS + j, hsrc[i]);
+        __stcs(obase + (long long)e * OW + j, hsrc[i]);
       }
       store_span(io.history + (long long)e0 * (A1_DOF * A1_HIST), &s.hist[0][0], ne * A1_DOF * A1_HIST, t,
                  A1_THREADS);
     }
 
     // ---- phase C: 187-point scan; obs[., 72 + t] = clip(clip((z - 0.5) - h, +-1) * h_scale [+ noise], +-clip_obs)
-    if (t < A1_POINTS) {
+    if (!BLIND && t < A1_POINTS) {
       float* orow = io.obs_buf + (long long)e0 * A1_OBS + A1_HEAD + t;
       float* mrow = (io.measured_heights != nullptr) ? io.measured_heights + (long long)e0 * A1_POINTS + t
                                                      : nullptr;

@@ -69,6 +69,8 @@ struct ShifuCtx {
   int tma_occ = 0;
   bool use_tma = true;
   bool grid_symmetric = false;     // measured-point grid is point-symmetric (what the pipelined scan assumes)
+  bool blind = false;              // num_obs = SHIFU_OBS_HEAD: no height columns, no scan
+  int blind_occ = 0;
 };
 
 static inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
@@ -86,6 +88,15 @@ static void a1_tma_fill(const void** t) {
   t[5] = (const void*)a1_post_physics_tma_kernel<true, false, true, OBS, NOISE>;
   t[6] = (const void*)a1_post_physics_tma_kernel<true, true, false, OBS, NOISE>;
   t[7] = (const void*)a1_post_physics_tma_kernel<true, true, true, OBS, NOISE>;
+}
+// the blind pipelined kernel's instantiations, index = 2*(OBS + NOISE) + HAS_EXTRA (NOISE only with OBS)
+constexpr int A1_BLIND_VARIANTS = 6;
+static const void* const* a1_blind_variants() {
+  static const void* const table[A1_BLIND_VARIANTS] = {
+      (const void*)a1_post_physics_blind_kernel<false, false, false>, (const void*)a1_post_physics_blind_kernel<true, false, false>,
+      (const void*)a1_post_physics_blind_kernel<false, true, false>, (const void*)a1_post_physics_blind_kernel<true, true, false>,
+      (const void*)a1_post_physics_blind_kernel<false, true, true>, (const void*)a1_post_physics_blind_kernel<true, true, true>};
+  return table;
 }
 static const void* const* a1_tma_variants() {
   static const void* table[A1_TMA_VARIANTS];
@@ -125,6 +136,9 @@ static int fill_a1obs(const ShifuA1Desc& d, A1Obs& o, bool& custom) {
     if (v != 0.0f && d.obs_layout == 0)
       return fail(SHIFU_E_RANGE, "observation noise needs obs_layout = 1 (obs_layout = 0 ignores the layout fields)");
   }
+  if (d.num_obs == A1_HEAD && d.obs_height_noise != 0.0f)
+    return fail(SHIFU_E_RANGE, "obs_height_noise=%g with num_obs = %d: a blind observation has no height columns",
+                (double)d.obs_height_noise, A1_HEAD);
   if (d.obs_layout == 0) return SHIFU_OK;
   for (int i = 0; i < 4; ++i) {
     if (d.obs_vec_src[i] < 0 || d.obs_vec_src[i] >= SHIFU_OBS_VEC_COUNT)
@@ -138,11 +152,13 @@ static int fill_a1obs(const ShifuA1Desc& d, A1Obs& o, bool& custom) {
     custom |= d.obs_scale[j] != 1.0f;
     o.scale[j] = d.obs_scale[j];
   }
-  if (!std::isfinite(d.obs_height_scale))
-    return fail(SHIFU_E_RANGE, "obs_height_scale=%g is not finite", (double)d.obs_height_scale);
-  custom |= d.obs_height_scale != 1.0f;
-  o.h_scale = d.obs_height_scale;
-  o.h_bound = std::fmin(d.height_clip * std::fabs(o.h_scale), d.clip_obs);
+  if (d.num_obs != A1_HEAD) {                              // a blind observation has no height columns
+    if (!std::isfinite(d.obs_height_scale))
+      return fail(SHIFU_E_RANGE, "obs_height_scale=%g is not finite", (double)d.obs_height_scale);
+    custom |= d.obs_height_scale != 1.0f;
+    o.h_scale = d.obs_height_scale;
+    o.h_bound = std::fmin(d.height_clip * std::fabs(o.h_scale), d.clip_obs);
+  }
   for (int j = 0; j < A1_HEAD; ++j) { o.noise[j] = d.obs_noise[j]; o.noisy |= d.obs_noise[j] != 0.0f; }
   o.h_noise = d.obs_height_noise;
   o.noisy |= d.obs_height_noise != 0.0f;
@@ -153,12 +169,12 @@ static int fill_a1obs(const ShifuA1Desc& d, A1Obs& o, bool& custom) {
 static int fill_a1k(const ShifuA1Desc& d, A1K& k) {
   if (d.abi_version != SHIFU_ABI_VERSION) return fail(SHIFU_E_RANGE, "ShifuA1Desc.abi_version %d != %d", d.abi_version, SHIFU_ABI_VERSION);
   if (d.num_envs <= 0) return fail(SHIFU_E_RANGE, "num_envs must be > 0 (got %d)", d.num_envs);
-  if (d.num_dof != A1_DOF || d.num_bodies != A1_BODIES || d.num_hist != A1_HIST || d.num_obs != A1_OBS ||
-      d.num_points_x != A1_NX || d.num_points_y != A1_NY)
+  if (d.num_dof != A1_DOF || d.num_bodies != A1_BODIES || d.num_hist != A1_HIST ||
+      (d.num_obs != A1_OBS && d.num_obs != A1_HEAD) || d.num_points_x != A1_NX || d.num_points_y != A1_NY)
     return fail(SHIFU_E_RANGE,
-                "this build is specialised for dof=%d bodies=%d hist=%d obs=%d grid=%dx%d (got %d %d %d %d %dx%d)",
-                A1_DOF, A1_BODIES, A1_HIST, A1_OBS, A1_NX, A1_NY, d.num_dof, d.num_bodies, d.num_hist, d.num_obs,
-                d.num_points_x, d.num_points_y);
+                "this build is specialised for dof=%d bodies=%d hist=%d obs=%d or %d grid=%dx%d (got %d %d %d %d %dx%d)",
+                A1_DOF, A1_BODIES, A1_HIST, A1_OBS, A1_HEAD, A1_NX, A1_NY, d.num_dof, d.num_bodies, d.num_hist,
+                d.num_obs, d.num_points_x, d.num_points_y);
   if (d.base_body < 0 || d.base_body >= A1_BODIES || d.force_body < 0 || d.force_body >= A1_BODIES)
     return fail(SHIFU_E_RANGE, "base_body/force_body out of range");
   if (d.num_leg_bodies < 0 || d.num_leg_bodies > SHIFU_MAX_LEG_BODIES) return fail(SHIFU_E_RANGE, "num_leg_bodies out of range");
@@ -312,6 +328,7 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
   int n = 0;
   if (a1 != nullptr) {
     c->is_a1 = true; c->a1 = *a1; c->a1k = a1k; c->a1o = a1o; c->obs_custom = obs_custom; n = a1->num_envs;
+    c->blind = a1->num_obs == A1_HEAD;
     c->grid_symmetric = true;
     for (int i = 0; i < A1_NX; ++i) c->grid_symmetric &= (a1k.px[i] == -a1k.px[A1_NX - 1 - i]);
     for (int i = 0; i < A1_NY; ++i) c->grid_symmetric &= (a1k.py[i] == -a1k.py[A1_NY - 1 - i]);
@@ -328,14 +345,15 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
   if (e == cudaSuccess && c->is_a1) {
     // all four instantiations share resources; ask for the full shared-memory carve-out so the
     // resident-CTA count is bounded by registers/threads, not by the default L1/smem split
-    const void* variants[4] = {
-        (const void*)a1_post_physics_kernel<false, false>, (const void*)a1_post_physics_kernel<true, false>,
-        (const void*)a1_post_physics_kernel<false, true>, (const void*)a1_post_physics_kernel<true, true>};
-    for (int v = 0; v < 4 && e == cudaSuccess; ++v)
+    const void* variants[6] = {
+        (const void*)a1_post_physics_kernel<false, false, false>, (const void*)a1_post_physics_kernel<true, false, false>,
+        (const void*)a1_post_physics_kernel<false, true, false>, (const void*)a1_post_physics_kernel<true, true, false>,
+        (const void*)a1_post_physics_kernel<false, false, true>, (const void*)a1_post_physics_kernel<false, true, true>};
+    for (int v = 0; v < 6 && e == cudaSuccess; ++v)
       e = cudaFuncSetAttribute(variants[v], cudaFuncAttributePreferredSharedMemoryCarveout, 75);
     int occ = 0;
     if (e == cudaSuccess)
-      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, a1_post_physics_kernel<false, false>, A1_THREADS, 0);
+      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, a1_post_physics_kernel<false, false, false>, A1_THREADS, 0);
     const int tiles = (n + A1_TILE - 1) / A1_TILE;
     const int cap = c->sm_count * (occ > 0 ? occ : 1);
     c->a1_grid = tiles < cap ? tiles : cap;
@@ -363,6 +381,23 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
       e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&tocc, a1_post_physics_tma_kernel<false, false, false, false, false>, V3_THREADS,
                                                         sizeof(V3Smem));
     c->tma_occ = tocc;
+    // blind pipelined variants: VB_CTAS_PER_SM CTAs of VBSmem each; no scan table, so L1 keeps the rest
+    if (e == cudaSuccess && smem_sm > 0) {
+      const long long need = (long long)VB_CTAS_PER_SM * ((long long)sizeof(VBSmem) + 1024);
+      carve = (int)((need * 100 + smem_sm - 1) / smem_sm);
+      if (carve > 100) carve = 100;
+    }
+    const void* const* blind_variants = a1_blind_variants();
+    for (int v = 0; v < A1_BLIND_VARIANTS && e == cudaSuccess; ++v) {
+      e = cudaFuncSetAttribute(blind_variants[v], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(VBSmem));
+      if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(blind_variants[v], cudaFuncAttributePreferredSharedMemoryCarveout, carve);
+    }
+    int bocc = 0;
+    if (e == cudaSuccess)
+      e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bocc, a1_post_physics_blind_kernel<false, false, false>, VB_THREADS,
+                                                        sizeof(VBSmem));
+    c->blind_occ = bocc;
     const char* kern = getenv("SHIFU_A1_KERNEL");
     c->use_tma = !(kern != nullptr && strcmp(kern, "phased") == 0);
   }
@@ -492,7 +527,9 @@ extern "C" int shifu_a1_eval_terms(ShifuCtx* c, const ShifuA1StepIO* io, float* 
 extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void* stream) {
   REQUIRE_PTR(c); REQUIRE_PTR(io);
   if (!c->is_a1) return fail(SHIFU_E_STATE, "shifu_a1_post_physics needs an A1 ctx");
-  if (c->d_table == nullptr) return fail(SHIFU_E_STATE, "call shifu_set_height_map first");
+  if (!c->blind && c->d_table == nullptr) return fail(SHIFU_E_STATE, "call shifu_set_height_map first");
+  if (c->blind && io->measured_heights != nullptr)
+    return fail(SHIFU_E_RANGE, "measured_heights must be NULL with num_obs = %d (no height scan)", A1_HEAD);
   REQUIRE_PTR(io->root_state); REQUIRE_PTR(io->dof_state); REQUIRE_PTR(io->contact_state);
   REQUIRE_PTR(io->actions); REQUIRE_PTR(io->torques); REQUIRE_PTR(io->history); REQUIRE_PTR(io->command);
   REQUIRE_PTR(io->ep_len); REQUIRE_PTR(io->base_lin_vel); REQUIRE_PTR(io->base_ang_vel);
@@ -511,13 +548,22 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
   // tail (< 32 envs) or everything when bulk copies are not possible.
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
   // the pipelined scan rotates once per point pair: it needs the point-symmetric grid (else: phased kernel)
-  const bool can_tma = c->use_tma && c->grid_symmetric && c->a1k.root_stride == 1 && c->a1k.root_offset == 0 && al16(io->root_state) &&
+  const bool can_tma = c->use_tma && (c->grid_symmetric || c->blind) && c->a1k.root_stride == 1 && c->a1k.root_offset == 0 && al16(io->root_state) &&
                        al16(io->dof_state) && al16(io->contact_state) && al16(io->history) && al16(io->torques) &&
                        al16(io->actions) && al16(io->obs_buf) && al16(io->ep_len) && al16(io->command) &&
                        al16(io->base_lin_vel) && al16(io->base_ang_vel) && al16(io->projected_gravity) &&
                        [&] { for (int q = 0; q < c->a1k.n_terms; ++q) if (!al16(io->ep_sums[q])) return false; return true; }();
   const int full_tiles = can_tma ? n / A1_TILE : 0;
-  if (full_tiles > 0) {
+  if (full_tiles > 0 && c->blind) {
+    const int cap = c->sm_count * (c->blind_occ > 0 ? c->blind_occ : 1);
+    const dim3 grid(full_tiles < cap ? full_tiles : cap), block(VB_THREADS);
+    bool extra = false;
+    for (int q = 0; q < c->a1k.n_terms; ++q) extra |= c->a1k.terms[q] >= SHIFU_REW_LIN_VEL_Z;
+    int tiles_arg = full_tiles;
+    void* args[4] = {(void*)&c->a1k, const_cast<ShifuA1StepIO*>(io), (void*)&tiles_arg, (void*)&c->a1o};
+    const int variant = (c->obs_custom ? 2 : 0) + (c->a1o.noisy ? 2 : 0) + (extra ? 1 : 0);
+    CUDA_TRY(cudaLaunchKernel(a1_blind_variants()[variant], grid, block, args, sizeof(VBSmem), S(stream)));
+  } else if (full_tiles > 0) {
     const int cap = c->sm_count * (c->tma_occ > 0 ? c->tma_occ : 1);
     const dim3 grid(full_tiles < cap ? full_tiles : cap), block(V3_THREADS);
     const size_t smem = sizeof(V3Smem);
@@ -535,12 +581,15 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     const dim3 grid(tiles < cap ? tiles : cap), block(A1_THREADS);
     const A1K& k = c->a1k;
     const A1Obs& o = c->a1o;
-    if (o.noisy) {
-      if (exact) a1_post_physics_kernel<true, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
-      else a1_post_physics_kernel<false, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+    if (c->blind) {
+      if (o.noisy) a1_post_physics_kernel<false, true, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      else a1_post_physics_kernel<false, false, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+    } else if (o.noisy) {
+      if (exact) a1_post_physics_kernel<true, true, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      else a1_post_physics_kernel<false, true, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
     } else {
-      if (exact) a1_post_physics_kernel<true, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
-      else a1_post_physics_kernel<false, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      if (exact) a1_post_physics_kernel<true, false, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      else a1_post_physics_kernel<false, false, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
     }
     CUDA_TRY(cudaGetLastError());
   }

@@ -112,12 +112,20 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
     if not isinstance(isg, TerrainGymEnv) or not isinstance(rb, LeggedRobot):
         raise NotFusable("needs a TerrainGymEnv with a LeggedRobot")
     tc = cfg.terrain
-    if (len(tc.measured_points_x), len(tc.measured_points_y)) != (nv.MAX_PX, nv.MAX_PY) or not tc.measure_heights:
+    # the observation width picks the step: 72 + 187 scans the terrain, 72 is blind (no height columns)
+    num_obs = cfg.num_obs
+    if num_obs not in (nv.OBS_HEAD, nv.OBS_HEAD + nv.MAX_PX * nv.MAX_PY) or cfg.num_privileged_obs is not None:
+        raise NotFusable("observation width is not 72 + 187 or 72")
+    blind = num_obs == nv.OBS_HEAD
+    if not blind and ((len(tc.measured_points_x), len(tc.measured_points_y)) != (nv.MAX_PX, nv.MAX_PY)
+                      or not tc.measure_heights):
         raise NotFusable("the fused kernel is compiled for the 17x11 measured-point grid")
+    store_heights = bool(getattr(cfg, "store_measured_heights", False))
+    if blind and store_heights:
+        raise NotFusable("store_measured_heights with a 72-column observation: the fused blind step does not scan "
+                         "the terrain")
     if (rb.num_dof, rb.num_bodies, cfg.num_actions, cfg.num_actions_history) != (12, 17, 12, 3):
         raise NotFusable("the fused kernel is compiled for 12 dofs / 17 bodies / 3 past actions")
-    if cfg.num_obs != 72 + nv.MAX_PX * nv.MAX_PY or cfg.num_privileged_obs is not None:
-        raise NotFusable("observation width is not 72 + 187")
     layout = rb.affine_root_layout()
     if layout is None:
         raise NotFusable("non-affine root_indices")
@@ -162,13 +170,13 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
     # ---- observation: slot sources, scales and noise scales ------------------------------------
     # (read once, here, like every fitted constant: a noise curriculum that changes noise_scale_vec
     # later does not reach the kernel)
-    obs = terms.compile_a1_obs(env)
+    obs = terms.compile_a1_obs(env, num_obs)
     # ---- the hot path over the env's own tensors -----------------------------------------------
     desc = a1_env_desc(env, [(t.name, t.code, t.p0, t.p1) for t in compiled], rng_seed=rng_seed, obs=obs,
                        action_scale=1.0,         # a subclass step() has already scaled (a1_conditional.py:122-124)
                        force_body=force_body, push_force_max=float(forces[0]), air_time_reset=air_time_reset,
-                       **terms.desc_extras(compiled))
-    hp = a1_hot_path(env, desc, names, carry_body_frame, bool(getattr(cfg, "store_measured_heights", False)))
+                       num_obs=num_obs, **terms.desc_extras(compiled))
+    hp = a1_hot_path(env, desc, names, carry_body_frame, store_heights)
     # the probes below run the user's hooks on the env's CURRENT tensors: point the hot path at them
     hp.adopt(actions=env.actions, history=env.actions_recorder.history_buf, command=env.command_buf,
              torques=rb.torques, base_lin_vel=rb.base_lin_vel, base_ang_vel=rb.base_ang_vel,
@@ -179,7 +187,7 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
         hp.adopt(swing_time=air[0], last_contacts=air[1])
     # ---- numerical checks ----------------------------------------------------------------------
     terms.verify_a1_terms(env, hp, env.reward_functions, compiled)
-    terms.verify_a1_obs(env, obs)
+    terms.verify_a1_obs(env, obs, num_obs=num_obs)
     _check_a1_termination(env)
     return hp
 
@@ -209,15 +217,19 @@ def a1_env_desc(env, terms, *, rng_seed: int, force_body: int, push_force_max: f
     """``hotpath.a1_desc`` of an A1-shaped env: dof gains and limits from its robot, the point grid and
     terrain scales from its config, curriculum, levels and env length from its gym env, and its episode
     lengths, clips and command ranges.  ``terms`` and ``kw`` (``obs``, ``action_scale``, ``air_time_reset``,
-    the compiled terms' extras) go to ``a1_desc`` as they are."""
+    the compiled terms' extras) go to ``a1_desc`` as they are; ``num_obs`` defaults to the config's.  A blind
+    descriptor (``num_obs = 72``) keeps the compiled 17x11 grid whatever the config's: the blind step does not
+    scan, and the on-demand heights come from the gym env's own scan."""
     rb, isg, tc = env.robot, env.isg_env, env.cfg.terrain
     stride, offset = rb.affine_root_layout()
+    kw.setdefault("num_obs", env.cfg.num_obs)
+    grid = {} if kw["num_obs"] == nv.OBS_HEAD else dict(points_x=tuple(tc.measured_points_x),
+                                                         points_y=tuple(tc.measured_points_y))
     desc = hotpath.a1_desc(
         env.num_envs, env_offset=env.env_offset, rng_seed=rng_seed, terms=terms,
         q0=tuple(rb.cfg.default_dof_pos), kp=tuple(float(v) for v in rb.p_gains.tolist()),
         kd=tuple(float(v) for v in rb.d_gains.tolist()), torque_limit=tuple(rb.torque_limits.tolist()),
-        points_x=tuple(tc.measured_points_x), points_y=tuple(tc.measured_points_y),
-        border_size=float(tc.border_size), horizontal_scale=tc.horizontal_scale, vertical_scale=tc.vertical_scale,
+        **grid, border_size=float(tc.border_size), horizontal_scale=tc.horizontal_scale, vertical_scale=tc.vertical_scale,
         max_episode_length=int(env.max_episode_length), max_episode_length_s=float(env.max_episode_length_s),
         default_root=tuple(rb.cfg.default_pos) + tuple(rb.cfg.default_quat), curriculum=tc.curriculum,
         max_terrain_level=isg.max_terrain_level, num_terrain_types=tc.num_cols, env_length=isg.terrain.env_length,
@@ -232,10 +244,11 @@ def a1_env_desc(env, terms, *, rng_seed: int, force_body: int, push_force_max: f
 
 
 def a1_hot_path(env, desc: nv.A1Desc, names, carry_body_frame: bool, want_measured_heights: bool) -> hotpath.A1HotPath:
-    """An ``A1HotPath`` for ``desc`` over the env's gym tensors."""
+    """An ``A1HotPath`` for ``desc`` over the env's gym tensors (a blind descriptor takes no height map)."""
     isg = env.isg_env
+    blind = desc.num_obs == nv.OBS_HEAD
     return hotpath.A1HotPath(desc, root_state=isg.root_state, dof_state=isg.dof_state, contact_state=isg.contact_state,
-                             height_samples=isg.height_samples, terrain_origins=isg.terrain_origins,
+                             height_samples=None if blind else isg.height_samples, terrain_origins=isg.terrain_origins,
                              terrain_types=isg.terrain_types, env_origins=isg.env_origins, terms=names,
                              carry_body_frame=carry_body_frame, want_measured_heights=want_measured_heights)
 
@@ -254,7 +267,9 @@ def bind_a1(env, hp):
     rb.base_lin_vel, rb.base_ang_vel = hp.base_lin_vel, hp.base_ang_vel
     rb.projected_gravity, rb.gravity_vec = hp.projected_gravity, hp.gravity_vec
     isg.measured_heights = hp.measured_heights          # None unless cfg.store_measured_heights: filled on demand
-    isg.__dict__["_heights_on_demand"] = hp.measured_heights is None
+    # (a blind task fills it on demand only when it measures heights, like user-hook mode does)
+    isg.__dict__["_heights_on_demand"] = hp.measured_heights is None and (not hp.blind or
+                                                                          bool(env.cfg.terrain.measure_heights))
     env.extras.update(hp.extras())
     hp.body_frame()
 

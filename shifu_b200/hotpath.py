@@ -133,13 +133,20 @@ def a1_desc(num_envs: int, *, env_offset: int = 0, rng_seed: int = 0x5EED,
             leg_bodies=(2, 3, 6, 7, 10, 11, 14, 15), force_body=0, root_stride=1, root_offset=0,
             action_scale=0.5, clip_actions=1., clip_obs=100.,
             dof_pos_limits=None, feet_bodies=(4, 8, 12, 16), feet_contact_force=1.0, air_time_cmd_min=0.1,
-            air_time_dt=0.02, air_time_reset=True, obs: Optional[ObsLayout] = None) -> nv.A1Desc:
+            air_time_dt=0.02, air_time_reset=True, obs: Optional[ObsLayout] = None,
+            num_obs: int = nv.OBS_HEAD + 187) -> nv.A1Desc:
     """Defaults = the constants of ``examples/a1_conditional`` (SURVEY.md Appendix A).  ``obs``: the
-    observation layout; ``None`` or the reference layout writes ``obs_layout = 0``."""
+    observation layout; ``None`` or the reference layout writes ``obs_layout = 0``.  ``num_obs``: 259, or
+    72 for a blind task (the observation without its 187 height columns; ``obs.height_noise`` must be 0)."""
+    if num_obs not in (nv.OBS_HEAD, nv.OBS_HEAD + 187):
+        raise ValueError(f"num_obs={num_obs}: the fused A1 observation has {nv.OBS_HEAD + 187} columns, or "
+                         f"{nv.OBS_HEAD} without the height scan")
+    if num_obs == nv.OBS_HEAD and obs is not None and obs.height_noise != 0.0:
+        raise ValueError("a blind observation (num_obs = 72) has no height columns to add height noise to")
     d = nv.A1Desc()
     d.abi_version = nv.ABI_VERSION
     d.num_envs, d.env_offset, d.rng_seed = num_envs, env_offset, rng_seed
-    d.num_dof, d.num_bodies, d.num_hist, d.num_obs = 12, 17, 3, 259
+    d.num_dof, d.num_bodies, d.num_hist, d.num_obs = 12, 17, 3, num_obs
     d.base_body, d.force_body = base_body, force_body
     d.num_leg_bodies = len(leg_bodies)
     for i, b in enumerate(leg_bodies):
@@ -416,7 +423,11 @@ class HeightScan:
 
 
 class A1HotPath(_StepStats):
-    """Fused A1 step. ``root_state`` / ``dof_state`` / ``contact_state`` are the gym's flat tensors."""
+    """Fused A1 step. ``root_state`` / ``dof_state`` / ``contact_state`` are the gym's flat tensors.
+
+    A blind descriptor (``num_obs = 72``) builds the (N, 72) observation without the height scan: it takes
+    ``height_samples=None`` and keeps no ``measured_heights``.  A height map, when given, is uploaded for
+    ``get_heights(out=...)``, which then needs its own output tensor."""
 
     def __init__(self, desc: nv.A1Desc, *, root_state, dof_state, contact_state, height_samples,
                  terrain_origins, terrain_types, env_origins, terms: Sequence[str] = A1_DEFAULT_TERMS,
@@ -426,14 +437,19 @@ class A1HotPath(_StepStats):
         self.desc = desc
         self.n = n = desc.num_envs
         self.terms = list(terms)
+        self.blind = desc.num_obs == nv.OBS_HEAD
+        if self.blind and want_measured_heights:
+            raise ValueError("a blind A1 step (num_obs = 72) does not scan: it cannot store measured_heights")
+        if height_samples is None and not self.blind:
+            raise ValueError("the 259-column A1 step scans the height map: height_samples is required")
         self.ctx = _Ctx(dev, a1=desc)
         self.lib = self.ctx.lib
         f = dict(device=dev, dtype=torch.float)
         # borrowed simulator tensors
         self.root_state, self.dof_state, self.contact_state = root_state, dof_state, contact_state
         # terrain (isaac_gym.py:336-347)
-        self.height_samples = height_samples.to(dev).contiguous()
-        assert self.height_samples.dtype == torch.int16
+        self.height_samples = height_samples.to(dev).contiguous() if height_samples is not None else None
+        assert self.height_samples is None or self.height_samples.dtype == torch.int16
         self.terrain_origins = terrain_origins.to(**f).contiguous()
         self.terrain_types = terrain_types.to(dev, torch.long).contiguous()
         self.env_origins = env_origins            # (N,3) fp32, shared with the gym façade
@@ -451,7 +467,7 @@ class A1HotPath(_StepStats):
         self.terrain_levels = torch.zeros(n, device=dev, dtype=torch.long)
         self.dof_targets = torch.zeros(n, 12, **f)
         self.rand_force = torch.zeros(n, 17, 3, **f)
-        self.obs_buf = torch.zeros(n, 259, **f)
+        self.obs_buf = torch.zeros(n, desc.num_obs, **f)
         self.rew_buf = torch.zeros(n, **f)
         self.reset_buf = torch.ones(n, device=dev, dtype=torch.bool)
         self.time_out_buf = torch.zeros(n, device=dev, dtype=torch.bool)
@@ -470,9 +486,10 @@ class A1HotPath(_StepStats):
         self._fork = None
         self.carry_body_frame = carry_body_frame
         self._io = None
-        nv.check(self.lib.shifu_set_height_map(self.ctx.handle, nv.ptr(self.height_samples),
-                                               self.height_samples.shape[0], self.height_samples.shape[1],
-                                               nv.current_stream()))
+        if self.height_samples is not None:
+            nv.check(self.lib.shifu_set_height_map(self.ctx.handle, nv.ptr(self.height_samples),
+                                                   self.height_samples.shape[0], self.height_samples.shape[1],
+                                                   nv.current_stream()))
         self.sync_level_sum()
 
     # ------------------------------------------------------------------

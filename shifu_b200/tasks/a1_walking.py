@@ -168,12 +168,16 @@ class A1Conditional(ShifuVecEnv):
             raise NotImplementedError("the fused A1 kernel needs affine root_indices")
         names = [fn.__name__ for fn in self.reward_functions]
         obs = None
-        if type(self).compute_observations is not A1Conditional.compute_observations:
+        num_obs = self.cfg.num_obs                  # 72 + 187, or 72 for a blind subclass
+        if num_obs == 72 and self._store_heights:
+            raise NotImplementedError("store_measured_heights with a 72-column observation: the fused blind step "
+                                      "does not scan the terrain (fused=False measures and keeps the heights)")
+        if type(self).compute_observations is not A1Conditional.compute_observations or num_obs != 259:
             # an edited observation hook: fused only when the kernel's observation layout expresses it,
             # never silently replaced by the reference observation
             try:
-                obs = terms.compile_a1_obs(self)
-                terms.verify_a1_obs(self, obs)
+                obs = terms.compile_a1_obs(self, num_obs)
+                terms.verify_a1_obs(self, obs, num_obs=num_obs)
             except terms.NotFusable as exc:
                 raise NotImplementedError(f"{exc} (fused=False runs any observation hook)") from exc
         # reference constants: the named terms' (hotpath.A1_TERM_PARAMS) and the push force

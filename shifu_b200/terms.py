@@ -362,12 +362,54 @@ def _exact_offset(q0: float) -> float:
     raise NotFusable(f"compute_observations: no exact dof-position probe around {q0}")
 
 
+class _NoHeights:
+    """Stands in for ``measured_heights`` while a blind (72-column) observation hook runs: the fused blind
+    step does not scan the terrain, so any use of the heights refuses the hook."""
+    REASON = ("compute_observations: the 72-column (blind) observation reads measured_heights; the fused blind "
+              "step does not scan the terrain")
+
+    def __init__(self):
+        self.touched = False
+
+    def _refuse(self, *args, **kwargs):
+        object.__setattr__(self, "touched", True)
+        raise NotFusable(self.REASON)
+
+    @classmethod
+    def __torch_function__(cls, func, types, args=(), kwargs=None):
+        for a in (*args, *(kwargs or {}).values()):
+            if isinstance(a, _NoHeights):
+                a._refuse()
+        raise NotFusable(cls.REASON)
+
+    def __getattr__(self, name):
+        self._refuse()
+
+    __getitem__ = __len__ = __iter__ = __array__ = _refuse
+    __add__ = __radd__ = __sub__ = __rsub__ = __mul__ = __rmul__ = __truediv__ = __rtruediv__ = __neg__ = _refuse
+
+
+def _blind_hook(env, heights):
+    """Runs ``compute_observations`` with ``heights`` (a ``_NoHeights``) as the measured heights; an error
+    the heights caused becomes NotFusable with the reason."""
+    env.isg_env.measured_heights = heights
+    try:
+        env.compute_observations()
+    except NotFusable:
+        raise
+    except Exception as exc:
+        if heights.touched:
+            raise NotFusable(_NoHeights.REASON) from exc
+        raise
+
+
 @contextmanager
-def _obs_draws(env, u):
+def _obs_draws(env, u, width: Optional[int] = None):
     """While ``compute_observations`` runs: ``torch.rand_like`` of the whole observation returns ``u`` (a
     number or a tensor of that shape), once per call; any other draw raises NotFusable.  legged_gym's noise
-    is ``obs_buf += (2 * torch.rand_like(obs_buf) - 1) * noise_scale_vec``, which the fused kernel adds."""
-    shape = (env.num_envs, nv.OBS_HEAD + env.isg_env.num_height_points)
+    is ``obs_buf += (2 * torch.rand_like(obs_buf) - 1) * noise_scale_vec``, which the fused kernel adds.
+    ``width``: the observation's columns (default 72 + the height points)."""
+    shape = (env.num_envs, width if width is not None else nv.OBS_HEAD + env.isg_env.num_height_points)
     calls = []
 
     def rand_like(t, *args, **kwargs):
@@ -400,7 +442,7 @@ def _obs_draws(env, u):
             setattr(torch, name, fn)
 
 
-def compile_a1_obs(env) -> ObsLayout:
+def compile_a1_obs(env, num_obs: Optional[int] = None) -> ObsLayout:
     """``env.compute_observations`` -> ObsLayout, by probing.  At the zero state (every input zero,
     dof_pos = default_dof_pos, base 0.5 above flat terrain) the observation must be all zeros; then each
     input is set alone to a power of two and must reach exactly one column of its block, the three
@@ -409,9 +451,15 @@ def compile_a1_obs(env) -> ObsLayout:
     Every probe so far runs with ``torch.rand_like`` at u = 0.5, where uniform noise vanishes.  Then, at the
     zero state, u = 1 gives each column's noise scale and u = 0 must give its negative; the heights share
     one scale, added after their clip and scale (probed at z - 0.5 - h = 3).
+    A hook that returns (N, 72) is blind: the same head probes run with the measured heights replaced by
+    a stand-in whose every use refuses the hook, and there are no height probes (the layout keeps height
+    scale 1 and no height noise).  ``num_obs``: the width the hook must return (default: 72 + the height
+    points, or 72 when the hook returns 72 columns).
     Anything else raises NotFusable naming the column and the reason."""
     rb, isg = env.robot, env.isg_env
     n_head = nv.OBS_HEAD
+    if num_obs is not None and num_obs not in (n_head, n_head + isg.num_height_points):
+        raise NotFusable(f"observation width {num_obs} is neither {n_head} nor {n_head + isg.num_height_points}")
     had = isg.__dict__.get("_measured_heights")
     with A1Probe(env) as pr:
         t = pr.tensors
@@ -426,14 +474,26 @@ def compile_a1_obs(env) -> ObsLayout:
             t["root"][rb.root_indices, 2] = 0.5
             heights.zero_()
 
-        def observe(u=0.5):
+        width = num_obs
+        if width is None:                           # the hook's own width: 72 (blind) or 72 + the heights
+            zero_state()
             isg.measured_heights = heights
-            with _obs_draws(env, u):
+            with _obs_draws(env, 0.5, env.obs_buf.shape[1]):
                 env.compute_observations()
+            width = n_head if tuple(env.obs_buf.shape) == (env.num_envs, n_head) else n_head + heights.shape[1]
+        blind = width == n_head
+
+        def observe(u=0.5):
+            with _obs_draws(env, u, width):
+                if blind:
+                    _blind_hook(env, _NoHeights())
+                else:
+                    isg.measured_heights = heights
+                    env.compute_observations()
             obs = env.obs_buf
-            if tuple(obs.shape) != (env.num_envs, n_head + heights.shape[1]):
+            if tuple(obs.shape) != (env.num_envs, width):
                 raise NotFusable(f"compute_observations: shape {tuple(obs.shape)}, the fused observation is "
-                                 f"({env.num_envs}, {n_head + heights.shape[1]})")
+                                 f"({env.num_envs}, {width})")
             return obs[0].float().cpu()
 
         def lit(o, lo=0, hi=n_head):
@@ -494,6 +554,16 @@ def compile_a1_obs(env) -> ObsLayout:
                     raise NotFusable(f"compute_observations: {label} reaches columns {[j for j, _ in hits]}; the "
                                      f"fused observation has it in column {col} alone")
                 scales[col] = hits[0][1] / x
+            if blind:                                       # no height columns: no height probes
+                zero_state()
+                up, down = observe(1.0), observe(0.0)
+                bad = torch.nonzero(down != -up).flatten().tolist()
+                if bad:
+                    j = bad[0]
+                    raise NotFusable(f"compute_observations: column {j} is {float(up[j]):g} at u = 1 and "
+                                     f"{float(down[j]):g} at u = 0 with every input at zero; the fused noise is "
+                                     "(2u - 1) * scale with u = torch.rand_like(obs_buf)")
+                return ObsLayout(tuple(slots), tuple(scales), 1.0, tuple(float(v) for v in up), 0.0)
             # heights: clip(z - 0.5 - h, +-1) * height_scale
             zero_state()
             heights[0] = -0.5
@@ -547,14 +617,19 @@ def compile_a1_obs(env) -> ObsLayout:
     return ObsLayout(tuple(slots), tuple(scales), hs, noise, hn)
 
 
-def a1_obs_definition(env, layout: ObsLayout, u: Optional[torch.Tensor] = None) -> torch.Tensor:
+def a1_obs_definition(env, layout: ObsLayout, u: Optional[torch.Tensor] = None, blind: bool = False) -> torch.Tensor:
     """The observation the fused kernel builds under ``layout``, in torch on the env's tensors (before the
-    final clip to +-clip_obs that the base class applies).  ``u``: the noise draws, (num_envs, 259)."""
+    final clip to +-clip_obs that the base class applies).  ``u``: the noise draws, (num_envs, 259), or
+    (num_envs, 72) when ``blind`` (the 72 head columns alone)."""
     rb, isg = env.robot, env.isg_env
     src = {name: getattr(rb if key != "command" else env, label) for name, (key, label) in _OBS_PROBE.items()}
     head = torch.cat([src[name] for name in layout.slots]
                      + [rb.dof_pos - rb.default_dof_pos, rb.dof_vel, env.actions_recorder.flatten()], dim=1)
     head = head * torch.tensor(layout.scales, dtype=torch.float, device=head.device)
+    if blind:
+        if u is not None and layout.has_noise():
+            head = head + (2 * u - 1) * torch.tensor(layout.noise, dtype=torch.float, device=head.device)
+        return head
     heights = torch.clip(rb.base_pose[:, 2].unsqueeze(1) - 0.5 - isg.measured_heights, -1, 1.) * layout.height_scale
     obs = torch.cat([head, heights], dim=1)
     if u is not None and layout.has_noise():
@@ -564,20 +639,27 @@ def a1_obs_definition(env, layout: ObsLayout, u: Optional[torch.Tensor] = None) 
     return obs
 
 
-def verify_a1_obs(env, layout: ObsLayout, seed: int = 4321):
+def verify_a1_obs(env, layout: ObsLayout, seed: int = 4321, num_obs: Optional[int] = None):
     """``env.compute_observations`` against the layout's definition (noise included) on a seeded random
-    state, with the same seeded draws given to the hook's ``torch.rand_like`` and to the definition."""
+    state, with the same seeded draws given to the hook's ``torch.rand_like`` and to the definition.
+    ``num_obs = 72``: the blind observation, with the heights replaced by a stand-in that refuses any use."""
     isg = env.isg_env
+    blind = num_obs == nv.OBS_HEAD
+    width = nv.OBS_HEAD + (0 if blind else isg.num_height_points)
     had = isg.__dict__.get("_measured_heights")
     with A1Probe(env) as pr:
         pr.randomize(seed)
         g = torch.Generator(device=env.device).manual_seed(seed)
-        isg.measured_heights = torch.randn(env.num_envs, isg.num_height_points, generator=g, device=env.device)
-        u = torch.rand(env.num_envs, nv.OBS_HEAD + isg.num_height_points, generator=g, device=env.device)
+        heights = torch.randn(env.num_envs, isg.num_height_points, generator=g, device=env.device)
+        u = torch.rand(env.num_envs, width, generator=g, device=env.device)
         try:
-            with _obs_draws(env, u):
-                env.compute_observations()
-            check_close(env.obs_buf, a1_obs_definition(env, layout, u), "compute_observations")
+            with _obs_draws(env, u, width):
+                if blind:
+                    _blind_hook(env, _NoHeights())
+                else:
+                    isg.measured_heights = heights
+                    env.compute_observations()
+            check_close(env.obs_buf, a1_obs_definition(env, layout, u, blind), "compute_observations")
         finally:
             if had is None:
                 del isg.measured_heights
