@@ -38,6 +38,8 @@ extern "C" {
 #define SHIFU_MAX_REWARD_TERMS 8
 #define SHIFU_NUM_STATS 16
 #define SHIFU_OBS_HEAD 72       /* observation columns before the 187 heights */
+#define SHIFU_OBS_HEAD_ACT 48   /* the action head (num_obs = 235 or 48): columns 0-35 as in the 72-column head,
+                                   then column 36 + d = the step's actions[d] (legged_gym's observation) */
 
 /* Philox stream of the observation noise (ShifuA1Desc.obs_noise / obs_height_noise).  Counter
  * (global env id, step, SHIFU_STREAM_OBS_NOISE, word), key rng_seed, u = (x >> 8) * 2^-24 like every other
@@ -53,7 +55,12 @@ extern "C" {
  * words.  The two lanes of height point pairs k, k^1 each evaluate word 18 + (k >> 1) for one env of an env
  * pair and swap halves, so every lane of those evaluations is used; the two idle scan lanes evaluate word 64
  * for nothing.
- * A 72-column (blind, num_obs = SHIFU_OBS_HEAD) observation draws words 0-17 only, with the same map. */
+ * A 72-column (blind, num_obs = SHIFU_OBS_HEAD) observation draws words 0-17 only, with the same map.
+ * The action head (num_obs = 235 or 48, head width SHIFU_OBS_HEAD_ACT) keeps every position: head column
+ * d + 12m (m < 4) uses the word and lane it has in the 72-column map (so the action column 36 + d uses the
+ * word and lane of history column 36 + d), words 3i + 2 are not drawn, and height point k (column 48 + k)
+ * uses word 18 + ... exactly as above.  The 235-column observation draws 12 + 47 = 59 words (0, 1, 3, 4, ...,
+ * 15, 16 and 18-64), the 48-column one 12. */
 #define SHIFU_STREAM_OBS_NOISE 8
 
 enum {
@@ -133,7 +140,12 @@ typedef struct ShifuA1Desc {
   int32_t num_obs;              /* 259, or SHIFU_OBS_HEAD (72) for a blind task: obs_buf is (N,72), the
                                    measured heights are neither scanned nor written (measured_heights must be
                                    NULL), obs_height_scale is not read, obs_height_noise must be 0, and
-                                   shifu_a1_post_physics needs no shifu_set_height_map */
+                                   shifu_a1_post_physics needs no shifu_set_height_map.
+                                   235 (SHIFU_OBS_HEAD_ACT + 187) or 48: the action head (legged_gym's
+                                   observation), which needs obs_layout = 1; obs_scale[j] and obs_noise[j]
+                                   are read for j < 48 only, column 36 + d is clip(actions[d] * obs_scale[36 + d]
+                                   [+ noise], +-clip_obs), and the heights follow at column 48.  48 is blind
+                                   like 72.  Anything else: SHIFU_E_RANGE */
   int32_t base_body;            /* contact_terminate_indices, a1_conditional.py:98-99 */
   int32_t num_leg_bodies;       /* 8 */
   int32_t leg_bodies[SHIFU_MAX_LEG_BODIES]; /* a1_conditional.py:59-61 */
@@ -221,7 +233,7 @@ typedef struct ShifuA1StepIO {
   uint8_t* reset_buf;             /* w (N) bool */
   uint8_t* time_out_buf;          /* w (N) bool */
   uint8_t* contact_term_buf;      /* w (N) bool */
-  float* measured_heights;        /* optional w (N,187), may be NULL; must be NULL when num_obs = 72 */
+  float* measured_heights;        /* optional w (N,187), may be NULL; must be NULL when num_obs = 72 or 48 */
   int64_t step;                   /* common_step_counter AFTER its increment (env.py:96): Philox counter */
   const int64_t* step_dev;        /* optional: when non-NULL the step is read from this device word
                                      instead (lets a captured CUDA graph replay with a moving

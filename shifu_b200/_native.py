@@ -14,6 +14,7 @@ from typing import Optional
 MAX_DOF, MAX_LEG, MAX_PX, MAX_PY, MAX_TERMS, NUM_STATS = 12, 8, 17, 11, 8, 16
 ABI_VERSION = 5
 OBS_HEAD = 72
+OBS_HEAD_ACT = 48          # the action head (num_obs = 235 or 48): SHIFU_OBS_HEAD_ACT
 
 # enum ShifuRewardTerm
 REW_TRACKING_LIN_VEL, REW_TRACKING_ANG_VEL, REW_STABILIZING_BASE, REW_SMOOTHING_ACTION = 0, 1, 2, 3

@@ -21,7 +21,7 @@ INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
 LIB_PATH = os.path.join(PKG_DIR, "libshifu_b200.so")
 
 SOURCES = ["capi.cu"]
-DEPS = ["capi.cu", "a1_kernels.cuh", "a1_fused.cuh", "a1_fused_tma.cuh", "tma_pipe.cuh", "f32x2.cuh","abb_kernels.cuh", "arm_ik.cuh", "camera_gather.cuh", "common_kernels.cuh", "exact_math.cuh", "philox.cuh", "terrain_gen.cuh", "scan_pairs.cuh"]
+DEPS = ["capi.cu", "a1_kernels.cuh", "a1_fused.cuh", "a1_fused_tma.cuh", "a1_fused_kernel.inc", "a1_fused_tma_kernel.inc", "tma_pipe.cuh", "f32x2.cuh","abb_kernels.cuh", "arm_ik.cuh", "camera_gather.cuh", "common_kernels.cuh", "exact_math.cuh", "philox.cuh", "terrain_gen.cuh", "scan_pairs.cuh"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -226,180 +226,21 @@ __device__ __noinline__ float a1_eval_term(int q, const A1K& k, const A1Smem& s,
 // column; a compile-time flag, so that the noiseless instantiations keep their registers and code.
 // The kernel starts at tile first_tile (the tiles before it are the pipelined kernel's); env indices
 // stay absolute, so k and io describe all k.n envs.
-// BLIND: the 72-column observation without the height scan (no phase C, obs rows of A1_HEAD floats);
-// EXACT_DIV does not apply.
-template <bool EXACT_DIV, bool NOISE, bool BLIND>
-__global__ void __launch_bounds__(A1_THREADS, 5)
-a1_post_physics_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io,
-                       const __grid_constant__ A1Obs o, int first_tile) {
-  __shared__ __align__(16) A1Smem s;
-  // projected gravity at the start of the step: warp 5 overwrites io.projected_gravity in phase B3
-  // (carry_body_frame) while the other threads build the head
-  __shared__ float pg0[A1_TILE][3];
-  const int t = threadIdx.x, warp = t >> 5, lane = t & 31;
-  const long long step = (io.step_dev != nullptr) ? *io.step_dev : io.step;
-  constexpr int OW = BLIND ? A1_HEAD : A1_OBS;     // obs row stride
-  // scan point owned by this thread (threads 187..191 idle in phase C)
-  const float bx = k.px[t % A1_NX], by = k.py[(t / A1_NX) % A1_NY];
+// BLIND: the head without the height scan (no phase C, obs rows of HEAD floats); EXACT_DIV does not apply.
+// HEAD: the head width, A1_HEAD or A1_HEAD_ACT (the action head, a1_post_physics_kernel_act: columns 36 + d
+// are the step's actions in place of the three history slots; heights at HEAD + point).
+#define A1_PHASED_KERNEL a1_post_physics_kernel
+#define A1_PHASED_HEAD A1_HEAD
+#include "a1_fused_kernel.inc"
+#undef A1_PHASED_KERNEL
+#undef A1_PHASED_HEAD
 
-  for (int e0 = (first_tile + blockIdx.x) * A1_TILE; e0 < k.n; e0 += gridDim.x * A1_TILE) {
-    const int ne = min(A1_TILE, k.n - e0);
-    const int ge = e0 + lane;                      // env of this lane in the lane = env phases
-    const bool lane_env = (lane < ne);
-
-    // ---- phase A -------------------------------------------------------------------------
-    long long len = 0;
-    float esum[SHIFU_MAX_REWARD_TERMS];
-    float c9[9];
-    if (warp == 0 && lane_env) {       // issued first, consumed after the tile loads are in flight
-      len = io.ep_len[ge];
-#pragma unroll
-      for (int j = 0; j < 3; ++j) {
-        c9[j] = io.command[ge * 3LL + j];
-        c9[3 + j] = io.base_lin_vel[ge * 3LL + j];
-        c9[6 + j] = io.base_ang_vel[ge * 3LL + j];
-      }
-#pragma unroll
-      for (int j = 0; j < SHIFU_MAX_REWARD_TERMS; ++j) esum[j] = (j < k.n_terms) ? io.ep_sums[j][ge] : 0.0f;
-    }
-    a1_stage_rows(s, k, io, e0, ne, t);
-    if (o.uses_pg)
-      for (int i = t; i < ne * 3; i += A1_THREADS) (&pg0[0][0])[i] = io.projected_gravity[e0 * 3LL + i];
-    if (warp == 0 && lane_env) {
-#pragma unroll
-      for (int j = 0; j < 9; ++j) s.cla[j / 3][lane][j % 3] = c9[j];
-    }
-    __syncthreads();
-
-    // ---- phase B1: reward terms spread over the warps, lane = env ---------------------------
-    bool contact_term = false;
-    if (lane_env) {
-#pragma unroll 1
-      for (int j = warp; j < k.n_terms; j += A1_THREADS / 32) s.rterm[j][lane] = a1_eval_term(j, k, s, lane, io, ge);
-      if (warp == 0)                                                    // a1_conditional.py:146-148
-        contact_term = force_exceeds(&s.contact[lane][k.base_body * 3], k.contact_thr_sq);
-      if (!BLIND && warp == 5)    // heights are measured at the PRE-reset pose (isaac_gym.py:320-322 runs before post_step)
-        s.ev[lane] = make_scan_env(s.root[lane]);
-    }
-    __syncthreads();
-
-    // ---- phase B2: warp 0, lane = env ---------------------------------------------------------
-    if (warp == 0) {
-      bool reset = false;
-      double st_sum[SHIFU_MAX_REWARD_TERMS];
-#pragma unroll
-      for (int j = 0; j < SHIFU_MAX_REWARD_TERMS; ++j) st_sum[j] = 0.0;
-      long long level_delta = 0;
-      if (lane_env) {
-        len += 1;                                                          // env.py:95
-        const bool time_out = len > k.max_len;                             // a1_conditional.py:149
-        reset = contact_term | time_out;
-        float rew = 0.0f;                                                  // env.py:180-185
-#pragma unroll
-        for (int j = 0; j < SHIFU_MAX_REWARD_TERMS; ++j) {
-          if (j < k.n_terms) {
-            const float r = s.rterm[j][lane];
-            esum[j] = add_rn(esum[j], r);
-            rew = add_rn(rew, r);
-          }
-        }
-        io.rew_buf[ge] = rew;
-        io.reset_buf[ge] = reset ? 1 : 0;
-        io.time_out_buf[ge] = time_out ? 1 : 0;
-        io.contact_term_buf[ge] = contact_term ? 1 : 0;
-        if (reset) {                                                       // env.py:101-102
-          float cmd[3] = {s.cla[0][lane][0], s.cla[0][lane][1], s.cla[0][lane][2]};
-          a1_reset_env<true>(k, io, step, ge, s.root[lane], s.dof[lane], s.hist[lane], cmd, esum, len, st_sum,
-                             level_delta, io.env_origins[ge * 3LL + 0], io.env_origins[ge * 3LL + 1],
-                             io.env_origins[ge * 3LL + 2], k.curriculum ? io.terrain_levels[ge] : 0,
-                             k.curriculum ? io.terrain_types[ge] : 0);
-          s.cla[0][lane][0] = cmd[0]; s.cla[0][lane][1] = cmd[1]; s.cla[0][lane][2] = cmd[2];
-        }
-        io.ep_len[ge] = len;
-#pragma unroll
-        for (int j = 0; j < SHIFU_MAX_REWARD_TERMS; ++j)
-          if (j < k.n_terms) io.ep_sums[j][ge] = esum[j];
-        s.zb[lane] = sub_rn(s.root[lane][2], k.h_off);                     // post-reset base z (D8)
-      }
-      a1_log_sums(k, reset, st_sum, level_delta, lane);
-    }
-    __syncthreads();
-
-    // ---- phase B3: obs head (a1_conditional.py:131-144), history push (train.py:12-14) --------
-    {
-      const float c = k.clip_obs;
-      // + the column's noise before the clip to +-clip_obs
-      auto nz = [&](float x, int e, int j) {
-        return NOISE ? add_rn(x, obs_noise_at(o, k.seed, k.env_offset + e0 + e, step, j)) : x;
-      };
-      // (env, dof) items: dof columns and history columns (+ in-place push)
-      for (int i = t; i < ne * A1_DOF; i += A1_THREADS) {
-        const int e = i / A1_DOF, d = i - e * A1_DOF;
-        float* h = s.head[e];
-        h[12 + d] = clampf(nz(mul_rn(sub_rn(s.dof[e][2 * d], k.q0[d]), o.scale[12 + d]), e, 12 + d), -c, c);
-        h[24 + d] = clampf(nz(mul_rn(s.dof[e][2 * d + 1], o.scale[24 + d]), e, 24 + d), -c, c);
-        const float a0 = s.hist[e][d * A1_HIST + 0], a1 = s.hist[e][d * A1_HIST + 1],
-                    a2 = s.hist[e][d * A1_HIST + 2];
-        h[36 + d] = clampf(nz(mul_rn(a0, o.scale[36 + d]), e, 36 + d), -c, c);    // HistoryRecorder.flatten: slot-major
-        h[48 + d] = clampf(nz(mul_rn(a1, o.scale[48 + d]), e, 48 + d), -c, c);
-        h[60 + d] = clampf(nz(mul_rn(a2, o.scale[60 + d]), e, 60 + d), -c, c);
-        s.hist[e][d * A1_HIST + 2] = a1;               // HistoryRecorder.add
-        s.hist[e][d * A1_HIST + 1] = a0;
-        s.hist[e][d * A1_HIST + 0] = s.act[e][d];
-      }
-      // (env, j < 12): the four vector slots (reference: command, body-frame velocities, gravity_vec)
-      for (int i = t; i < ne * 12; i += A1_THREADS) {
-        const int e = i / 12, j = i - e * 12;
-        s.head[e][j] = clampf(nz(mul_rn(a1_obs_vec(o, j, s.cla, e, pg0[e][j % 3]), o.scale[j]), e, j), -c, c);
-      }
-      // carried body-frame velocities for the next control step (robot.py:222-229, D7)
-      if (io.carry_body_frame && warp == 5 && lane_env) {
-        const float* r = s.root[lane];
-        float o[3];
-        rotate_inverse(r + 3, r[7], r[8], r[9], o);
-        io.base_lin_vel[ge * 3LL + 0] = o[0]; io.base_lin_vel[ge * 3LL + 1] = o[1];
-        io.base_lin_vel[ge * 3LL + 2] = o[2];
-        rotate_inverse(r + 3, r[10], r[11], r[12], o);
-        io.base_ang_vel[ge * 3LL + 0] = o[0]; io.base_ang_vel[ge * 3LL + 1] = o[1];
-        io.base_ang_vel[ge * 3LL + 2] = o[2];
-        rotate_inverse(r + 3, 0.0f, 0.0f, -1.0f, o);
-        io.projected_gravity[ge * 3LL + 0] = o[0]; io.projected_gravity[ge * 3LL + 1] = o[1];
-        io.projected_gravity[ge * 3LL + 2] = o[2];
-      }
-    }
-    __syncthreads();
-
-    // ---- phase D: obs head + history tile ------------------------------------------------------
-    {
-      float* obase = io.obs_buf + (long long)e0 * OW;
-      const float* hsrc = &s.head[0][0];
-      for (int i = t; i < ne * A1_HEAD; i += A1_THREADS) {
-        const int e = i / A1_HEAD, j = i - e * A1_HEAD;
-        __stcs(obase + (long long)e * OW + j, hsrc[i]);
-      }
-      store_span(io.history + (long long)e0 * (A1_DOF * A1_HIST), &s.hist[0][0], ne * A1_DOF * A1_HIST, t,
-                 A1_THREADS);
-    }
-
-    // ---- phase C: 187-point scan; obs[., 72 + t] = clip(clip((z - 0.5) - h, +-1) * h_scale [+ noise], +-clip_obs)
-    if (!BLIND && t < A1_POINTS) {
-      float* orow = io.obs_buf + (long long)e0 * A1_OBS + A1_HEAD + t;
-      float* mrow = (io.measured_heights != nullptr) ? io.measured_heights + (long long)e0 * A1_POINTS + t
-                                                     : nullptr;
-#pragma unroll (NOISE ? 1 : 4)            // with NOISE: a Philox evaluation per env, unrolled it spills
-      for (int e = 0; e < ne; ++e) {
-        unsigned px, py;
-        const float hgt = scan_point<EXACT_DIV>(s.ev[e], bx, by, k, &px, &py);
-        float v = mul_rn(clampf(sub_rn(s.zb[e], hgt), -k.h_clip, k.h_clip), o.h_scale);
-        if (NOISE) v = add_rn(v, obs_noise_at(o, k.seed, k.env_offset + e0 + e, step, A1_HEAD + t));
-        v = clampf(v, -k.clip_obs, k.clip_obs);
-        __stcs(orow + (long long)e * A1_OBS, v);
-        if (mrow != nullptr) __stcs(mrow + (long long)e * A1_POINTS, hgt);
-      }
-    }
-    __syncthreads();   // shared memory is reused by the next tile of a grid-stride CTA
-  }
-}
+// The action head (num_obs = 235, or 48 with BLIND).
+#define A1_PHASED_KERNEL a1_post_physics_kernel_act
+#define A1_PHASED_HEAD A1_HEAD_ACT
+#include "a1_fused_kernel.inc"
+#undef A1_PHASED_KERNEL
+#undef A1_PHASED_HEAD
 
 // Row a7 stand-alone (shifu_a1_eval_terms): the descriptor's term list on the current tensors, one
 // CTA per 32 envs with the rows staged like phase A of the fused kernel; writes nothing but out.

@@ -108,19 +108,22 @@ __device__ __forceinline__ void v3_issue_loads(V3In& in, const A1K& k, const Shi
   for (int q = 0; q < k.n_terms; ++q) pipe::bulk_load(in.esum[q], io.ep_sums[q] + e0, sizeof(in.esum[q]), bar);
 }
 
-// With noise: the six head noise values of column d + 12m (m < 6) of env gid, words 3(d>>1) .. +2 of
-// SHIFU_STREAM_OBS_NOISE.  The lanes of columns d and d^1 (lane ^ 1) share the words: each evaluates one of
-// 3(d>>1), 3(d>>1)+1 and swaps halves with its neighbour, both evaluate 3(d>>1)+2.  hns: the six scales.
-__device__ __forceinline__ void head_noise6(const A1K& k, long long gid, long long step, int d, const float (&hns)[6],
-                                            float (&hn)[6]) {
+// With noise: the M head noise values of column d + 12m (m < M) of env gid, words 3(d>>1) .. of
+// SHIFU_STREAM_OBS_NOISE; M = 6 for the 72-column head, 4 for the action head (words 3(d>>1) + 2 not drawn).
+// The lanes of columns d and d^1 (lane ^ 1) share the words: each evaluates one of 3(d>>1), 3(d>>1)+1 and
+// swaps halves with its neighbour; with M = 6 both evaluate 3(d>>1)+2.  hns: the M scales.
+template <int M>
+__device__ __forceinline__ void head_noise(const A1K& k, long long gid, long long step, int d, const float (&hns)[M],
+                                           float (&hn)[M]) {
+  static_assert(M == 6 || M == 4, "a 72- or 48-column head");
   const int c = d & 1;
   const U4 wa = obs_noise_word(k.seed, gid, step, 3 * (d >> 1) + c);
-  const U4 wc = obs_noise_word(k.seed, gid, step, 3 * (d >> 1) + 2);
+  const U4 wc = M == 6 ? obs_noise_word(k.seed, gid, step, 3 * (d >> 1) + 2) : U4{0u, 0u, 0u, 0u};
   const uint32_t r0 = __shfl_xor_sync(~0u, c ? wa.x : wa.y, 1), r1 = __shfl_xor_sync(~0u, c ? wa.z : wa.w, 1);
   const uint32_t o0 = c ? wa.y : wa.x, o1 = c ? wa.w : wa.z;
   const uint32_t x[6] = {c ? r0 : o0, c ? r1 : o1, c ? o0 : r0, c ? o1 : r1, c ? wc.y : wc.x, c ? wc.w : wc.z};
 #pragma unroll
-  for (int m = 0; m < 6; ++m) hn[m] = mul_rn(u_pm1(x[m]), hns[m]);
+  for (int m = 0; m < M; ++m) hn[m] = mul_rn(u_pm1(x[m]), hns[m]);
 }
 
 // The B group (warps 0 .. V3_BG_WARPS-1, lane = env) of the pipelined kernels: the reward-term list
@@ -240,248 +243,21 @@ __device__ __forceinline__ void v3_b_group(const A1K& k, const ShifuA1StepIO& io
 // `o` is not read and the reference observation is built.
 // NOISE (only with OBS): uniform noise o.noise / o.h_noise is added before the clip to +-clip_obs, drawn
 // on STREAM_OBS_NOISE with the word map of include/shifu_b200.h.
-template <bool EXACT_DIV, bool HAS_MROW, bool HAS_EXTRA, bool OBS, bool NOISE>
-__global__ void __launch_bounds__(V3_THREADS, V3_CTAS_PER_SM)
-a1_post_physics_tma_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io, int num_tiles,
-                           const __grid_constant__ A1Obs o) {
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  V3Smem& s = *reinterpret_cast<V3Smem*>(smem_raw);
-  const int t = threadIdx.x;
-  const long long step = (io.step_dev != nullptr) ? *io.step_dev : io.step;
-  const int first = blockIdx.x, stride = gridDim.x;
-  const int my_tiles = (first < num_tiles) ? (num_tiles - first + stride - 1) / stride : 0;
+// HEAD (A1_HEAD_ACT only with OBS; a1_post_physics_tma_kernel_act): the action head.  A scan thread's head
+// item writes 4 columns, the last the step's action in.act[e][d] (read before the stage is released); the
+// heights follow at column 48 of a 235-column row.
+#define A1_TMA_KERNEL a1_post_physics_tma_kernel
+#define A1_TMA_HEAD A1_HEAD
+#include "a1_fused_tma_kernel.inc"
+#undef A1_TMA_KERNEL
+#undef A1_TMA_HEAD
 
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int b = 0; b < V3_STAGES; ++b) {
-      pipe::mbar_init(&s.full_in[b], 1);
-      // every thread of the producing group arrives itself: no group barrier, fast warps move on
-      pipe::mbar_init(&s.e_done[b], 32);                     // yaw / xy of the tile's envs are in the ring
-      pipe::mbar_init(&s.b_done[b], V3_B2_THREADS);
-      pipe::mbar_init(&s.h_done[b], V3_C_THREADS);
-    }
-    pipe::fence_barrier_init();
-  }
-  __syncthreads();
-
-  // =========================================================================================
-  if (t >= V3_DMA_BASE && t < V3_DMA_BASE + V3_DMA_THREADS) {
-    // ---------------- DMA warp ----------------
-    if (t != V3_DMA_BASE) return;
-    for (int j = 0; j < V3_STAGES && j < my_tiles; ++j)
-      v3_issue_loads(s.in[j], k, io, (long long)(first + j * stride) * A1_TILE, &s.full_in[j], true);
-    for (int j = 0; j < my_tiles; ++j) {
-      const int b = j % V3_STAGES;
-      const uint32_t par = (j / V3_STAGES) & 1;
-      const long long e0 = (long long)(first + j * stride) * A1_TILE;
-      // input rows are dead once the head / history phase is over: store the pushed history and
-      // refill the stage right away, long before the tile's height scan finishes
-      pipe::mbar_wait<64>(&s.h_done[b], par);
-      pipe::bulk_store(io.history + e0 * (A1_DOF * A1_HIST), s.in[b].hist, V3_HIST_BYTES);
-      if (io.carry_body_frame) {                              // robot.py:222-229 for the next control step (D7)
-        pipe::bulk_store(io.base_lin_vel + e0 * 3, s.in[b].cout[0], sizeof(s.in[b].cout[0]));
-        pipe::bulk_store(io.base_ang_vel + e0 * 3, s.in[b].cout[1], sizeof(s.in[b].cout[1]));
-        pipe::bulk_store(io.projected_gravity + e0 * 3, s.in[b].cout[2], sizeof(s.in[b].cout[2]));
-      }
-      pipe::bulk_commit();
-      // every other row of the stage is dead already: refill it while the store still reads hist
-      const long long en = (long long)(first + (j + V3_STAGES) * stride) * A1_TILE;
-      if (j + V3_STAGES < my_tiles) v3_issue_loads(s.in[b], k, io, en, &s.full_in[b], false);
-      pipe::bulk_wait_read_all();
-      if (j + V3_STAGES < my_tiles) v3_issue_hist_load(s.in[b], io, en, &s.full_in[b]);
-    }
-    pipe::bulk_wait_all();                                    // global writes done before exit
-    return;
-  }
-
-  if (t < V3_B_THREADS) {
-    v3_b_group<HAS_EXTRA, true, V3_STAGES>(k, io, s, my_tiles, first, stride, step, t);
-    return;
-  }
-
-  // ---------------- scan group: thread = scan point ----------------
-  {
-    const int p = t - V3_SCAN_BASE;                          // index in the scan group
-    const int sw = p >> 5, lane = p & 31;
-    // clip(clip(v,+-a),+-b) == clip(v,+-min(a,b)); with OBS, clip(clip(v,+-a)*s,+-b) == clip(v*s,+-h_bound)
-    // (with NOISE the noise sits between the two clips: heights are clipped to +-h_clip, scaled, noised
-    // and clipped to +-clip_obs)
-    const float hclip = NOISE ? k.clip_obs : OBS ? o.h_bound : fminf(k.h_clip, k.clip_obs);
-    const short* __restrict__ table = k.table;
-    const PairScanK sk = pair_scan_k(k);
-    const f2_t VS = pk(k.vscale, k.vscale);
-    // Work items of a tile (a lane owns a point and its mirror, see scan_pairs.cuh).
-    // Item = (group of 32 point pairs [3 groups cover the 94 pairs], batch of 4 envs): warp w owns pair
-    // group w % 3 for the env pairs 2*(V3_ITEMS*(w/3) + it), +1.  (The host routes grids that are not
-    // point-symmetric to the phased kernel.)
-    static_assert(V3_SCAN_WARPS % 3 == 0 && 8 % (V3_SCAN_WARPS / 3) == 0, "scan warps: 3 pair groups x rows");
-    constexpr int V3_ITEMS = 8 / (V3_SCAN_WARPS / 3);
-    // with NOISE: the noise scales of this thread's six head columns d + 12m, loaded once (a lane-dependent
-    // index into the parameter space would serialise the loads in the tile loop)
-    float hns[6];
-    if (NOISE) {
-      const int pd = p % A1_DOF;
-#pragma unroll
-      for (int m = 0; m < 6; ++m) hns[m] = o.noise[pd + 12 * m];
-    }
-    for (int j = 0; j < my_tiles; ++j) {
-      const int b = j % V3_STAGES;
-      const uint32_t par = (j / V3_STAGES) & 1;
-      const long long e0 = (long long)(first + j * stride) * A1_TILE;
-      const int rb = j & 3;
-      pipe::mbar_wait<32>(&s.e_done[b], par);
-      {
-        // item -> (scan point of this lane, first env pair of the batch)
-        struct Item { float bx, by; int q0, pt, it; bool live; };
-        auto item = [&](int it) {
-          Item r;
-          const int raw = 32 * (sw % 3) + lane;
-          r.live = raw <= A1_POINTS / 2;                      // pairs 0..93; 93 is the centre, its own mirror
-          r.pt = r.live ? raw : A1_POINTS / 2;                // idle lanes shadow the centre, stores masked
-          r.q0 = 2 * (V3_ITEMS * (sw / 3) + it);
-          r.bx = k.px[r.pt % A1_NX]; r.by = k.py[r.pt / A1_NX];
-          r.it = it;
-          return r;
-        };
-        // Index arithmetic of one item in packed fp32x2 (two envs per instruction).
-        auto index_batch = [&](const Item& w, unsigned (&idx)[8]) {
-          const f2_t BX = pk(w.bx, w.bx), BY = pk(w.by, w.by), NBY = pk(-w.by, -w.by);
-#pragma unroll
-          for (int u = 0; u < 2; ++u)
-            point_pair_cells<EXACT_DIV>(sk, BX, BY, NBY, s.sA[rb][w.q0 + u], s.sB[rb][w.q0 + u],
-                                        *reinterpret_cast<const float2*>(&s.sC[rb][w.q0 + u]), idx + 4 * u);
-        };
-        auto load_batch = [&](const unsigned (&idx)[8], int (&h)[8]) {
-#pragma unroll
-          for (int u = 0; u < 8; ++u) h[u] = __ldg(table + idx[u]);          // isaac_gym.py:427-431 (folded)
-        };
-        auto store_batch = [&](const Item& w, const int (&h)[8]) {
-          float* orow = io.obs_buf + (e0 + 2 * w.q0) * A1_OBS + A1_HEAD + w.pt;
-          float* mb = HAS_MROW ? io.measured_heights + (e0 + 2 * w.q0) * A1_POINTS + w.pt : nullptr;
-          // one packed pair of cells -> (z - 0.5) - h*vertical_scale, clipped, to rows r and r+1
-          auto emit = [&](float2 zb, int h0, int h1, float* ob, float* m, f2_t noise) {
-            const f2_t hg2 = fma2(pk((float)h0, (float)h1), VS, sk.nz);         // * vertical_scale, :433
-            float v0, v1;
-            f2_t d2 = sub2(pk(zb.x, zb.y), hg2);                                  // a1_conditional.py:132
-            if (NOISE) {
-              // fma(a, b, -0) is the product rounded once; a mul2 followed by the add2 would be contracted
-              // into one FFMA2 (DESIGN.md section 2)
-              upk(d2, v0, v1);
-              d2 = pk(clampf(v0, -k.h_clip, k.h_clip), clampf(v1, -k.h_clip, k.h_clip));
-              d2 = add2(fma2(d2, pk(o.h_scale, o.h_scale), sk.nz), noise);
-            } else if (OBS) {
-              d2 = mul2(d2, pk(o.h_scale, o.h_scale));
-            }
-            upk(d2, v0, v1);
-            __stcs(ob, clampf(v0, -hclip, hclip));
-            __stcs(ob + A1_OBS, clampf(v1, -hclip, hclip));
-            if (HAS_MROW) {
-              float g0, g1;
-              upk(hg2, g0, g1);
-              __stcs(m, g0);
-              __stcs(m + A1_POINTS, g1);
-            }
-          };
-          if (NOISE || w.live) {                                                // NOISE: every lane shuffles
-            const int mir = (A1_POINTS - 1) - 2 * w.pt;                           // column of the mirror point
-#pragma unroll
-            for (int u = 0; u < 2; ++u) {
-              // with NOISE: the envs 2(q0+u), +1 and the point pairs k, k^1 of this lane and its neighbour share
-              // word 18 + (k >> 1); lane k&1 evaluates it for env 2(q0+u) + (k&1) and swaps the neighbour's half
-              f2_t npt = 0, nmir = 0;
-              if (NOISE) {
-                const int c = lane & 1;                                             // = k & 1
-                const U4 q = obs_noise_word(k.seed, k.env_offset + e0 + 2 * (w.q0 + u) + c, step, 18 + (w.pt >> 1));
-                const uint32_t r0 = __shfl_xor_sync(~0u, c ? q.x : q.z, 1), r1 = __shfl_xor_sync(~0u, c ? q.y : q.w, 1);
-                const uint32_t o0 = c ? q.z : q.x, o1 = c ? q.w : q.y;            // (point, mirror) of own env
-                const float sh = o.h_noise;
-                const float p0 = mul_rn(u_pm1(c ? r0 : o0), sh), p1 = mul_rn(u_pm1(c ? o0 : r0), sh);
-                npt = pk(p0, p1);
-                nmir = (w.pt == A1_POINTS / 2) ? npt                              // the centre is its own mirror
-                                                : pk(mul_rn(u_pm1(c ? r1 : o1), sh), mul_rn(u_pm1(c ? o1 : r1), sh));
-              }
-              if (!NOISE || w.live) {
-                const float2 zb = *reinterpret_cast<const float2*>(&s.sC[rb][w.q0 + u].z);
-                emit(zb, h[4 * u], h[4 * u + 1], orow + (2 * u) * A1_OBS, mb + (2 * u) * A1_POINTS, npt);
-                emit(zb, h[4 * u + 2], h[4 * u + 3], orow + (2 * u) * A1_OBS + mir, mb + (2 * u) * A1_POINTS + mir, nmir);
-              }
-            }
-          }
-        };
-        // Rolled software pipeline (the body stays small enough for the instruction cache shared with
-        // the other warp roles): the gathers of item i are issued at the END of a trip and consumed
-        // in the MIDDLE of the next one, after the index arithmetic of item i+1 — so their L1/L2
-        // latency hides under ~200 instructions of independent math, with no register copies.  The
-        // first item's gathers are issued BEFORE the head phase, which hides them as well.
-        unsigned idx[8];
-        int h[8];    // sign-extended int16 cells
-        Item cur = item(0);
-        index_batch(cur, idx);
-        load_batch(idx, h);
-        // with OBS, a slot of projected_gravity reads its pre-step value from global memory, issued here to
-        // hide the latency: this tile's rows are bulk-stored over only after this thread's h_done arrival
-        float pgv = 0.0f;
-        if (OBS) {
-          const int pe = p / A1_DOF, pd = p - pe * A1_DOF;
-          if (o.src[pd / 3] == SHIFU_OBS_PROJECTED_GRAVITY) pgv = io.projected_gravity[(e0 + pe) * 3 + pd % 3];
-        }
-        // with NOISE, this thread's six head noise values: words 3(d>>1) .. +2 of its env, shared with the
-        // lane of column d^1 (the first word is split between the two lanes, the third read by both)
-        float hn[6];
-        if (NOISE) {
-          const int pe = p / A1_DOF, pd = p - pe * A1_DOF;
-          head_noise6(k, k.env_offset + e0 + pe, step, pd, hns, hn);
-        }
-        // ---- obs head (a1_conditional.py:131-144) + history push (train.py:12-14): post-reset rows
-        pipe::mbar_wait<32>(&s.b_done[b], par);
-        {
-          // One (env, dof) item and one (env, column) item per thread.  Everything the head reads from the
-          // stage is loaded FIRST and the history is pushed, then the stage is handed back (fence + arrive),
-          // and only then are the 6 observation values clamped and stored: the MEMBAR behind
-          // fence.proxy.async waits for every memory operation the thread has in flight, so with the
-          // global stores issued before it the stage release waited for their acknowledgements.
-          static_assert(A1_TILE * A1_DOF == V3_C_THREADS && A1_TILE * 12 == V3_C_THREADS, "one item per scan thread");
-          V3In& in = s.in[b];
-          const float c = k.clip_obs;
-          const int e = p / A1_DOF, d = p - e * A1_DOF;                    // e, d serve both items (12 columns each)
-          float* hrow = io.obs_buf + (e0 + e) * A1_OBS;
-          const float2 qd = *reinterpret_cast<const float2*>(&in.dof[e][2 * d]);
-          const float a0 = in.hist[e][d * A1_HIST + 0], a1 = in.hist[e][d * A1_HIST + 1],
-                      a2 = in.hist[e][d * A1_HIST + 2];
-          // command, velocities, gravity_vec; with OBS the slot's source
-          const float v = OBS ? a1_obs_vec(o, d, in.cla, e, pgv)
-                              : (d < 9) ? in.cla[d / 3][e][d % 3] : ((d == 11) ? -1.0f : 0.0f);
-          in.hist[e][d * A1_HIST + 2] = a1;              // HistoryRecorder.add (train.py:12-14)
-          in.hist[e][d * A1_HIST + 1] = a0;
-          in.hist[e][d * A1_HIST + 0] = in.act[e][d];
-          pipe::fence_proxy_async();                            // pushed history -> visible to the TMA store
-          pipe::mbar_arrive(&s.h_done[b]);
-          // with OBS: x_j * scale[j] before the clip
-          // with NOISE: + noise of column d + 12m before the clip
-          auto sc = [&](float x, int m) {
-            const float y = OBS ? mul_rn(x, o.scale[d + 12 * m]) : x;
-            return NOISE ? add_rn(y, hn[m]) : y;
-          };
-          __stcs(hrow + d, clampf(sc(v, 0), -c, c));
-          __stcs(hrow + 12 + d, clampf(sc(sub_rn(qd.x, k.q0[d]), 1), -c, c));
-          __stcs(hrow + 24 + d, clampf(sc(qd.y, 2), -c, c));
-          __stcs(hrow + 36 + d, clampf(sc(a0, 3), -c, c));   // HistoryRecorder.flatten: slot-major
-          __stcs(hrow + 48 + d, clampf(sc(a1, 4), -c, c));
-          __stcs(hrow + 60 + d, clampf(sc(a2, 5), -c, c));
-        }
-#pragma unroll 1
-        for (int it = 1; it < V3_ITEMS; ++it) {
-          const Item nxt = item(it);
-          index_batch(nxt, idx);
-          store_batch(cur, h);
-          load_batch(idx, h);
-          cur = nxt;
-        }
-        store_batch(cur, h);
-      }
-    }
-  }
-}
+// The action head (num_obs = 235): instantiated with OBS = true only.
+#define A1_TMA_KERNEL a1_post_physics_tma_kernel_act
+#define A1_TMA_HEAD A1_HEAD_ACT
+#include "a1_fused_tma_kernel.inc"
+#undef A1_TMA_KERNEL
+#undef A1_TMA_HEAD
 
 // ===================================================================================================
 // Blind form (72-column observation, no height scan): a streaming kernel.  Without the scan there is
@@ -514,11 +290,14 @@ struct alignas(128) VBSmem {
 };
 
 // Processes tiles [0, num_tiles) like the sighted kernel (the ragged tail is the phased kernel's).
-// HAS_EXTRA, OBS and NOISE as above; EXACT_DIV and HAS_MROW do not apply.  Noise uses words 0-17.
-template <bool HAS_EXTRA, bool OBS, bool NOISE>
-__global__ void __launch_bounds__(VB_THREADS, VB_CTAS_PER_SM)
-a1_post_physics_blind_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io, int num_tiles,
-                             const __grid_constant__ A1Obs o) {
+// HAS_EXTRA, OBS, NOISE and HEAD as above; EXACT_DIV and HAS_MROW do not apply.  Noise uses words 0-17
+// (the action head: words 3i and 3i + 1).  With HEAD = A1_HEAD_ACT the tile's observation is a 32 x 48
+// block (6 144 B) at the start of the stage's obs buffer (a1_post_physics_blind_kernel_act).
+template <bool HAS_EXTRA, bool OBS, bool NOISE, int HEAD>
+__device__ __forceinline__ void a1_post_physics_blind_body(const A1K& k, const ShifuA1StepIO& io, int num_tiles,
+                                                           const A1Obs& o) {
+  static_assert(HEAD == A1_HEAD || (OBS && HEAD == A1_HEAD_ACT), "the action head is an OBS layout");
+  constexpr int NM = HEAD / 12;                               // head columns per (env, dof) item
   extern __shared__ __align__(128) unsigned char smem_raw[];
   VBSmem& s = *reinterpret_cast<VBSmem*>(smem_raw);
   const int t = threadIdx.x;
@@ -547,7 +326,7 @@ a1_post_physics_blind_kernel(const __grid_constant__ A1K k, const __grid_constan
       const uint32_t par = (j / VB_STAGES) & 1;
       const long long e0 = (long long)(first + j * stride) * A1_TILE;
       pipe::mbar_wait<64>(&s.h_done[b], par);
-      pipe::bulk_store(io.obs_buf + e0 * A1_HEAD, s.in[b].obs, sizeof(s.in[b].obs));
+      pipe::bulk_store(io.obs_buf + e0 * HEAD, s.in[b].obs, A1_TILE * HEAD * 4);
       pipe::bulk_store(io.history + e0 * (A1_DOF * A1_HIST), s.in[b].hist, V3_HIST_BYTES);
       if (io.carry_body_frame) {                              // robot.py:222-229 for the next control step (D7)
         pipe::bulk_store(io.base_lin_vel + e0 * 3, s.in[b].cout[0], sizeof(s.in[b].cout[0]));
@@ -575,10 +354,10 @@ a1_post_physics_blind_kernel(const __grid_constant__ A1K k, const __grid_constan
   const int p = t - VB_HEAD_BASE;
   const int d = p % A1_DOF, g = p / A1_DOF;
   constexpr int NG = VB_H_THREADS / A1_DOF;                   // env groups: envs g + NG*r
-  float hns[6];                                               // this thread's six noise scales (columns d + 12m)
+  float hns[NM];                                              // this thread's noise scales (columns d + 12m)
   if (NOISE) {
 #pragma unroll
-    for (int m = 0; m < 6; ++m) hns[m] = o.noise[d + 12 * m];
+    for (int m = 0; m < NM; ++m) hns[m] = o.noise[d + 12 * m];
   }
   const bool pg_slot = OBS && o.src[d / 3] == SHIFU_OBS_PROJECTED_GRAVITY;
   for (int j = 0; j < my_tiles; ++j) {
@@ -598,8 +377,8 @@ a1_post_physics_blind_kernel(const __grid_constant__ A1K k, const __grid_constan
     for (int r = 0; r < VB_ENVS_PER_THREAD; ++r) {
       // obs head (a1_conditional.py:131-144) + history push (train.py:12-14) of env e, from the post-reset rows
       const int e = g + NG * r;
-      float hn[6];
-      if (NOISE) head_noise6(k, k.env_offset + e0 + e, step, d, hns, hn);
+      float hn[NM];
+      if (NOISE) head_noise<NM>(k, k.env_offset + e0 + e, step, d, hns, hn);
       const float2 qd = *reinterpret_cast<const float2*>(&in.dof[e][2 * d]);
       const float a0 = in.hist[e][d * A1_HIST + 0], a1 = in.hist[e][d * A1_HIST + 1],
                   a2 = in.hist[e][d * A1_HIST + 2];
@@ -612,17 +391,36 @@ a1_post_physics_blind_kernel(const __grid_constant__ A1K k, const __grid_constan
         const float y = OBS ? mul_rn(x, o.scale[d + 12 * m]) : x;
         return NOISE ? add_rn(y, hn[m]) : y;
       };
-      float* h = in.obs[e];
+      float* h = HEAD == A1_HEAD ? in.obs[e] : &in.obs[0][0] + e * HEAD;
       h[d] = clampf(sc(v, 0), -c, c);
       h[12 + d] = clampf(sc(sub_rn(qd.x, k.q0[d]), 1), -c, c);
       h[24 + d] = clampf(sc(qd.y, 2), -c, c);
-      h[36 + d] = clampf(sc(a0, 3), -c, c);                  // HistoryRecorder.flatten: slot-major
-      h[48 + d] = clampf(sc(a1, 4), -c, c);
-      h[60 + d] = clampf(sc(a2, 5), -c, c);
+      if constexpr (HEAD == A1_HEAD) {
+        h[36 + d] = clampf(sc(a0, 3), -c, c);                // HistoryRecorder.flatten: slot-major
+        h[48 + d] = clampf(sc(a1, 4), -c, c);
+        h[60 + d] = clampf(sc(a2, 5), -c, c);
+      } else {
+        h[36 + d] = clampf(sc(in.act[e][d], 3), -c, c);      // legged_gym's self.actions
+      }
     }
     pipe::fence_proxy_async();                                // obs block + pushed history -> the TMA stores
     pipe::mbar_arrive(&s.h_done[b]);
   }
+}
+
+template <bool HAS_EXTRA, bool OBS, bool NOISE>
+__global__ void __launch_bounds__(VB_THREADS, VB_CTAS_PER_SM)
+a1_post_physics_blind_kernel(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io, int num_tiles,
+                             const __grid_constant__ A1Obs o) {
+  a1_post_physics_blind_body<HAS_EXTRA, OBS, NOISE, A1_HEAD>(k, io, num_tiles, o);
+}
+
+// The 48-column action head (num_obs = 48): always an OBS layout.
+template <bool HAS_EXTRA, bool NOISE>
+__global__ void __launch_bounds__(VB_THREADS, VB_CTAS_PER_SM)
+a1_post_physics_blind_kernel_act(const __grid_constant__ A1K k, const __grid_constant__ ShifuA1StepIO io,
+                                 int num_tiles, const __grid_constant__ A1Obs o) {
+  a1_post_physics_blind_body<HAS_EXTRA, true, NOISE, A1_HEAD_ACT>(k, io, num_tiles, o);
 }
 
 }  // namespace shifu

@@ -83,14 +83,20 @@ struct A1Obs {
 };
 static_assert(STREAM_OBS_NOISE == SHIFU_STREAM_OBS_NOISE, "observation-noise stream");
 
-// Noise n = (2u - 1) * s of head column j < 72 or height column j >= 72 of env gid (the phased kernel's
+// Head width of the action head (ShifuA1Desc.num_obs = 235 or 48): the slots, dof_pos - q0, dof_vel and the
+// step's actions, where the 72-column head has the three history slots.
+constexpr int A1_HEAD_ACT = 48;
+static_assert(A1_HEAD_ACT == SHIFU_OBS_HEAD_ACT, "action head width");
+
+// Noise n = (2u - 1) * s of head column j < HEAD or height column j >= HEAD of env gid (the phased kernel's
 // form: one Philox evaluation per column; the pipelined kernel shares the words between lanes).
+template <int HEAD = A1_HEAD>
 __device__ __forceinline__ float obs_noise_at(const A1Obs& o, unsigned long long seed, long long gid, long long step,
                                               int j) {
   uint32_t word;
   int lane;
-  obs_noise_slot(j, word, lane);
-  return mul_rn(u_pm1(u4_lane(obs_noise_word(seed, gid, step, word), lane)), j < A1_HEAD ? o.noise[j] : o.h_noise);
+  obs_noise_slot(j, word, lane, HEAD);
+  return mul_rn(u_pm1(u4_lane(obs_noise_word(seed, gid, step, word), lane)), j < HEAD ? o.noise[j] : o.h_noise);
 }
 
 // Value of head column j < 12 of env e: slot j / 3, component j % 3.  cla = command, base lin vel,

@@ -69,15 +69,16 @@ struct ShifuCtx {
   int tma_occ = 0;
   bool use_tma = true;
   bool grid_symmetric = false;     // measured-point grid is point-symmetric (what the pipelined scan assumes)
-  bool blind = false;              // num_obs = SHIFU_OBS_HEAD: no height columns, no scan
+  bool blind = false;              // num_obs = SHIFU_OBS_HEAD or SHIFU_OBS_HEAD_ACT: no height columns, no scan
+  bool act_head = false;           // num_obs = 235 or 48: the action head (SHIFU_OBS_HEAD_ACT columns)
   int blind_occ = 0;
 };
 
 static inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
 // the pipelined kernel's instantiations, index = 8*(OBS + NOISE) + 4*EXACT_DIV + 2*HAS_MROW + HAS_EXTRA
-// (NOISE only with OBS)
-constexpr int A1_TMA_VARIANTS = 24;
+// (NOISE only with OBS), then the action head's (always OBS): 24 + 8*NOISE + 4*EXACT_DIV + 2*HAS_MROW + HAS_EXTRA
+constexpr int A1_TMA_VARIANTS = 40;
 template <bool OBS, bool NOISE>
 static void a1_tma_fill(const void** t) {
   t[0] = (const void*)a1_post_physics_tma_kernel<false, false, false, OBS, NOISE>;
@@ -89,19 +90,34 @@ static void a1_tma_fill(const void** t) {
   t[6] = (const void*)a1_post_physics_tma_kernel<true, true, false, OBS, NOISE>;
   t[7] = (const void*)a1_post_physics_tma_kernel<true, true, true, OBS, NOISE>;
 }
-// the blind pipelined kernel's instantiations, index = 2*(OBS + NOISE) + HAS_EXTRA (NOISE only with OBS)
-constexpr int A1_BLIND_VARIANTS = 6;
+template <bool NOISE>
+static void a1_tma_act_fill(const void** t) {
+  t[0] = (const void*)a1_post_physics_tma_kernel_act<false, false, false, true, NOISE>;
+  t[1] = (const void*)a1_post_physics_tma_kernel_act<false, false, true, true, NOISE>;
+  t[2] = (const void*)a1_post_physics_tma_kernel_act<false, true, false, true, NOISE>;
+  t[3] = (const void*)a1_post_physics_tma_kernel_act<false, true, true, true, NOISE>;
+  t[4] = (const void*)a1_post_physics_tma_kernel_act<true, false, false, true, NOISE>;
+  t[5] = (const void*)a1_post_physics_tma_kernel_act<true, false, true, true, NOISE>;
+  t[6] = (const void*)a1_post_physics_tma_kernel_act<true, true, false, true, NOISE>;
+  t[7] = (const void*)a1_post_physics_tma_kernel_act<true, true, true, true, NOISE>;
+}
+// the blind pipelined kernel's instantiations, index = 2*(OBS + NOISE) + HAS_EXTRA (NOISE only with OBS),
+// then the 48-column action head's: 6 + 2*NOISE + HAS_EXTRA
+constexpr int A1_BLIND_VARIANTS = 10;
 static const void* const* a1_blind_variants() {
   static const void* const table[A1_BLIND_VARIANTS] = {
       (const void*)a1_post_physics_blind_kernel<false, false, false>, (const void*)a1_post_physics_blind_kernel<true, false, false>,
       (const void*)a1_post_physics_blind_kernel<false, true, false>, (const void*)a1_post_physics_blind_kernel<true, true, false>,
-      (const void*)a1_post_physics_blind_kernel<false, true, true>, (const void*)a1_post_physics_blind_kernel<true, true, true>};
+      (const void*)a1_post_physics_blind_kernel<false, true, true>, (const void*)a1_post_physics_blind_kernel<true, true, true>,
+      (const void*)a1_post_physics_blind_kernel_act<false, false>, (const void*)a1_post_physics_blind_kernel_act<true, false>,
+      (const void*)a1_post_physics_blind_kernel_act<false, true>, (const void*)a1_post_physics_blind_kernel_act<true, true>};
   return table;
 }
 static const void* const* a1_tma_variants() {
   static const void* table[A1_TMA_VARIANTS];
   static const bool filled = (a1_tma_fill<false, false>(table), a1_tma_fill<true, false>(table + 8),
-                              a1_tma_fill<true, true>(table + 16), true);
+                              a1_tma_fill<true, true>(table + 16), a1_tma_act_fill<false>(table + 24),
+                              a1_tma_act_fill<true>(table + 32), true);
   (void)filled;
   return table;
 }
@@ -120,25 +136,32 @@ static float sqrt_threshold(float thr) {
 }
 
 // Observation layout of the descriptor -> o (identity for layout 0); custom = it differs from the reference.
+// The action head (num_obs = 235 or 48) reads obs_scale / obs_noise for j < SHIFU_OBS_HEAD_ACT only and is
+// always custom: it is never the reference observation.
 static int fill_a1obs(const ShifuA1Desc& d, A1Obs& o, bool& custom) {
   if (d.obs_layout != 0 && d.obs_layout != 1) return fail(SHIFU_E_RANGE, "obs_layout=%d must be 0 or 1", d.obs_layout);
+  const bool act = d.num_obs == A1_HEAD_ACT + A1_POINTS || d.num_obs == A1_HEAD_ACT;
+  const int head = act ? A1_HEAD_ACT : A1_HEAD;
+  if (act && d.obs_layout != 1)
+    return fail(SHIFU_E_RANGE, "num_obs = %d (the action head) needs obs_layout = 1: it is never the reference "
+                "observation", d.num_obs);
   std::memset(&o, 0, sizeof(o));
   for (int i = 0; i < 4; ++i) o.src[i] = i;                // COMMAND, BASE_LIN_VEL, BASE_ANG_VEL, GRAVITY_VEC
   for (int j = 0; j < A1_HEAD; ++j) o.scale[j] = 1.0f;
   o.h_scale = 1.0f;
   o.h_bound = std::fmin(d.height_clip, d.clip_obs);
   custom = false;
-  for (int j = 0; j <= A1_HEAD; ++j) {
-    const float v = j < A1_HEAD ? d.obs_noise[j] : d.obs_height_noise;
+  for (int j = 0; j <= head; ++j) {
+    const float v = j < head ? d.obs_noise[j] : d.obs_height_noise;
     if (!std::isfinite(v))
-      return j < A1_HEAD ? fail(SHIFU_E_RANGE, "obs_noise[%d]=%g is not finite", j, (double)v)
-                         : fail(SHIFU_E_RANGE, "obs_height_noise=%g is not finite", (double)v);
+      return j < head ? fail(SHIFU_E_RANGE, "obs_noise[%d]=%g is not finite", j, (double)v)
+                      : fail(SHIFU_E_RANGE, "obs_height_noise=%g is not finite", (double)v);
     if (v != 0.0f && d.obs_layout == 0)
       return fail(SHIFU_E_RANGE, "observation noise needs obs_layout = 1 (obs_layout = 0 ignores the layout fields)");
   }
-  if (d.num_obs == A1_HEAD && d.obs_height_noise != 0.0f)
+  if ((d.num_obs == A1_HEAD || d.num_obs == A1_HEAD_ACT) && d.obs_height_noise != 0.0f)
     return fail(SHIFU_E_RANGE, "obs_height_noise=%g with num_obs = %d: a blind observation has no height columns",
-                (double)d.obs_height_noise, A1_HEAD);
+                (double)d.obs_height_noise, d.num_obs);
   if (d.obs_layout == 0) return SHIFU_OK;
   for (int i = 0; i < 4; ++i) {
     if (d.obs_vec_src[i] < 0 || d.obs_vec_src[i] >= SHIFU_OBS_VEC_COUNT)
@@ -147,19 +170,20 @@ static int fill_a1obs(const ShifuA1Desc& d, A1Obs& o, bool& custom) {
     o.src[i] = d.obs_vec_src[i];
     o.uses_pg |= d.obs_vec_src[i] == SHIFU_OBS_PROJECTED_GRAVITY;
   }
-  for (int j = 0; j < A1_HEAD; ++j) {
+  custom |= act;
+  for (int j = 0; j < head; ++j) {
     if (!std::isfinite(d.obs_scale[j])) return fail(SHIFU_E_RANGE, "obs_scale[%d]=%g is not finite", j, (double)d.obs_scale[j]);
     custom |= d.obs_scale[j] != 1.0f;
     o.scale[j] = d.obs_scale[j];
   }
-  if (d.num_obs != A1_HEAD) {                              // a blind observation has no height columns
+  if (d.num_obs != A1_HEAD && d.num_obs != A1_HEAD_ACT) {  // a blind observation has no height columns
     if (!std::isfinite(d.obs_height_scale))
       return fail(SHIFU_E_RANGE, "obs_height_scale=%g is not finite", (double)d.obs_height_scale);
     custom |= d.obs_height_scale != 1.0f;
     o.h_scale = d.obs_height_scale;
     o.h_bound = std::fmin(d.height_clip * std::fabs(o.h_scale), d.clip_obs);
   }
-  for (int j = 0; j < A1_HEAD; ++j) { o.noise[j] = d.obs_noise[j]; o.noisy |= d.obs_noise[j] != 0.0f; }
+  for (int j = 0; j < head; ++j) { o.noise[j] = d.obs_noise[j]; o.noisy |= d.obs_noise[j] != 0.0f; }
   o.h_noise = d.obs_height_noise;
   o.noisy |= d.obs_height_noise != 0.0f;
   custom |= o.noisy != 0;
@@ -170,11 +194,13 @@ static int fill_a1k(const ShifuA1Desc& d, A1K& k) {
   if (d.abi_version != SHIFU_ABI_VERSION) return fail(SHIFU_E_RANGE, "ShifuA1Desc.abi_version %d != %d", d.abi_version, SHIFU_ABI_VERSION);
   if (d.num_envs <= 0) return fail(SHIFU_E_RANGE, "num_envs must be > 0 (got %d)", d.num_envs);
   if (d.num_dof != A1_DOF || d.num_bodies != A1_BODIES || d.num_hist != A1_HIST ||
-      (d.num_obs != A1_OBS && d.num_obs != A1_HEAD) || d.num_points_x != A1_NX || d.num_points_y != A1_NY)
+      (d.num_obs != A1_OBS && d.num_obs != A1_HEAD && d.num_obs != A1_HEAD_ACT + A1_POINTS && d.num_obs != A1_HEAD_ACT) ||
+      d.num_points_x != A1_NX || d.num_points_y != A1_NY)
     return fail(SHIFU_E_RANGE,
-                "this build is specialised for dof=%d bodies=%d hist=%d obs=%d or %d grid=%dx%d (got %d %d %d %d %dx%d)",
-                A1_DOF, A1_BODIES, A1_HIST, A1_OBS, A1_HEAD, A1_NX, A1_NY, d.num_dof, d.num_bodies, d.num_hist,
-                d.num_obs, d.num_points_x, d.num_points_y);
+                "this build is specialised for dof=%d bodies=%d hist=%d obs=%d or %d (%d or %d with the action head) "
+                "grid=%dx%d (got %d %d %d %d %dx%d)",
+                A1_DOF, A1_BODIES, A1_HIST, A1_OBS, A1_HEAD, A1_HEAD_ACT + A1_POINTS, A1_HEAD_ACT, A1_NX, A1_NY,
+                d.num_dof, d.num_bodies, d.num_hist, d.num_obs, d.num_points_x, d.num_points_y);
   if (d.base_body < 0 || d.base_body >= A1_BODIES || d.force_body < 0 || d.force_body >= A1_BODIES)
     return fail(SHIFU_E_RANGE, "base_body/force_body out of range");
   if (d.num_leg_bodies < 0 || d.num_leg_bodies > SHIFU_MAX_LEG_BODIES) return fail(SHIFU_E_RANGE, "num_leg_bodies out of range");
@@ -328,7 +354,8 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
   int n = 0;
   if (a1 != nullptr) {
     c->is_a1 = true; c->a1 = *a1; c->a1k = a1k; c->a1o = a1o; c->obs_custom = obs_custom; n = a1->num_envs;
-    c->blind = a1->num_obs == A1_HEAD;
+    c->blind = a1->num_obs == A1_HEAD || a1->num_obs == A1_HEAD_ACT;
+    c->act_head = a1->num_obs == A1_HEAD_ACT + A1_POINTS || a1->num_obs == A1_HEAD_ACT;
     c->grid_symmetric = true;
     for (int i = 0; i < A1_NX; ++i) c->grid_symmetric &= (a1k.px[i] == -a1k.px[A1_NX - 1 - i]);
     for (int i = 0; i < A1_NY; ++i) c->grid_symmetric &= (a1k.py[i] == -a1k.py[A1_NY - 1 - i]);
@@ -345,11 +372,14 @@ static int ctx_create_impl(int device, const ShifuA1Desc* a1, const ShifuAbbDesc
   if (e == cudaSuccess && c->is_a1) {
     // all four instantiations share resources; ask for the full shared-memory carve-out so the
     // resident-CTA count is bounded by registers/threads, not by the default L1/smem split
-    const void* variants[6] = {
+    const void* variants[12] = {
         (const void*)a1_post_physics_kernel<false, false, false>, (const void*)a1_post_physics_kernel<true, false, false>,
         (const void*)a1_post_physics_kernel<false, true, false>, (const void*)a1_post_physics_kernel<true, true, false>,
-        (const void*)a1_post_physics_kernel<false, false, true>, (const void*)a1_post_physics_kernel<false, true, true>};
-    for (int v = 0; v < 6 && e == cudaSuccess; ++v)
+        (const void*)a1_post_physics_kernel<false, false, true>, (const void*)a1_post_physics_kernel<false, true, true>,
+        (const void*)a1_post_physics_kernel_act<false, false, false>, (const void*)a1_post_physics_kernel_act<true, false, false>,
+        (const void*)a1_post_physics_kernel_act<false, true, false>, (const void*)a1_post_physics_kernel_act<true, true, false>,
+        (const void*)a1_post_physics_kernel_act<false, false, true>, (const void*)a1_post_physics_kernel_act<false, true, true>};
+    for (int v = 0; v < 12 && e == cudaSuccess; ++v)
       e = cudaFuncSetAttribute(variants[v], cudaFuncAttributePreferredSharedMemoryCarveout, 75);
     int occ = 0;
     if (e == cudaSuccess)
@@ -529,7 +559,7 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
   if (!c->is_a1) return fail(SHIFU_E_STATE, "shifu_a1_post_physics needs an A1 ctx");
   if (!c->blind && c->d_table == nullptr) return fail(SHIFU_E_STATE, "call shifu_set_height_map first");
   if (c->blind && io->measured_heights != nullptr)
-    return fail(SHIFU_E_RANGE, "measured_heights must be NULL with num_obs = %d (no height scan)", A1_HEAD);
+    return fail(SHIFU_E_RANGE, "measured_heights must be NULL with num_obs = %d (no height scan)", c->a1.num_obs);
   REQUIRE_PTR(io->root_state); REQUIRE_PTR(io->dof_state); REQUIRE_PTR(io->contact_state);
   REQUIRE_PTR(io->actions); REQUIRE_PTR(io->torques); REQUIRE_PTR(io->history); REQUIRE_PTR(io->command);
   REQUIRE_PTR(io->ep_len); REQUIRE_PTR(io->base_lin_vel); REQUIRE_PTR(io->base_ang_vel);
@@ -561,7 +591,8 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     for (int q = 0; q < c->a1k.n_terms; ++q) extra |= c->a1k.terms[q] >= SHIFU_REW_LIN_VEL_Z;
     int tiles_arg = full_tiles;
     void* args[4] = {(void*)&c->a1k, const_cast<ShifuA1StepIO*>(io), (void*)&tiles_arg, (void*)&c->a1o};
-    const int variant = (c->obs_custom ? 2 : 0) + (c->a1o.noisy ? 2 : 0) + (extra ? 1 : 0);
+    const int variant = c->act_head ? 6 + (c->a1o.noisy ? 2 : 0) + (extra ? 1 : 0)
+                                    : (c->obs_custom ? 2 : 0) + (c->a1o.noisy ? 2 : 0) + (extra ? 1 : 0);
     CUDA_TRY(cudaLaunchKernel(a1_blind_variants()[variant], grid, block, args, sizeof(VBSmem), S(stream)));
   } else if (full_tiles > 0) {
     const int cap = c->sm_count * (c->tma_occ > 0 ? c->tma_occ : 1);
@@ -572,7 +603,8 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     for (int q = 0; q < c->a1k.n_terms; ++q) extra |= c->a1k.terms[q] >= SHIFU_REW_LIN_VEL_Z;
     int tiles_arg = full_tiles;
     void* args[4] = {(void*)&c->a1k, const_cast<ShifuA1StepIO*>(io), (void*)&tiles_arg, (void*)&c->a1o};
-    const int variant = (c->obs_custom ? 8 : 0) + (c->a1o.noisy ? 8 : 0) + (exact ? 4 : 0) + (mrow ? 2 : 0) + (extra ? 1 : 0);
+    const int variant = (c->act_head ? 24 : c->obs_custom ? 8 : 0) + (c->a1o.noisy ? 8 : 0) + (exact ? 4 : 0) +
+                        (mrow ? 2 : 0) + (extra ? 1 : 0);
     CUDA_TRY(cudaLaunchKernel(a1_tma_variants()[variant], grid, block, args, smem, S(stream)));
   }
   const int tiles = (n + A1_TILE - 1) / A1_TILE - full_tiles;    // the ragged tail, or every tile
@@ -581,7 +613,18 @@ extern "C" int shifu_a1_post_physics(ShifuCtx* c, const ShifuA1StepIO* io, void*
     const dim3 grid(tiles < cap ? tiles : cap), block(A1_THREADS);
     const A1K& k = c->a1k;
     const A1Obs& o = c->a1o;
-    if (c->blind) {
+    if (c->act_head) {
+      if (c->blind) {
+        if (o.noisy) a1_post_physics_kernel_act<false, true, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+        else a1_post_physics_kernel_act<false, false, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      } else if (o.noisy) {
+        if (exact) a1_post_physics_kernel_act<true, true, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+        else a1_post_physics_kernel_act<false, true, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      } else {
+        if (exact) a1_post_physics_kernel_act<true, false, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+        else a1_post_physics_kernel_act<false, false, false><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
+      }
+    } else if (c->blind) {
       if (o.noisy) a1_post_physics_kernel<false, true, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
       else a1_post_physics_kernel<false, false, true><<<grid, block, 0, S(stream)>>>(k, *io, o, full_tiles);
     } else if (o.noisy) {

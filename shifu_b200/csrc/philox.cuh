@@ -56,14 +56,15 @@ __device__ __forceinline__ U4 obs_noise_word(uint64_t seed, int64_t gid, int64_t
   return philox4x32_10((uint32_t)gid, (uint32_t)step, STREAM_OBS_NOISE, word, (uint32_t)seed, (uint32_t)(seed >> 32));
 }
 
-// The (word, lane) of observation column `col` < 259 (the map of include/shifu_b200.h).
-__device__ __forceinline__ void obs_noise_slot(int col, uint32_t& word, int& lane) {
-  if (col < 72) {                                   // head: column d + 12m, lane pair d = 2i, 2i+1
+// The (word, lane) of observation column `col` < head + 187 (the map of include/shifu_b200.h).  head: the
+// head width, 72 or 48 (the action head: its column d + 12m, m < 4, keeps the word and lane it has at 72).
+__device__ __forceinline__ void obs_noise_slot(int col, uint32_t& word, int& lane, int head = 72) {
+  if (col < head) {                                 // head: column d + 12m, lane pair d = 2i, 2i+1
     const int m = col / 12, d = col - 12 * m;
     word = 3 * (d >> 1) + (m >> 1);
     lane = (d & 1) + 2 * (m & 1);
   } else {                                          // heights: point pair k = (pt, 186 - pt)
-    const int pt = col - 72, k = min(pt, 186 - pt);
+    const int pt = col - head, k = min(pt, 186 - pt);
     word = 18 + (k >> 1);
     lane = 2 * (k & 1) + (pt != k ? 1 : 0);
   }

@@ -112,19 +112,25 @@ def fuse_a1(env, carry_body_frame: bool = True, rng_seed: int = 0x5EED):
     if not isinstance(isg, TerrainGymEnv) or not isinstance(rb, LeggedRobot):
         raise NotFusable("needs a TerrainGymEnv with a LeggedRobot")
     tc = cfg.terrain
-    # the observation width picks the step: 72 + 187 scans the terrain, 72 is blind (no height columns)
+    # the observation width picks the step: a 72- or 48-column head (48: the step's actions in place of the
+    # action history, legged_gym's own observation), + 187 heights scanned from the terrain, or blind
     num_obs = cfg.num_obs
-    if num_obs not in (nv.OBS_HEAD, nv.OBS_HEAD + nv.MAX_PX * nv.MAX_PY) or cfg.num_privileged_obs is not None:
-        raise NotFusable("observation width is not 72 + 187 or 72")
-    blind = num_obs == nv.OBS_HEAD
+    points = nv.MAX_PX * nv.MAX_PY
+    if num_obs not in (nv.OBS_HEAD, nv.OBS_HEAD + points, nv.OBS_HEAD_ACT, nv.OBS_HEAD_ACT + points) \
+            or cfg.num_privileged_obs is not None:
+        raise NotFusable("observation width is not 72 + 187 or 72, or 48 + 187 or 48 with the step's actions")
+    blind = num_obs in (nv.OBS_HEAD, nv.OBS_HEAD_ACT)
     if not blind and ((len(tc.measured_points_x), len(tc.measured_points_y)) != (nv.MAX_PX, nv.MAX_PY)
                       or not tc.measure_heights):
         raise NotFusable("the fused kernel is compiled for the 17x11 measured-point grid")
     store_heights = bool(getattr(cfg, "store_measured_heights", False))
     if blind and store_heights:
-        raise NotFusable("store_measured_heights with a 72-column observation: the fused blind step does not scan "
-                         "the terrain")
-    if (rb.num_dof, rb.num_bodies, cfg.num_actions, cfg.num_actions_history) != (12, 17, 12, 3):
+        raise NotFusable(f"store_measured_heights with a {num_obs}-column observation: the fused blind step does not "
+                         "scan the terrain")
+    if cfg.num_actions_history != 3:
+        raise NotFusable(f"num_actions_history = {cfg.num_actions_history}: the fused step keeps a history of "
+                         "exactly 3 past actions (an observation of the step's actions alone still needs it)")
+    if (rb.num_dof, rb.num_bodies, cfg.num_actions) != (12, 17, 12):
         raise NotFusable("the fused kernel is compiled for 12 dofs / 17 bodies / 3 past actions")
     layout = rb.affine_root_layout()
     if layout is None:
@@ -218,12 +224,12 @@ def a1_env_desc(env, terms, *, rng_seed: int, force_body: int, push_force_max: f
     terrain scales from its config, curriculum, levels and env length from its gym env, and its episode
     lengths, clips and command ranges.  ``terms`` and ``kw`` (``obs``, ``action_scale``, ``air_time_reset``,
     the compiled terms' extras) go to ``a1_desc`` as they are; ``num_obs`` defaults to the config's.  A blind
-    descriptor (``num_obs = 72``) keeps the compiled 17x11 grid whatever the config's: the blind step does not
+    descriptor (``num_obs = 72`` or 48) keeps the compiled 17x11 grid whatever the config's: the blind step does not
     scan, and the on-demand heights come from the gym env's own scan."""
     rb, isg, tc = env.robot, env.isg_env, env.cfg.terrain
     stride, offset = rb.affine_root_layout()
     kw.setdefault("num_obs", env.cfg.num_obs)
-    grid = {} if kw["num_obs"] == nv.OBS_HEAD else dict(points_x=tuple(tc.measured_points_x),
+    grid = {} if kw["num_obs"] in (nv.OBS_HEAD, nv.OBS_HEAD_ACT) else dict(points_x=tuple(tc.measured_points_x),
                                                          points_y=tuple(tc.measured_points_y))
     desc = hotpath.a1_desc(
         env.num_envs, env_offset=env.env_offset, rng_seed=rng_seed, terms=terms,
@@ -246,7 +252,7 @@ def a1_env_desc(env, terms, *, rng_seed: int, force_body: int, push_force_max: f
 def a1_hot_path(env, desc: nv.A1Desc, names, carry_body_frame: bool, want_measured_heights: bool) -> hotpath.A1HotPath:
     """An ``A1HotPath`` for ``desc`` over the env's gym tensors (a blind descriptor takes no height map)."""
     isg = env.isg_env
-    blind = desc.num_obs == nv.OBS_HEAD
+    blind = desc.num_obs in (nv.OBS_HEAD, nv.OBS_HEAD_ACT)
     return hotpath.A1HotPath(desc, root_state=isg.root_state, dof_state=isg.dof_state, contact_state=isg.contact_state,
                              height_samples=None if blind else isg.height_samples, terrain_origins=isg.terrain_origins,
                              terrain_types=isg.terrain_types, env_origins=isg.env_origins, terms=names,

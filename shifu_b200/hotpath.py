@@ -50,7 +50,7 @@ A1_OBS_SLOTS = ("COMMAND", "BASE_LIN_VEL", "BASE_ANG_VEL", "GRAVITY_VEC")      #
 
 @dataclass(frozen=True)
 class ObsLayout:
-    """Layout of the 259-column A1 observation the fused kernel builds.
+    """Layout of the 259-column A1 observation the fused kernel builds, or of the 235-column action head.
 
     Columns 0-11 are four 3-column slots, ``slots[i]`` naming the source of columns 3i..3i+2 (a key of
     ``OBS_SOURCES``); every head column j < 72 is ``clip(x_j * scales[j], +-clip_obs)`` (the dof-position
@@ -62,11 +62,16 @@ class ObsLayout:
     ``noise`` / ``height_noise``: legged_gym's uniform observation noise (``noise_scale_vec``), one scale per
     head column and one for all 187 heights.  Column j gets ``+ (2u - 1) * noise[j]`` before the clip to
     +-clip_obs, u drawn per env, step and column from the kernels' Philox stream
-    (``shifu_b200.utils.philox.obs_noise_u01``).  All zero: no noise."""
+    (``shifu_b200.utils.philox.obs_noise_u01``).  All zero: no noise.
+
+    The head width is ``len(scales)``: 72, or 48 for the action head (legged_gym's own observation), whose
+    columns 0-35 are the 72-column head's and whose column 36 + d is the step's ``actions[:, d]`` times
+    ``scales[36 + d]``; its heights follow at column 48.  ``noise`` has one scale per head column (default:
+    zeros of the head width)."""
     slots: Tuple[str, str, str, str] = A1_OBS_SLOTS
     scales: Tuple[float, ...] = (1.0,) * nv.OBS_HEAD
     height_scale: float = 1.0
-    noise: Tuple[float, ...] = (0.0,) * nv.OBS_HEAD
+    noise: Optional[Tuple[float, ...]] = None
     height_noise: float = 0.0
 
     def __post_init__(self):
@@ -74,14 +79,15 @@ class ObsLayout:
         if len(slots) != 4 or any(s not in OBS_SOURCES for s in slots):
             raise ValueError(f"slots must be 4 names out of {sorted(OBS_SOURCES)}, got {slots}")
         scales = tuple(float(np.float32(v)) for v in self.scales)
-        if len(scales) != nv.OBS_HEAD:
-            raise ValueError(f"{len(scales)} column scales: the observation head has {nv.OBS_HEAD} columns")
+        if len(scales) not in (nv.OBS_HEAD, nv.OBS_HEAD_ACT):
+            raise ValueError(f"{len(scales)} column scales: the observation head has {nv.OBS_HEAD} columns, or "
+                             f"{nv.OBS_HEAD_ACT} with the step's actions")
         hs = float(np.float32(self.height_scale))
         if not all(math.isfinite(v) for v in (*scales, hs)):
             raise ValueError("observation scales must be finite")
-        noise = tuple(float(np.float32(v)) for v in self.noise)
-        if len(noise) != nv.OBS_HEAD:
-            raise ValueError(f"{len(noise)} column noise scales: the observation head has {nv.OBS_HEAD} columns")
+        noise = tuple(float(np.float32(v)) for v in (self.noise if self.noise is not None else (0.0,) * len(scales)))
+        if len(noise) != len(scales):
+            raise ValueError(f"{len(noise)} column noise scales: the observation head has {len(scales)} columns")
         hn = float(np.float32(self.height_noise))
         if not all(math.isfinite(v) for v in (*noise, hn)):
             raise ValueError("observation noise scales must be finite")
@@ -91,13 +97,19 @@ class ObsLayout:
         object.__setattr__(self, "noise", noise)
         object.__setattr__(self, "height_noise", hn)
 
+    @property
+    def head(self) -> int:
+        """The head width: 72, or 48 for the action head."""
+        return len(self.scales)
+
     def has_noise(self) -> bool:
         return any(v != 0.0 for v in self.noise) or self.height_noise != 0.0
 
     def is_reference(self) -> bool:
-        """The reference observation (a1_conditional.py:131-144): identity scales, reference slots, no noise."""
-        return (self.slots == A1_OBS_SLOTS and all(v == 1.0 for v in self.scales) and self.height_scale == 1.0
-                and not self.has_noise())
+        """The reference observation (a1_conditional.py:131-144): identity scales, reference slots, no noise.
+        The action head never is."""
+        return (self.head == nv.OBS_HEAD and self.slots == A1_OBS_SLOTS and all(v == 1.0 for v in self.scales)
+                and self.height_scale == 1.0 and not self.has_noise())
 
 
 def compile_reward_terms(names: Sequence[str], codes: Dict[str, int], params: Dict[str, tuple]):
@@ -137,12 +149,21 @@ def a1_desc(num_envs: int, *, env_offset: int = 0, rng_seed: int = 0x5EED,
             num_obs: int = nv.OBS_HEAD + 187) -> nv.A1Desc:
     """Defaults = the constants of ``examples/a1_conditional`` (SURVEY.md Appendix A).  ``obs``: the
     observation layout; ``None`` or the reference layout writes ``obs_layout = 0``.  ``num_obs``: 259, or
-    72 for a blind task (the observation without its 187 height columns; ``obs.height_noise`` must be 0)."""
-    if num_obs not in (nv.OBS_HEAD, nv.OBS_HEAD + 187):
+    72 for a blind task (the observation without its 187 height columns; ``obs.height_noise`` must be 0);
+    235 or 48 (blind) for the action head, which needs an ``obs`` of head width 48 and always writes
+    ``obs_layout = 1``."""
+    head = nv.OBS_HEAD_ACT if num_obs in (nv.OBS_HEAD_ACT, nv.OBS_HEAD_ACT + 187) else nv.OBS_HEAD
+    if num_obs not in (head, head + 187):
         raise ValueError(f"num_obs={num_obs}: the fused A1 observation has {nv.OBS_HEAD + 187} columns, or "
-                         f"{nv.OBS_HEAD} without the height scan")
-    if num_obs == nv.OBS_HEAD and obs is not None and obs.height_noise != 0.0:
-        raise ValueError("a blind observation (num_obs = 72) has no height columns to add height noise to")
+                         f"{nv.OBS_HEAD} without the height scan ({nv.OBS_HEAD_ACT + 187} or {nv.OBS_HEAD_ACT} "
+                         "with the step's actions in place of the action history)")
+    if head == nv.OBS_HEAD_ACT and obs is None:
+        raise ValueError(f"num_obs={num_obs} (the action head) needs an ObsLayout: it is never the reference "
+                         "observation")
+    if obs is not None and obs.head != head:
+        raise ValueError(f"num_obs={num_obs} has a {head}-column head; the layout has {obs.head} columns")
+    if num_obs == head and obs is not None and obs.height_noise != 0.0:
+        raise ValueError(f"a blind observation (num_obs = {num_obs}) has no height columns to add height noise to")
     d = nv.A1Desc()
     d.abi_version = nv.ABI_VERSION
     d.num_envs, d.env_offset, d.rng_seed = num_envs, env_offset, rng_seed
@@ -190,7 +211,7 @@ def a1_desc(num_envs: int, *, env_offset: int = 0, rng_seed: int = 0x5EED,
     for i, (code, p0, p1) in enumerate(comp):
         d.reward_terms[i] = code
         d.reward_params[i][0], d.reward_params[i][1] = p0, p1
-    if obs is not None and not obs.is_reference():
+    if obs is not None and not obs.is_reference():           # (the action head never collapses to layout 0)
         d.obs_layout = 1
         for i, name in enumerate(obs.slots):
             d.obs_vec_src[i] = OBS_SOURCES[name]
@@ -425,8 +446,8 @@ class HeightScan:
 class A1HotPath(_StepStats):
     """Fused A1 step. ``root_state`` / ``dof_state`` / ``contact_state`` are the gym's flat tensors.
 
-    A blind descriptor (``num_obs = 72``) builds the (N, 72) observation without the height scan: it takes
-    ``height_samples=None`` and keeps no ``measured_heights``.  A height map, when given, is uploaded for
+    A blind descriptor (``num_obs = 72``, or 48 with the action head) builds the (N, 72) or (N, 48)
+    observation without the height scan: it takes ``height_samples=None`` and keeps no ``measured_heights``.  A height map, when given, is uploaded for
     ``get_heights(out=...)``, which then needs its own output tensor."""
 
     def __init__(self, desc: nv.A1Desc, *, root_state, dof_state, contact_state, height_samples,
@@ -437,11 +458,12 @@ class A1HotPath(_StepStats):
         self.desc = desc
         self.n = n = desc.num_envs
         self.terms = list(terms)
-        self.blind = desc.num_obs == nv.OBS_HEAD
+        self.blind = desc.num_obs in (nv.OBS_HEAD, nv.OBS_HEAD_ACT)
         if self.blind and want_measured_heights:
-            raise ValueError("a blind A1 step (num_obs = 72) does not scan: it cannot store measured_heights")
+            raise ValueError(f"a blind A1 step (num_obs = {desc.num_obs}) does not scan: it cannot store "
+                             "measured_heights")
         if height_samples is None and not self.blind:
-            raise ValueError("the 259-column A1 step scans the height map: height_samples is required")
+            raise ValueError(f"the {desc.num_obs}-column A1 step scans the height map: height_samples is required")
         self.ctx = _Ctx(dev, a1=desc)
         self.lib = self.ctx.lib
         f = dict(device=dev, dtype=torch.float)

@@ -168,10 +168,10 @@ class A1Conditional(ShifuVecEnv):
             raise NotImplementedError("the fused A1 kernel needs affine root_indices")
         names = [fn.__name__ for fn in self.reward_functions]
         obs = None
-        num_obs = self.cfg.num_obs                  # 72 + 187, or 72 for a blind subclass
-        if num_obs == 72 and self._store_heights:
-            raise NotImplementedError("store_measured_heights with a 72-column observation: the fused blind step "
-                                      "does not scan the terrain (fused=False measures and keeps the heights)")
+        num_obs = self.cfg.num_obs                  # 72 + 187, or 72 for a blind subclass (48 + 187, 48: actions)
+        if num_obs in (72, 48) and self._store_heights:
+            raise NotImplementedError(f"store_measured_heights with a {num_obs}-column observation: the fused blind "
+                                      "step does not scan the terrain (fused=False measures and keeps the heights)")
         if type(self).compute_observations is not A1Conditional.compute_observations or num_obs != 259:
             # an edited observation hook: fused only when the kernel's observation layout expresses it,
             # never silently replaced by the reference observation

@@ -365,8 +365,8 @@ def _exact_offset(q0: float) -> float:
 class _NoHeights:
     """Stands in for ``measured_heights`` while a blind (72-column) observation hook runs: the fused blind
     step does not scan the terrain, so any use of the heights refuses the hook."""
-    REASON = ("compute_observations: the 72-column (blind) observation reads measured_heights; the fused blind "
-              "step does not scan the terrain")
+    REASON = ("compute_observations: the blind (72- or 48-column) observation reads measured_heights; the fused "
+              "blind step does not scan the terrain")
 
     def __init__(self):
         self.touched = False
@@ -453,13 +453,18 @@ def compile_a1_obs(env, num_obs: Optional[int] = None) -> ObsLayout:
     one scale, added after their clip and scale (probed at z - 0.5 - h = 3).
     A hook that returns (N, 72) is blind: the same head probes run with the measured heights replaced by
     a stand-in whose every use refuses the hook, and there are no height probes (the layout keeps height
-    scale 1 and no height noise).  ``num_obs``: the width the hook must return (default: 72 + the height
-    points, or 72 when the hook returns 72 columns).
+    scale 1 and no height noise).
+    A 48-column head (num_obs 48 + the height points, or 48 blind) is the action head, legged_gym's own
+    observation: each ``env.actions[:, d]`` must reach column 36 + d alone, as a scale times the action, and
+    the action history none; in a 72-column head the step's actions must reach no column.  The heights and
+    their noise then start at column 48.  ``num_obs``: the width the hook must return (default: the
+    hook's own width when it is one of these four, else 72 + the height points).
     Anything else raises NotFusable naming the column and the reason."""
     rb, isg = env.robot, env.isg_env
-    n_head = nv.OBS_HEAD
-    if num_obs is not None and num_obs not in (n_head, n_head + isg.num_height_points):
-        raise NotFusable(f"observation width {num_obs} is neither {n_head} nor {n_head + isg.num_height_points}")
+    widths = [h + p for h in (nv.OBS_HEAD, nv.OBS_HEAD_ACT) for p in (isg.num_height_points, 0)]
+    if num_obs is not None and num_obs not in widths:
+        raise NotFusable(f"observation width {num_obs} is none of {widths} (72 or 48 head columns, with or "
+                         "without the height points)")
     had = isg.__dict__.get("_measured_heights")
     with A1Probe(env) as pr:
         t = pr.tensors
@@ -475,12 +480,15 @@ def compile_a1_obs(env, num_obs: Optional[int] = None) -> ObsLayout:
             heights.zero_()
 
         width = num_obs
-        if width is None:                           # the hook's own width: 72 (blind) or 72 + the heights
+        if width is None:                           # the hook's own width: a head, or a head + the heights
             zero_state()
             isg.measured_heights = heights
             with _obs_draws(env, 0.5, env.obs_buf.shape[1]):
                 env.compute_observations()
-            width = n_head if tuple(env.obs_buf.shape) == (env.num_envs, n_head) else n_head + heights.shape[1]
+            shape = tuple(env.obs_buf.shape)
+            width = shape[1] if len(shape) == 2 and shape[0] == env.num_envs and shape[1] in widths \
+                else nv.OBS_HEAD + heights.shape[1]
+        n_head = nv.OBS_HEAD_ACT if width in (nv.OBS_HEAD_ACT, nv.OBS_HEAD_ACT + heights.shape[1]) else nv.OBS_HEAD
         blind = width == n_head
 
         def observe(u=0.5):
@@ -534,26 +542,51 @@ def compile_a1_obs(env, num_obs: Optional[int] = None) -> ObsLayout:
                 if src is None:
                     raise NotFusable(f"compute_observations: columns {3 * i}-{3 * i + 2} follow none of "
                                      f"{[label for _, label in _OBS_PROBE.values()]}")
-            # dof positions (dof_pos - default_dof_pos), dof velocities, history slot-major
+            # dof positions (dof_pos - default_dof_pos), dof velocities, then the step's actions (48-column
+            # head) or the history slot-major (72-column head); col None: the input must reach no column
+            act = n_head == nv.OBS_HEAD_ACT
             probes = []
             for d in range(12):
                 probes.append((12 + d, f"dof_pos[:, {d}] - default_dof_pos[{d}]", ("dof", d, 0)))
                 probes.append((24 + d, f"dof_vel[:, {d}]", ("dof", d, 1)))
+                probes.append((36 + d if act else None, f"actions[:, {d}]", ("actions", 0, d)))
                 for h in range(3):
-                    probes.append((36 + 12 * h + d, f"actions_recorder.get_last({h})[:, {d}]", ("history", d, h)))
-            for col, label, (key, a, b) in probes:
+                    probes.append((None if act else 36 + 12 * h + d, f"actions_recorder.get_last({h})[:, {d}]",
+                                   ("history", d, h)))
+            mixed = (f"the {n_head}-column head observes "
+                     + ("the step's actions (env.actions, column 36 + d), not the action history (actions_recorder)"
+                        if act else "the action history (actions_recorder), not the step's actions (env.actions): "
+                        "the step's actions are the 48-column action head (num_obs 235 or 48)"))
+
+            def probe(key, a, b, x):
                 zero_state()
                 if key == "dof" and b == 0:
-                    x = _exact_offset(float(q0[a]))
                     dof[0, a, 0] = float(torch.tensor(float(q0[a]), dtype=torch.float) + x)
+                elif key == "actions":
+                    t["actions"][0, b] = x
                 else:
-                    x = 1.0
                     (dof if key == "dof" else t["history"])[0, a, b] = x
-                hits = lit(observe(), 0, None)
+                return lit(observe(), 0, None)
+
+            for col, label, (key, a, b) in probes:
+                x = _exact_offset(float(q0[a])) if key == "dof" and b == 0 else 1.0
+                hits = probe(key, a, b, x)
+                if col is None:
+                    if hits:
+                        raise NotFusable(f"compute_observations: {label} reaches columns {[j for j, _ in hits]}; "
+                                         + mixed)
+                    continue
                 if len(hits) != 1 or hits[0][0] != col:
                     raise NotFusable(f"compute_observations: {label} reaches columns {[j for j, _ in hits]}; the "
-                                     f"fused observation has it in column {col} alone")
+                                     f"fused observation has it in column {col} alone"
+                                     + (f" ({mixed})" if key in ("actions", "history") else ""))
                 scales[col] = hits[0][1] / x
+                if key == "actions":                    # a scale times the action: half the input, half the value
+                    half = probe(key, a, b, 0.5 * x)
+                    if len(half) != 1 or half[0][0] != col or half[0][1] != 0.5 * hits[0][1]:
+                        raise NotFusable(f"compute_observations: column {col} is {hits[0][1]:g} at {label} = 1 "
+                                         f"and {half[0][1] if half else 0.0:g} at 0.5; the fused observation takes "
+                                         "the step's actions times a scale, no other function of them")
             if blind:                                       # no height columns: no height probes
                 zero_state()
                 up, down = observe(1.0), observe(0.0)
@@ -619,12 +652,14 @@ def compile_a1_obs(env, num_obs: Optional[int] = None) -> ObsLayout:
 
 def a1_obs_definition(env, layout: ObsLayout, u: Optional[torch.Tensor] = None, blind: bool = False) -> torch.Tensor:
     """The observation the fused kernel builds under ``layout``, in torch on the env's tensors (before the
-    final clip to +-clip_obs that the base class applies).  ``u``: the noise draws, (num_envs, 259), or
-    (num_envs, 72) when ``blind`` (the 72 head columns alone)."""
+    final clip to +-clip_obs that the base class applies).  ``u``: the noise draws, (num_envs, head + 259 -
+    72), or (num_envs, head) when ``blind`` (the head columns alone).  A 48-column layout (the action head)
+    ends its head with the step's ``env.actions``, a 72-column one with ``actions_recorder.flatten()``."""
     rb, isg = env.robot, env.isg_env
     src = {name: getattr(rb if key != "command" else env, label) for name, (key, label) in _OBS_PROBE.items()}
-    head = torch.cat([src[name] for name in layout.slots]
-                     + [rb.dof_pos - rb.default_dof_pos, rb.dof_vel, env.actions_recorder.flatten()], dim=1)
+    last = env.actions if layout.head == nv.OBS_HEAD_ACT else env.actions_recorder.flatten()
+    head = torch.cat([src[name] for name in layout.slots] + [rb.dof_pos - rb.default_dof_pos, rb.dof_vel, last],
+                     dim=1)
     head = head * torch.tensor(layout.scales, dtype=torch.float, device=head.device)
     if blind:
         if u is not None and layout.has_noise():
@@ -642,10 +677,11 @@ def a1_obs_definition(env, layout: ObsLayout, u: Optional[torch.Tensor] = None, 
 def verify_a1_obs(env, layout: ObsLayout, seed: int = 4321, num_obs: Optional[int] = None):
     """``env.compute_observations`` against the layout's definition (noise included) on a seeded random
     state, with the same seeded draws given to the hook's ``torch.rand_like`` and to the definition.
-    ``num_obs = 72``: the blind observation, with the heights replaced by a stand-in that refuses any use."""
+    ``num_obs = layout.head``: the blind observation, with the heights replaced by a stand-in that refuses
+    any use."""
     isg = env.isg_env
-    blind = num_obs == nv.OBS_HEAD
-    width = nv.OBS_HEAD + (0 if blind else isg.num_height_points)
+    blind = num_obs == layout.head
+    width = layout.head + (0 if blind else isg.num_height_points)
     had = isg.__dict__.get("_measured_heights")
     with A1Probe(env) as pr:
         pr.randomize(seed)

@@ -43,26 +43,28 @@ def draw_randint(seed: int, env_ids: torch.Tensor, step: int, stream: int, high:
     return ((x >> 8) * high) >> 24
 
 
-STREAM_OBS_NOISE, OBS_COLS, OBS_HEAD = 8, 259, 72
+STREAM_OBS_NOISE, OBS_COLS, OBS_HEAD, OBS_HEAD_ACT, OBS_POINTS = 8, 259, 72, 48, 187
 
 
-def obs_noise_slots():
-    """(word, lane) int64 tensors of the 259 observation columns (map: include/shifu_b200.h)."""
-    col = torch.arange(OBS_COLS)
+def obs_noise_slots(head: int = OBS_HEAD):
+    """(word, lane) int64 tensors of the head + 187 observation columns (map: include/shifu_b200.h).
+    ``head``: 72, or 48 for the action head, whose column d + 12m keeps the 72-column head's position."""
+    col = torch.arange(head + OBS_POINTS)
     m, d = col // 12, col % 12
-    pt = (col - OBS_HEAD).clamp(min=0)
+    pt = (col - head).clamp(min=0)
     k = torch.minimum(pt, 186 - pt)
-    head = col < OBS_HEAD
+    head = col < head
     word = torch.where(head, 3 * (d >> 1) + (m >> 1), 18 + (k >> 1))
     lane = torch.where(head, (d & 1) + 2 * (m & 1), 2 * (k & 1) + (pt != k).long())
     return word, lane
 
 
-def obs_noise_u01(seed: int, env_ids: torch.Tensor, step: int) -> torch.Tensor:
-    """(R, 259) float32 u of the fused kernels' observation noise for global env ids ``env_ids`` at ``step``
-    (the step the same step's reset draws use): a user-hook ``compute_observations`` that takes
-    ``torch.rand_like(obs_buf)`` from here adds the noise the kernel adds."""
-    word, lane = (t.to(env_ids.device) for t in obs_noise_slots())
+def obs_noise_u01(seed: int, env_ids: torch.Tensor, step: int, head: int = OBS_HEAD) -> torch.Tensor:
+    """(R, head + 187) float32 u of the fused kernels' observation noise for global env ids ``env_ids`` at
+    ``step`` (the step the same step's reset draws use): a user-hook ``compute_observations`` that takes
+    ``torch.rand_like(obs_buf)`` from here adds the noise the kernel adds (a blind one takes the first
+    ``head`` columns).  ``head``: 72, or 48 for the action head."""
+    word, lane = (t.to(env_ids.device) for t in obs_noise_slots(head))
     n_words = int(word.max()) + 1
     e = (env_ids.to(torch.int64) & _MASK).unsqueeze(1)
     z = torch.zeros(e.shape[0], n_words, dtype=torch.int64, device=env_ids.device)
